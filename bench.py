@@ -21,6 +21,9 @@ One JSON line on rank 0:
             timed on this box's host cores on a bounded sample of the same workload
 
 `--impl reference` times the CPU path only (rank 0), same metric/config.
+`--dump-outputs DIR` writes the result records of the last timed step (one per pair, 2 MB at the default 8192 pairs),
+one .npy per field, in the job's pair order whatever the number of GPUs; the workload is seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -57,7 +60,47 @@ def parse_args():
     ap.add_argument("--cpu-sample-pairs", type=int, default=12)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-threads", type=int, default=0, help="threads of the CPU arm (0 = all host cores)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result records of the last timed step as DIR/<field>.npy (float32 / float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def job_pair_ids(n_cur, n_cand, world):
+    """the job's pair index (current-major over the current x candidate grid) of every record, in the order the ranks'
+    blocks are gathered (rank-major, current-major inside a block)"""
+    split_cur, split_cand = shard_grid(n_cur, n_cand, world)
+    bc, bk = n_cur // split_cur, n_cand // split_cand
+    ids = [(r // split_cand * bc + ci) * n_cand + r % split_cand * bk + ri
+           for r in range(world) for ci in range(bc) for ri in range(bk)]
+    return np.array(ids, np.int64)
+
+
+def dump_outputs(records, pair_ids, out_dir):
+    """One .npy per field of the RESULT_DTYPE records (include/nicp_b200.h: nicp_align_result), rows in the job's pair
+    order (pair_ids: the pair index of each record), so that runs on any number of GPUs line up.  T and omega stay
+    column-major as the C-ABI returns them; integer fields are stored as float64, which holds them exactly.  `reserved`
+    holds the kernels' work counters, not a result, and is left out.  A job whose records would exceed DUMP_MAX_BYTES is
+    written as a fixed, seeded sample of pairs, listed in pair_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    records = records[np.argsort(pair_ids)]
+    names = [n for n in records.dtype.names if n != "reserved"]
+    per_record = sum(8 * int(np.prod(records.dtype[n].shape, dtype=np.int64)) for n in names)
+    if len(records) * per_record > DUMP_MAX_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(len(records), DUMP_MAX_BYTES // per_record - 1, replace=False))
+        records = records[keep]
+        np.save(os.path.join(out_dir, "pair_index.npy"), keep.astype(np.float64))
+    for name in names:
+        a = records[name]
+        a = a.astype(np.float64) if a.dtype.kind in "iu" else a.astype(np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -463,6 +506,7 @@ def run_ours(args):
         sumMacc += float(results["reserved"][:, 1].sum())
     e1.record(stream)
     barrier()
+    last_step = allrec.copy()  # the e2e leg below writes into the same buffer
     clocks = sampler.stop()
     launches = ctx.launch_count() - launches0
     dev_ms = max_over_ranks(e0.elapsed_time(e1))
@@ -571,6 +615,8 @@ def run_ours(args):
                                                         tracking_frames=args.tracking_frames)
             except Exception as e:
                 line["configs"] = {"error": "%s: %s" % (type(e).__name__, e)}
+        if args.dump_outputs:
+            dump_outputs(last_step, job_pair_ids(n_cur_total, n_cand_total, world), args.dump_outputs)
         emit(line)
     if world > 1:
         dist.barrier()
