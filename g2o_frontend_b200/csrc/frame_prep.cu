@@ -640,9 +640,9 @@ static int launch_prep_set(nicp_context *ctx, const PrepBatch &B, const nicp_pro
     k_integral_rows<false><<<dim3(rows, F), 256, smem, ctx->stream>>>(B, rows, cols, a, proj->min_distance, proj->max_distance, d_pc);
   NICP_CHECK_LAUNCH(ctx);
   const size_t stripBytes = (size_t)rows * 32 * sizeof(float);
-  // batches stream the columns (enough threads to cover the memory latency); a lone frame stages strips in shared memory
-  static const int streamFrom = getenv("NICP_PREP_STREAM_FROM") ? atoi(getenv("NICP_PREP_STREAM_FROM")) : 4;
-  if (F >= streamFrom) {
+  // batches of 4 or more frames stream the columns (enough threads to cover the memory latency); fewer frames stage strips
+  // in shared memory
+  if (F >= 4) {
     k_integral_cols_stream<<<dim3((cols + 127) / 128, kIntegralCh, F), 128, 0, ctx->stream>>>(B, rows, cols);
   } else if (stripBytes <= 200 * 1024) {
     // per context = per device: the attribute is a per-device property of the kernel

@@ -280,8 +280,7 @@ static AlignConsts make_consts(const nicp_projector *proj, const nicp_align_para
 // most ctx->groupSize (<= kMaxGroup) pairs.
 static int stage_groups(nicp_context *ctx, int m, const int *curSlotOf) {
   PairGroup *g = host_groups(ctx);
-  const int cap = ctx->groupWarps >= 2 ? kMaxGroup : kMaxGroup / 2;  // shared-memory T slots of the kernel instantiation
-  const int maxCount = ctx->groupSize < 1 ? 1 : (ctx->groupSize > cap ? cap : ctx->groupSize);
+  const int maxCount = ctx->groupSize < 1 ? 1 : (ctx->groupSize > kMaxGroup ? kMaxGroup : ctx->groupSize);
   int n = 0;
   for (int i = 0; i < m;) {
     int j = i + 1;
@@ -455,17 +454,7 @@ int nicp_create(int device, nicp_context **out) {
   NICP_CUDA(cudaGetDeviceProperties(&prop, device));
   ctx->smCount = prop.multiProcessorCount;
   ctx->blocksPerPair = 296;  // lower bound of the partial-row allocation
-  ctx->corrVariant = env_int("NICP_CORR_VARIANT", 1) - 1;  // grouped-kernel variant (corr_lin.cuh VAR), 1-based in the environment
-  // fixed per context (not per batch) so that a pair's H/b never depend on batch size or GPU count
-  ctx->tileConfig = env_int("NICP_TILE_CONFIG", 1) - 1;
-  if (ctx->tileConfig < 0 || ctx->tileConfig > 3) ctx->tileConfig = 0;
   ctx->groupSize = env_int("NICP_GROUP", 16);
-  ctx->groupMinBlocks = env_int("NICP_GROUP_MINB", 16);
-  ctx->groupWarps = env_int("NICP_GROUP_WARPS", 1);
-  {
-    const char *v = getenv("NICP_PROJECT_BY_REFERENCE");
-    ctx->projByReference = (v && *v) ? atoi(v) : 1;
-  }
   {
     const char *v = getenv("NICP_GROUP_MIN_AVG");  // 0 = always the grouped kernel (tests)
     ctx->groupMinAvg = (v && *v) ? atoi(v) : 3;
@@ -1165,7 +1154,7 @@ struct HostPrior {
 struct GraphKey {
   AlignConsts ac;
   float co[16];
-  int outer, inner, numPriors, corrVariant, tileConfig, slots, partialRows;
+  int outer, inner, numPriors, slots, partialRows;
   float imgThr;
   size_t slotPixels;
   const void *desc, *results, *statHb, *trace, *priors, *refZ;
@@ -1282,7 +1271,7 @@ static int align_common(nicp_context *ctx, int n, const nicp_cloud *const *refs,
       key.ac = ac;
       memcpy(key.co, co, sizeof co);
       key.outer = ap->outer_iterations; key.inner = ap->inner_iterations; key.numPriors = numPriors;
-      key.corrVariant = ctx->corrVariant; key.tileConfig = ctx->tileConfig; key.slots = ctx->slots;
+      key.slots = ctx->slots;
       key.partialRows = ctx->partialRows; key.imgThr = imgThr; key.slotPixels = ctx->slotPixels;
       key.desc = ctx->d_desc; key.results = ctx->d_results; key.statHb = ctx->d_statHb; key.trace = ctx->d_trace;
       key.priors = ctx->d_priors; key.refZ = ctx->d_refZ;

@@ -33,7 +33,7 @@ void set_error(const char *fmt, ...);
 
 constexpr int kMaxCams = 8;       // NICP_MAX_CAMERAS
 constexpr int kRowGroups = 16;    // first-level CTAs per pair of k_reduce_solve (align.cu); partials2 holds that many rows per slot
-constexpr int kMaxGroup = 32;     // pairs per group of the grouped fused kernel (corr_lin.cuh)
+constexpr int kMaxGroup = 16;     // pairs per group of the grouped fused kernel (corr_lin.cuh: T of each in shared memory)
 constexpr int kMaxPrepBatch = 8;  // frames per frame-preparation launch set (their scratch stays L2 resident)
 constexpr int kAccum = 32;        // accumulator slots per partial (30 used)
 constexpr int kIntegralCh = 10;   // n,x,y,z,xx,xy,xz,yy,yz,zz
@@ -284,13 +284,8 @@ struct nicp_context {
   int slots;          // allocated slots
   size_t slotPixels;  // pixels per slot
   int blocksPerPair;            // lower bound of the partial-row allocation
-  int corrVariant;              // reserved (one fused-kernel variant is compiled)
-  int tileConfig;               // fused-kernel variant: 0 = grouped kernel (default), 1..3 = round-1 per-pair kernels
   int groupSize;                // pairs per group of the grouped kernel (pairs of a group share their current cloud)
-  int groupMinBlocks;           // its __launch_bounds__ min-blocks instantiation (16 or 20 warps per SM)
   int groupMinAvg;              // mean pairs per group from which a chunk takes the grouped kernel (else the per-pair one)
-  int groupWarps;               // warps per CTA of the grouped kernel (1 or 2; they share the current side of the tile)
-  int projByReference;          // k_project walks the pairs of a chunk grouped by reference cloud (L2 reuse of the point stream)
   int partialRows;              // rows of d_partials per slot
   unsigned long long *d_refZ;   // [slots][2][P]
   unsigned long long *d_curZ;   // [slots][P]

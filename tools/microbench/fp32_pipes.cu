@@ -1,7 +1,7 @@
 // fp32_pipes.cu -- how many FP32 operations per clock per SM the B200 sustains for scalar FFMA / FADD and for the
 // packed FFMA2 / FADD2 (fma.rn.f32x2, add.rn.f32x2: sm_100 only).  Decides whether the Linearizer term of the fused
-// kernel (align.cu accumulate_term, ~200 FP32 instructions per accepted correspondence) should be written with packed
-// operations.  Build: nvcc -O3 -gencode arch=compute_100a,code=sm_100a -o fp32_pipes fp32_pipes.cu
+// kernel (~200 scalar FP32 instructions per accepted correspondence) should be written with packed operations; it is
+// (term_add_e in corr_lin.cuh).  Build: nvcc -O3 -gencode arch=compute_100a,code=sm_100a -o fp32_pipes fp32_pipes.cu
 #include <cstdio>
 #include <cuda_runtime.h>
 

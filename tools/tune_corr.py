@@ -1,5 +1,5 @@
 """Kernel tuning harness (not part of the product): times the fused correspondence+linearise kernel and the
-whole align step on a 64-pair batch for the variant selected by the environment."""
+whole align step on a 64-pair batch."""
 import os
 import sys
 import time
@@ -36,9 +36,9 @@ def main():
     nl = max(kt["corr_lin_launches"], 1)
     byts = (8.0 * P * len(pairs) * 10 + 56.0 * res["reserved"][:, 0].sum() + 48.0 * res["reserved"][:, 1].sum()) * reps
     gbs = byts / (kt["corr_lin_ms"] * 1e-3) / 1e9
-    print("tile_config=%s slots=%s pairs=%d: step %.2f ms (%.0f align/s) | corr_lin %.1f us/launch, %.0f GB/s (%.3f of 6540) | "
+    print("slots=%s pairs=%d: step %.2f ms (%.0f align/s) | corr_lin %.1f us/launch, %.0f GB/s (%.3f of 6540) | "
           "project %.1f us/launch | checksum inliers=%d T00=%.9f" %
-          (os.environ.get("NICP_TILE_CONFIG", "1"), os.environ.get("NICP_BATCH_SLOTS", "64"), len(pairs), dt * 1e3,
+          (os.environ.get("NICP_BATCH_SLOTS", "64"), len(pairs), dt * 1e3,
            len(pairs) / dt, kt["corr_lin_ms"] / nl * 1e3, gbs, gbs / 6539.9, kt["project_ms"] / max(kt["project_launches"], 1) * 1e3,
            int(res["inliers"].sum()), float(res["T"][:, 0].mean())))
     ctx.close()
