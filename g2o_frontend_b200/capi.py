@@ -27,6 +27,7 @@ SYMBOLS = [
     "nicp_project", "nicp_correspond_linearize", "nicp_linearize",
     "nicp_align", "nicp_align_get_state", "nicp_align_get_trace", "nicp_align_batch", "nicp_align_batch_priors",
     "nicp_multi_image_size", "nicp_multi_depth_to_cloud", "nicp_multi_project", "nicp_multi_align",
+    "nicp_multi_raw_depth_to_cloud_batch", "nicp_multi_align_batch",
     "nicp_cloud_compute_gaussians", "nicp_cloud_has_gaussians", "nicp_cloud_download_gaussians",
     "nicp_cloud_upload_gaussians", "nicp_merge", "nicp_voxelize",
     "nicp_shard_pool_create", "nicp_shard_pool_destroy", "nicp_shard_pool_size", "nicp_align_frames_sharded",
@@ -556,6 +557,63 @@ class Context:
         _check(self.L, self.L.nicp_multi_align(self.handle, ref.handle, cur.handle, C.byref(mp), C.byref(ap), _fptr(ro),
                                                _fptr(co), _fptr(g), parr, len(priors), C.c_float(img_threshold), C.byref(res)))
         return res
+
+    def multi_raw_depth_to_cloud_batch(self, frames, mp, sp, depth_scale=0.001, step=1, max_depth_cov=0.01, sensor_offset=None,
+                                       keep_stats=False, clouds=None):
+        """n rig frames -> n clouds (nicp_multi_raw_depth_to_cloud_batch).  frames: n sequences of mp.num_cameras raw uint16
+        images in sensor orientation (camera i: (height_i * step) x (width_i * step), the same shape in every frame), numpy
+        arrays or numpy views of pinned buffers.  Asynchronous like raw_depth_to_cloud_batch."""
+        n, nc = len(frames), mp.num_cameras
+        imgs = []
+        for fr in frames:
+            assert len(fr) == nc, "a frame needs one raw image per camera"
+            imgs += [r if (isinstance(r, np.ndarray) and r.dtype == np.uint16 and r.flags.c_contiguous)
+                     else np.ascontiguousarray(r, np.uint16) for r in fr]
+        shapes = [imgs[i].shape for i in range(nc)] if n else []
+        for k, im in enumerate(imgs):
+            assert im.shape == shapes[k % nc], "camera %d has a different raw size in frame %d" % (k % nc, k // nc)
+        rr = np.array([s[0] for s in shapes] or [0], np.int32)
+        rc = np.array([s[1] for s in shapes] or [0], np.int32)
+        rows, cols = multi_image_size(mp, self.verify)
+        clouds = clouds or [self.new_cloud(rows * cols) for _ in range(n)]
+        so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
+        RA = (C.c_void_p * max(len(imgs), 1))(*[im.ctypes.data for im in imgs])
+        CA = (C.c_void_p * max(n, 1))(*[c.handle for c in clouds])
+        _check(self.L, self.L.nicp_multi_raw_depth_to_cloud_batch(self.handle, n, RA, _iptr(rr), _iptr(rc), C.c_float(depth_scale),
+                                                                  int(step), C.c_float(max_depth_cov), C.byref(mp), C.byref(sp),
+                                                                  _fptr(so), int(keep_stats), CA))
+        self._keepalive = imgs  # the copies are asynchronous: keep the host frames alive until the next call
+        return clouds
+
+    def multi_align_batch(self, refs, curs, mp, ap, guesses=None, ref_offset=None, cur_offset=None, img_threshold=50.0,
+                          results=None, priors=None):
+        """align_batch with a MultiPointProjector (nicp_multi_align_batch): record i equals multi_align on pair i.
+        priors: None or n lists of Prior.  Returns a numpy structured array (RESULT_DTYPE) of n records."""
+        n = len(refs)
+        assert len(curs) == n
+        eye = np.eye(4, dtype=np.float32)
+        ro = colmajor(eye if ref_offset is None else ref_offset)
+        co = colmajor(eye if cur_offset is None else cur_offset)
+        if guesses is None:
+            g = np.tile(colmajor(eye), (n, 1))
+        else:
+            g = np.asarray(guesses, np.float32).transpose(0, 2, 1).reshape(n, 16)
+        g = np.ascontiguousarray(g, np.float32)
+        RA = (C.c_void_p * max(n, 1))(*[r.handle for r in refs])
+        CA = (C.c_void_p * max(n, 1))(*[c.handle for c in curs])
+        if results is None:
+            results = np.zeros(n, RESULT_DTYPE)
+        parr, offs = None, None
+        if priors is not None:
+            assert len(priors) == n
+            flat = [p for ps in priors for p in ps]
+            offs = np.zeros(n + 1, np.int32)
+            offs[1:] = np.cumsum([len(ps) for ps in priors])
+            parr = (Prior * max(len(flat), 1))(*flat)
+        _check(self.L, self.L.nicp_multi_align_batch(self.handle, n, RA, CA, C.byref(mp), C.byref(ap), _fptr(ro), _fptr(co),
+                                                     _fptr(g), parr, None if offs is None else _iptr(offs),
+                                                     C.c_float(img_threshold), results.ctypes.data_as(C.POINTER(AlignResult))))
+        return results
 
     def align_state(self, rows, cols, max_corr=None):
         ri = np.zeros((rows, cols), np.int32)

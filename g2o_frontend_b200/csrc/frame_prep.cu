@@ -40,26 +40,19 @@ struct PrepBatch {
   int *count[kMaxPrepBatch];
 };
 
-__global__ void k_depth_convert(PrepBatch B, int rows, int cols, float scale, int step, float maxCov) {
-  const uint16_t *__restrict__ raw = B.raw[blockIdx.y];
-  float *__restrict__ out = B.depth[blockIdx.y];
-  int drows = rows / step, dcols = cols / step;
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= drows * dcols) return;
-  int r = i / dcols, c = i - r * dcols;
-  if (step <= 1) {
-    uint16_t v = raw[i];
-    out[i] = v ? fmul(scale, (float)v) : 0.0f;
-    return;
-  }
+// DepthImage_convert_16UC1_to_32FC1 of one raw value
+__device__ __forceinline__ float depth_u16_to_m(uint16_t v, float scale) { return v ? fmul(scale, (float)v) : 0.0f; }
+
+// DepthImage_scale(step > 1) of the converted rows x cols raw image at scaled pixel (r, c)
+__device__ __forceinline__ float depth_scale_pixel(const uint16_t *__restrict__ raw, int rows, int cols, int r, int c, float scale,
+                                                   int step, float maxCov) {
   float acc = 0.f, acc2 = 0.f;
   int np = 0;
   int sr = r * step, sc = c * step;
   for (int a = 0; a < step; a++)
     for (int b = 0; b < step; b++) {
       if (sr + a < rows && sc + b < cols) {
-        uint16_t v = raw[(size_t)(sr + a) * cols + sc + b];
-        float f = v ? fmul(scale, (float)v) : 0.0f;
+        float f = depth_u16_to_m(raw[(size_t)(sr + a) * cols + sc + b], scale);
         acc = fadd(acc, f);
         acc2 = fadd(acc2, fmul(f, f));
         np += f > 0;
@@ -71,7 +64,57 @@ __global__ void k_depth_convert(PrepBatch B, int rows, int cols, float scale, in
     float sigma = fsub(fdiv(acc2, (float)np), fmul(mu, mu));
     if (!(sigma > maxCov)) res = mu;
   }
-  out[i] = res;
+  return res;
+}
+
+__global__ void k_depth_convert(PrepBatch B, int rows, int cols, float scale, int step, float maxCov) {
+  const uint16_t *__restrict__ raw = B.raw[blockIdx.y];
+  float *__restrict__ out = B.depth[blockIdx.y];
+  int drows = rows / step, dcols = cols / step;
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= drows * dcols) return;
+  int r = i / dcols, c = i - r * dcols;
+  if (step <= 1) {
+    out[i] = depth_u16_to_m(raw[i], scale);
+    return;
+  }
+  out[i] = depth_scale_pixel(raw, rows, cols, r, c, scale, step, maxCov);
+}
+
+// Raw frames of a MultiPointProjector rig -> composite depth images in the layout of CamSet (the one the Aligner projects
+// into): camera i's raw image is H_i x W_i in sensor orientation (row = v, column = u) and scales to height_i x width_i;
+// composite[u][colOff_i + v] = scaled pixel (v, u), and rows [width_i, rows) of camera i's column block are 0.
+// grid = (ceil(max height / 32), ceil(rows / 32), frames x cameras), 32 x 8 threads: a 32 x 32 tile is converted along u
+// (coalesced raw reads at step 1; at step > 1 a lane reads its own step x step box) into shared memory and written out
+// transposed along v (coalesced composite writes).
+struct RigFrames {
+  const uint16_t *raw[kMaxPrepBatch * kMaxCams];  // frame f, camera i at f * nCams + i
+  float *depth[kMaxPrepBatch];
+  int nCams;
+  int rawRows[kMaxCams], rawCols[kMaxCams], width[kMaxCams], height[kMaxCams], colOff[kMaxCams];
+};
+
+__global__ void __launch_bounds__(256) k_rig_depth_convert(RigFrames R, int rows, int cols, float scale, int step, float maxCov) {
+  __shared__ float tile[32][33];  // [v][u], +1: the transposed reads hit 32 different banks
+  const int f = blockIdx.z / R.nCams, cam = blockIdx.z - f * R.nCams;
+  const int width = R.width[cam], height = R.height[cam];
+  const int v0 = blockIdx.x * 32, u0 = blockIdx.y * 32;
+  if (v0 >= height) return;  // the grid covers the tallest camera
+  const uint16_t *__restrict__ raw = R.raw[blockIdx.z];
+  const int rawRows = R.rawRows[cam], rawCols = R.rawCols[cam];
+  for (int k = threadIdx.y; k < 32; k += 8) {
+    const int v = v0 + k, u = u0 + threadIdx.x;
+    float d = 0.0f;
+    if (v < height && u < width)
+      d = step <= 1 ? depth_u16_to_m(raw[(size_t)v * rawCols + u], scale) : depth_scale_pixel(raw, rawRows, rawCols, v, u, scale, step, maxCov);
+    tile[k][threadIdx.x] = d;
+  }
+  __syncthreads();
+  float *__restrict__ out = R.depth[f] + R.colOff[cam];
+  for (int k = threadIdx.y; k < 32; k += 8) {
+    const int u = u0 + k, v = v0 + threadIdx.x;
+    if (u < rows && v < height) out[(size_t)u * cols + v] = tile[threadIdx.x][k];
+  }
 }
 
 int launch_depth_convert(nicp_context *ctx, const uint16_t *d_raw, int rows, int cols, float scale, int step,
@@ -736,6 +779,42 @@ int launch_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw
   k_depth_convert<<<dim3((outPx + 255) / 256, n), 256, 0, ctx->stream>>>(B, rawRows, rawCols, scale, step, maxCov);
   NICP_CHECK_LAUNCH(ctx);
   return launch_prep_set(ctx, B, proj, sp, sensorOffset, nullptr, nullptr, nullptr);
+}
+
+// the same for n rig frames: d_raw[f * cams.n + i] = camera i of frame f on the device (rawRows[i] x rawCols[i]), proj = the
+// composite image (rows = max width, cols = sum of heights); one conversion launch for every camera of every frame
+int launch_rig_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw, const int *rawRows, const int *rawCols,
+                              float scale, int step, float maxCov, const nicp_projector *proj, const CamSet &cams,
+                              const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds) {
+  const size_t px = (size_t)proj->rows * proj->cols;
+  if (n > ctx->batchSlots || px > ctx->batchPixels) {
+    set_error("internal: batch prep scratch too small");
+    return NICP_ERR_INVALID;
+  }
+  PrepBatch B;
+  memset(&B, 0, sizeof B);
+  RigFrames R;
+  memset(&R, 0, sizeof R);
+  R.nCams = cams.n;
+  int maxHeight = 0;
+  for (int i = 0; i < cams.n; i++) {
+    R.rawRows[i] = rawRows[i];
+    R.rawCols[i] = rawCols[i];
+    R.width[i] = cams.width[i];
+    R.height[i] = cams.height[i];
+    R.colOff[i] = cams.colOff[i];
+    if (cams.height[i] > maxHeight) maxHeight = cams.height[i];
+  }
+  for (int f = 0; f < n; f++) {
+    prep_batch_add(B, ctx->d_bDepth + (size_t)f * ctx->batchPixels, ctx->d_bIntegral + (size_t)f * ctx->batchPixels * kIntegralCh,
+                   clouds[f], keepStats != 0);
+    R.depth[f] = B.depth[f];
+    for (int i = 0; i < cams.n; i++) R.raw[f * cams.n + i] = d_raw[f * cams.n + i];
+  }
+  k_rig_depth_convert<<<dim3((maxHeight + 31) / 32, (proj->rows + 31) / 32, n * cams.n), dim3(32, 8), 0, ctx->stream>>>(
+      R, proj->rows, proj->cols, scale, step, maxCov);
+  NICP_CHECK_LAUNCH(ctx);
+  return launch_prep_set(ctx, B, proj, sp, sensorOffset, nullptr, nullptr, &cams);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -2,6 +2,7 @@
 // Host-side orchestration only: scratch management, H2D/D2H, kernel sequencing, and the tiny
 // dense statistics of Aligner::_computeStatistics (aligner.cpp:152-199).  No CPU fallback: every
 // compute entry point launches CUDA kernels or fails.
+#include <climits>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstring>
@@ -123,8 +124,13 @@ static void free_align(nicp_context *ctx) {
 }
 static int ensure_align(nicp_context *ctx, int slots, size_t pixels) {
   if (slots <= ctx->slots && pixels <= ctx->slotPixels) return NICP_OK;
-  if (slots < ctx->slots) slots = ctx->slots;
-  if (pixels < ctx->slotPixels) pixels = ctx->slotPixels;
+  // keep the larger old dimension only while that does not make the allocation bigger than both the old one and the request:
+  // many slots of small images followed by a few of large ones (a rig chunk after pinhole batches) must not multiply out
+  const size_t keepSlots = std::max<size_t>(slots, ctx->slots), keepPixels = std::max(pixels, ctx->slotPixels);
+  if (keepSlots * keepPixels <= std::max((size_t)slots * pixels, (size_t)ctx->slots * ctx->slotPixels)) {
+    slots = (int)keepSlots;
+    pixels = keepPixels;
+  }
   free_align(ctx);
   int rc;
   if ((rc = dev_alloc(&ctx->d_refZ, 2 * (size_t)slots * pixels))) return rc;
@@ -958,6 +964,104 @@ int nicp_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *cons
   return NICP_OK;
 }
 
+// frames per launch set of nicp_multi_raw_depth_to_cloud_batch for a composite image of px pixels: a set's scratch (depth +
+// integral image, 44 B per pixel and frame) stays within that of a full pinhole set (kMaxPrepBatch frames of 640x480,
+// 108 MB), at least one frame.  Frames are batched so that their row and column chains fill the GPU; a composite of
+// 1280 x 3840 already brings 1280 row passes and 38 400 column chains on its own, so it runs one frame per set (216 MB)
+// instead of 1.7 GB for eight.
+static int rig_prep_frames(size_t px) {
+  const size_t f = (size_t)kMaxPrepBatch * 640 * 480 / px;
+  return f < 1 ? 1 : (f > (size_t)kMaxPrepBatch ? kMaxPrepBatch : (int)f);
+}
+
+int nicp_multi_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *const *raws, const int *raw_rows,
+                                        const int *raw_cols, float depth_scale, int step, float max_depth_cov,
+                                        const nicp_multi_projector *mp, const nicp_stats_params *sp,
+                                        const float sensor_offset[16], int keep_stats, nicp_cloud *const *clouds) {
+  if (!ctx || n < 0 || !mp || !sp) return NICP_ERR_INVALID;
+  NICP_CUDA(cudaSetDevice(ctx->device));
+  if (n == 0) return NICP_OK;
+  if (!raws || !clouds || !raw_rows || !raw_cols) return NICP_ERR_INVALID;
+  if (step < 1) step = 1;
+  CamSet cams;
+  int rows, cols, rc;
+  if ((rc = camset_multi(mp, cams, rows, cols))) return rc;
+  const int nc = cams.n;
+  size_t rpx = 0;
+  for (int i = 0; i < nc; i++) {
+    if (raw_rows[i] <= 0 || raw_cols[i] <= 0 || raw_rows[i] / step != cams.height[i] || raw_cols[i] / step != cams.width[i]) {
+      set_error("camera %d: raw image %dx%d at step %d does not scale to the projector's %dx%d (rows x cols = height x width)",
+                i, raw_rows[i], raw_cols[i], step, cams.height[i], cams.width[i]);
+      return NICP_ERR_INVALID;
+    }
+    rpx += (size_t)raw_rows[i] * raw_cols[i];
+  }
+  const size_t px = (size_t)rows * cols;
+  for (int f = 0; f < n; f++) {
+    for (int i = 0; i < nc; i++)
+      if (!raws[f * nc + i]) {
+        set_error("null raw image of camera %d in frame %d", i, f);
+        return NICP_ERR_INVALID;
+      }
+    if (!clouds[f]) {
+      set_error("null cloud at index %d", f);
+      return NICP_ERR_INVALID;
+    }
+    if ((size_t)clouds[f]->capacity < px) {
+      set_error("cloud %d: capacity %d smaller than the composite image (%zu pixels)", f, clouds[f]->capacity, px);
+      return NICP_ERR_INVALID;
+    }
+    if (clouds[f]->device != ctx->device) {
+      set_error("cloud %d lives on GPU %d, the context on GPU %d", f, clouds[f]->device, ctx->device);
+      return NICP_ERR_INVALID;
+    }
+    for (int j = 0; j < f; j++)
+      if (clouds[j] == clouds[f]) {
+        set_error("cloud %d and cloud %d are the same object", j, f);
+        return NICP_ERR_INVALID;
+      }
+  }
+  int sub = env_int("NICP_PREP_BATCH", kMaxPrepBatch);
+  if (sub > rig_prep_frames(px)) sub = rig_prep_frames(px);
+  if (sub < 1) sub = 1;
+  if (sub > n) sub = n;
+  if ((rc = ensure_batch_prep(ctx, sub, px, rpx))) return rc;
+  float eye[16];
+  mat4_identity(eye);
+  for (int base = 0; base < n; base += sub) {
+    const int m = n - base < sub ? n - base : sub;
+    // as in nicp_raw_depth_to_cloud_batch: sub-batch k is uploaded into staging set k & 1 while sub-batch k - 1 computes;
+    // the cameras of a frame sit back to back in its staging slot
+    const int b = (ctx->bRawToggle ^= 1);
+    uint16_t *stage = ctx->d_bRaw + (size_t)b * ctx->batchSlots * ctx->batchRawPixels;
+    const uint16_t *d_raw[kMaxPrepBatch * kMaxCams];
+    NICP_CUDA(cudaStreamWaitEvent(ctx->copyStream, ctx->evBRawUsed[b], 0));
+    for (int f = 0; f < m; f++) {
+      uint16_t *dst = stage + (size_t)f * ctx->batchRawPixels;
+      for (int i = 0; i < nc; i++) {
+        const size_t cpx = (size_t)raw_rows[i] * raw_cols[i];
+        NICP_CUDA(cudaMemcpyAsync(dst, raws[(size_t)(base + f) * nc + i], cpx * sizeof(uint16_t), cudaMemcpyHostToDevice,
+                                  ctx->copyStream));
+        d_raw[f * nc + i] = dst;
+        dst += cpx;
+      }
+    }
+    NICP_CUDA(cudaEventRecord(ctx->evBRawCopied[b], ctx->copyStream));
+    NICP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evBRawCopied[b], 0));
+    for (int f = 0; f < m; f++)
+      if (keep_stats && (rc = ensure_stats(clouds[base + f]))) return rc;
+    nicp_projector proj = mp->camera[0];
+    proj.rows = rows;
+    proj.cols = cols;
+    if ((rc = launch_rig_raw_prep_batch(ctx, m, d_raw, raw_rows, raw_cols, depth_scale, step, max_depth_cov, &proj, cams, sp,
+                                        sensor_offset ? sensor_offset : eye, keep_stats, clouds + base)))
+      return rc;
+    NICP_CUDA(cudaEventRecord(ctx->evBRawUsed[b], ctx->stream));
+  }
+  ctx->lastRows = 0;
+  return NICP_OK;
+}
+
 // ---- stage-level statistics / information matrices (host buffers in, host buffers out) -----------------------------
 int nicp_stats_compute(nicp_context *ctx, const float *points4, int n, const int *index_image, const int *interval_image,
                        int rows, int cols, const nicp_stats_params *sp, float *normals4, float *stats16, float *eigenvalues3,
@@ -1165,11 +1269,12 @@ static int align_common(nicp_context *ctx, int n, const nicp_cloud *const *refs,
                         const nicp_projector *proj, const nicp_align_params *ap, const float *refOffset,
                         const float *curOffset, const float *guesses, float imgThr, nicp_align_result *results,
                         bool single, const nicp_prior *priors = nullptr, int numPriors = 0, const CamSet *multiCams = nullptr,
-                        const int *priorOffsets = nullptr) {
+                        const int *priorOffsets = nullptr, int slotCap = INT_MAX) {
   // priorOffsets (batch): pair i owns priors[priorOffsets[i] .. priorOffsets[i + 1]); null: every pair gets all numPriors
   if (priorOffsets) numPriors = priorOffsets[n];
   const size_t P = (size_t)proj->rows * proj->cols;
   int maxSlots = single ? 1 : env_int("NICP_BATCH_SLOTS", 256);
+  if (maxSlots > slotCap) maxSlots = slotCap;
   if (maxSlots > n) maxSlots = n;
   int rc;
   if ((rc = ensure_align(ctx, maxSlots, P))) return rc;
@@ -1366,6 +1471,15 @@ static int align_common(nicp_context *ctx, int n, const nicp_cloud *const *refs,
   return NICP_OK;
 }
 
+// prior_offsets of a batch: n + 1 non-decreasing entries from 0 (or NULL: no priors)
+static bool prior_offsets_valid(int n, const nicp_prior *priors, const int *prior_offsets) {
+  if (!prior_offsets) return true;
+  if (prior_offsets[0] != 0) return false;
+  for (int i = 0; i < n; i++)
+    if (prior_offsets[i + 1] < prior_offsets[i]) return false;
+  return !(prior_offsets[n] > 0 && !priors);
+}
+
 int nicp_align(nicp_context *ctx, const nicp_cloud *reference, const nicp_cloud *current, const nicp_projector *proj,
                const nicp_align_params *ap, const float reference_sensor_offset[16], const float current_sensor_offset[16],
                const float initial_guess[16], const nicp_prior *priors, int num_priors, float frame_inlier_depth_threshold,
@@ -1397,12 +1511,7 @@ int nicp_align_batch_priors(nicp_context *ctx, int n, const nicp_cloud *const *r
   NICP_CUDA(cudaSetDevice(ctx->device));
   if (n == 0) return NICP_OK;
   if (!references || !currents || !results) return NICP_ERR_INVALID;
-  if (prior_offsets) {
-    if (prior_offsets[0] != 0) return NICP_ERR_INVALID;
-    for (int i = 0; i < n; i++)
-      if (prior_offsets[i + 1] < prior_offsets[i]) return NICP_ERR_INVALID;
-    if (prior_offsets[n] > 0 && !priors) return NICP_ERR_INVALID;
-  }
+  if (!prior_offsets_valid(n, priors, prior_offsets)) return NICP_ERR_INVALID;
   return align_common(ctx, n, references, currents, proj, ap, reference_sensor_offset, current_sensor_offset, initial_guesses,
                       frame_inlier_depth_threshold, results, false, priors, 0, nullptr, prior_offsets);
 }
@@ -1482,6 +1591,29 @@ int nicp_multi_align(nicp_context *ctx, const nicp_cloud *reference, const nicp_
   proj.cols = cols;
   return align_common(ctx, 1, &reference, &current, &proj, ap, reference_sensor_offset, current_sensor_offset, initial_guess,
                       frame_inlier_depth_threshold, result, true, priors, num_priors, &cams);
+}
+
+int nicp_multi_align_batch(nicp_context *ctx, int n, const nicp_cloud *const *references, const nicp_cloud *const *currents,
+                           const nicp_multi_projector *mp, const nicp_align_params *ap, const float reference_sensor_offset[16],
+                           const float current_sensor_offset[16], const float *initial_guesses, const nicp_prior *priors,
+                           const int *prior_offsets, float frame_inlier_depth_threshold, nicp_align_result *results) {
+  if (!ctx || n < 0 || !mp || !ap) return NICP_ERR_INVALID;
+  NICP_CUDA(cudaSetDevice(ctx->device));
+  if (n == 0) return NICP_OK;
+  if (!references || !currents || !results) return NICP_ERR_INVALID;
+  if (!prior_offsets_valid(n, priors, prior_offsets)) return NICP_ERR_INVALID;
+  CamSet cams;
+  int rows, cols, rc;
+  if ((rc = camset_multi(mp, cams, rows, cols))) return rc;
+  nicp_projector proj = mp->camera[0];
+  proj.rows = rows;
+  proj.cols = cols;
+  // a slot holds 32 B per pixel of z-buffers and index images: a chunk gets at most the memory of 256 pinhole 640x480 slots
+  // (2.5 GB; 16 slots at 1280x3840)
+  const size_t P = (size_t)rows * cols;
+  const int slotCap = (int)std::max<size_t>(1, (size_t)256 * 640 * 480 / P);
+  return align_common(ctx, n, references, currents, &proj, ap, reference_sensor_offset, current_sensor_offset, initial_guesses,
+                      frame_inlier_depth_threshold, results, false, priors, 0, &cams, prior_offsets, slotCap);
 }
 
 int nicp_align_get_state(nicp_context *ctx, int *reference_index, float *reference_depth, int *current_index,

@@ -357,6 +357,9 @@ int launch_frame_prep(nicp_context *ctx, const float *d_depth, const nicp_projec
 int launch_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw, int rawRows, int rawCols, float scale, int step,
                           float maxCov, const nicp_projector *proj, const nicp_stats_params *sp, const float sensorOffset[16],
                           int keepStats, nicp_cloud *const *clouds);
+int launch_rig_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw, const int *rawRows, const int *rawCols,
+                              float scale, int step, float maxCov, const nicp_projector *proj, const CamSet &cams,
+                              const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds);
 int launch_stats_stage(nicp_context *ctx, const float4 *d_points, int n, const int *d_index, const int *d_interval, int rows,
                        int cols, const nicp_stats_params *sp, float *d_integral, float4 *d_normals, float *d_stats16,
                        float *d_eigvals, int *d_statsN, float *d_curvature);

@@ -360,6 +360,34 @@ int nicp_multi_align(nicp_context *ctx, const nicp_cloud *reference, const nicp_
                      const float reference_sensor_offset[16], const float current_sensor_offset[16],
                      const float initial_guess[16], const nicp_prior *priors, int num_priors,
                      float frame_inlier_depth_threshold, nicp_align_result *result);
+/* Rig frames from raw 16-bit images, n frames at a time: the rig counterpart of nicp_raw_depth_to_cloud_batch.
+ * raws[f * num_cameras + i] is camera i of frame f as the sensor delivers it, raw_rows[i] x raw_cols[i] (row = pixel v,
+ * column = pixel u).  Each image is converted (depth_scale) and scaled (DepthImage_scale(step), in sensor orientation) like
+ * nicp_raw_depth_to_cloud, then transposed into the composite image of nicp_multi_depth_to_cloud:
+ *   composite rows = max over cameras of width_i, composite cols = sum of height_i,
+ *   composite[u][colOff_i + v] = scaled image i at (v, u), camera i owning columns [colOff_i, colOff_i + height_i),
+ *   rows [width_i, rows) of that block are empty (0).
+ * width_i = mp->camera[i].rows and height_i = mp->camera[i].cols (addPointProjector(p, offset, width, height)); mp describes
+ * the rig AFTER scaling, so raw_rows[i] / step must equal height_i and raw_cols[i] / step width_i.  Every frame's cloud is
+ * bit-identical to nicp_multi_depth_to_cloud of that composite.  clouds[f] receives frame f (distinct clouds, capacity >=
+ * composite pixels).  One launch set takes clamp(8 * 640 * 480 / composite pixels, 1, 8) frames (1 at 1280 x 3840), so its
+ * scratch stays within that of 8 pinhole 640x480 frames.  ASYNCHRONOUS like nicp_raw_depth_to_cloud_batch (no index images are returned); pinned raw buffers
+ * must stay unchanged until the next synchronous call on this context returns. */
+int nicp_multi_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *const *raws, const int *raw_rows,
+                                        const int *raw_cols, float depth_scale, int step, float max_depth_cov,
+                                        const nicp_multi_projector *mp, const nicp_stats_params *sp,
+                                        const float sensor_offset[16], int keep_stats, nicp_cloud *const *clouds);
+/* Batched rig alignment of n independent pairs (a rig loop closer verifying one frame against many candidates), with
+ * priors per pair as in nicp_align_batch_priors (priors / prior_offsets may be NULL).  Record i is identical, byte for
+ * byte, to nicp_multi_align on pair i with the same guess and priors.  A lock-step chunk holds at most
+ * max(1, 256 * 640 * 480 / composite pixels) pairs (32 B of scratch per pixel and pair: 16 pairs at 1280 x 3840), or
+ * NICP_BATCH_SLOTS when that is lower. */
+int nicp_multi_align_batch(nicp_context *ctx, int n, const nicp_cloud *const *references,
+                           const nicp_cloud *const *currents, const nicp_multi_projector *mp,
+                           const nicp_align_params *ap, const float reference_sensor_offset[16],
+                           const float current_sensor_offset[16], const float *initial_guesses,
+                           const nicp_prior *priors, const int *prior_offsets,
+                           float frame_inlier_depth_threshold, nicp_align_result *results);
 
 #ifdef __cplusplus
 }
