@@ -31,6 +31,7 @@ SYMBOLS = [
     "nicp_cloud_compute_gaussians", "nicp_cloud_has_gaussians", "nicp_cloud_download_gaussians",
     "nicp_cloud_upload_gaussians", "nicp_merge", "nicp_voxelize",
     "nicp_shard_pool_create", "nicp_shard_pool_destroy", "nicp_shard_pool_size", "nicp_align_frames_sharded",
+    "nicp_multi_align_frames_sharded",
 ]
 
 GAUSS_FLOATS = 24
@@ -715,6 +716,46 @@ class ShardPool:
                                                         C.c_float(max_depth_cov), C.byref(proj), C.byref(sp), _fptr(so), n,
                                                         _iptr(rf), _iptr(cf), _fptr(g), C.byref(ap), C.c_float(img_threshold),
                                                         results.ctypes.data_as(C.POINTER(AlignResult))))
+        return results
+
+    def multi_align_frames(self, frames, mp, sp, ref_frame, cur_frame, guesses, ap, priors=None, depth_scale=0.001, step=1,
+                           max_depth_cov=0.01, sensor_offset=None, img_threshold=50.0):
+        """rig frames in, records out (nicp_multi_align_frames_sharded).  frames: n sequences of mp.num_cameras raw uint16
+        images, as in Context.multi_raw_depth_to_cloud_batch; pair i = (ref_frame[i], cur_frame[i]) with guesses[i] (None:
+        identity); priors: None or one list of Prior per pair.  Returns RESULT_DTYPE records."""
+        nc = mp.num_cameras
+        imgs = []
+        for fr in frames:
+            assert len(fr) == nc, "a frame needs one raw image per camera"
+            imgs += [r if (isinstance(r, np.ndarray) and r.dtype == np.uint16 and r.flags.c_contiguous)
+                     else np.ascontiguousarray(r, np.uint16) for r in fr]
+        shapes = [imgs[i].shape for i in range(nc)] if frames else [(0, 0)] * nc
+        for k, im in enumerate(imgs):
+            assert im.shape == shapes[k % nc], "camera %d has a different raw size in frame %d" % (k % nc, k // nc)
+        rr = np.array([s[0] for s in shapes], np.int32)
+        rc = np.array([s[1] for s in shapes], np.int32)
+        n = len(ref_frame)
+        assert len(cur_frame) == n
+        RA = (C.c_void_p * max(len(imgs), 1))(*[im.ctypes.data for im in imgs])
+        rf = np.ascontiguousarray(ref_frame, np.int32)
+        cf = np.ascontiguousarray(cur_frame, np.int32)
+        g = None
+        if guesses is not None:
+            g = np.ascontiguousarray(np.asarray(guesses, np.float32).transpose(0, 2, 1)).reshape(n, 16)
+        so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
+        parr, offs = None, None
+        if priors is not None:
+            assert len(priors) == n
+            flat = [p for ps in priors for p in ps]
+            offs = np.zeros(n + 1, np.int32)
+            offs[1:] = np.cumsum([len(ps) for ps in priors])
+            parr = (Prior * max(len(flat), 1))(*flat)
+        results = np.zeros(n, RESULT_DTYPE)
+        _check(self.L, self.L.nicp_multi_align_frames_sharded(
+            self.handle, len(frames), RA, _iptr(rr), _iptr(rc), C.c_float(depth_scale), int(step), C.c_float(max_depth_cov),
+            C.byref(mp), C.byref(sp), _fptr(so), n, _iptr(rf), _iptr(cf), None if g is None else _fptr(g), parr,
+            None if offs is None else _iptr(offs), C.byref(ap), C.c_float(img_threshold),
+            results.ctypes.data_as(C.POINTER(AlignResult))))
         return results
 
     def close(self):

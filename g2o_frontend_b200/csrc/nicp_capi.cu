@@ -1471,15 +1471,6 @@ static int align_common(nicp_context *ctx, int n, const nicp_cloud *const *refs,
   return NICP_OK;
 }
 
-// prior_offsets of a batch: n + 1 non-decreasing entries from 0 (or NULL: no priors)
-static bool prior_offsets_valid(int n, const nicp_prior *priors, const int *prior_offsets) {
-  if (!prior_offsets) return true;
-  if (prior_offsets[0] != 0) return false;
-  for (int i = 0; i < n; i++)
-    if (prior_offsets[i + 1] < prior_offsets[i]) return false;
-  return !(prior_offsets[n] > 0 && !priors);
-}
-
 int nicp_align(nicp_context *ctx, const nicp_cloud *reference, const nicp_cloud *current, const nicp_projector *proj,
                const nicp_align_params *ap, const float reference_sensor_offset[16], const float current_sensor_offset[16],
                const float initial_guess[16], const nicp_prior *priors, int num_priors, float frame_inlier_depth_threshold,

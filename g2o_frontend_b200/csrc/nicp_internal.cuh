@@ -348,6 +348,15 @@ struct nicp_context {
 };
 
 namespace nicp {
+// prior_offsets of a batch: n + 1 non-decreasing entries from 0 (or NULL: no priors)
+inline bool prior_offsets_valid(int n, const nicp_prior *priors, const int *prior_offsets) {
+  if (!prior_offsets) return true;
+  if (prior_offsets[0] != 0) return false;
+  for (int i = 0; i < n; i++)
+    if (prior_offsets[i + 1] < prior_offsets[i]) return false;
+  return !(prior_offsets[n] > 0 && !priors);
+}
+
 // frame_prep.cu
 int launch_depth_convert(nicp_context *ctx, const uint16_t *d_raw, int rows, int cols, float scale, int step,
                          float maxCov, float *d_out);

@@ -388,6 +388,27 @@ int nicp_multi_align_batch(nicp_context *ctx, int n, const nicp_cloud *const *re
                            const float current_sensor_offset[16], const float *initial_guesses,
                            const nicp_prior *priors, const int *prior_offsets,
                            float frame_inlier_depth_threshold, nicp_align_result *results);
+/* The rig counterpart of nicp_align_frames_sharded: raw rig frames in, records out, over the workers of a shard pool.
+ * raws[f * num_cameras + i] is camera i of frame f, raw_rows[i] x raw_cols[i] in every frame, as in
+ * nicp_multi_raw_depth_to_cloud_batch; pair i = (reference_frame[i], current_frame[i]) with initial_guesses + 16 i (NULL:
+ * identity) and priors as in nicp_multi_align_batch (priors / prior_offsets may be NULL); sensor_offset is the rig pose
+ * used for the frame preparation and for both sides of every alignment.  Worker g takes pairs [g n / G, (g + 1) n / G)
+ * and walks them in windows: the longest runs of consecutive pairs whose distinct frames fit in its frame cap, building
+ * only the frames a window needs and does not hold yet (in current-major order the candidates stay resident and only the
+ * current frames rotate).  The cap is max(2, 0.5 * device memory / (112 B * composite pixels) / workers on that device),
+ * about 160 frames at 1280 x 3840 on a 180 GB GPU; NICP_SHARD_FRAMES, read when the pool is created, lowers it.  Rig
+ * clouds are cached per worker apart from the pinhole ones, so rig calls leave nicp_align_frames_sharded as it was.
+ * Record i is byte-identical to nicp_multi_align on the clouds nicp_multi_raw_depth_to_cloud_batch builds from its two
+ * frames, whatever the device list, the workers per device or the cap.  Arguments are checked before any worker starts
+ * (frame indices, null images, raw sizes, prior_offsets); synchronous. */
+int nicp_multi_align_frames_sharded(nicp_shard_pool *pool, int n_frames, const uint16_t *const *raws, const int *raw_rows,
+                                    const int *raw_cols, float depth_scale, int step, float max_depth_cov,
+                                    const nicp_multi_projector *mp, const nicp_stats_params *sp,
+                                    const float sensor_offset[16], int n_pairs, const int *reference_frame,
+                                    const int *current_frame, const float *initial_guesses,
+                                    const nicp_prior *priors, const int *prior_offsets,
+                                    const nicp_align_params *ap, float frame_inlier_depth_threshold,
+                                    nicp_align_result *results);
 
 #ifdef __cplusplus
 }
