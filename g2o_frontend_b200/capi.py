@@ -159,6 +159,37 @@ def _iptr(a):
     return a.ctypes.data_as(C.POINTER(C.c_int))
 
 
+def _guesses(guesses, n):
+    """n (4, 4) poses -> pointer to n x 16 column-major floats (the pointer keeps the array alive); None -> NULL (identity)"""
+    if guesses is None:
+        return None
+    return _fptr(np.ascontiguousarray(np.asarray(guesses, np.float32).transpose(0, 2, 1)).reshape(n, 16))
+
+
+def _priors(priors, n):
+    """None or n lists of Prior -> (priors, prior_offsets) arguments: pair i owns priors[offs[i] .. offs[i + 1])"""
+    if priors is None:
+        return None, None
+    assert len(priors) == n
+    flat = [p for ps in priors for p in ps]
+    offs = np.zeros(n + 1, np.int32)
+    offs[1:] = np.cumsum([len(ps) for ps in priors])
+    return (Prior * max(len(flat), 1))(*flat), _iptr(offs)
+
+
+def _rig_frames(frames, nc):
+    """n rig frames of nc raw uint16 images each -> (the n * nc images, frame-major, as C-contiguous arrays, raw_rows,
+    raw_cols); camera i must have the same shape in every frame"""
+    imgs = []
+    for fr in frames:
+        assert len(fr) == nc, "a frame needs one raw image per camera"
+        imgs += [np.ascontiguousarray(r, np.uint16) for r in fr]
+    shapes = [im.shape for im in imgs[:nc]] if imgs else [(0, 0)] * nc
+    for k, im in enumerate(imgs):
+        assert im.shape == shapes[k % nc], "camera %d has a different raw size in frame %d" % (k % nc, k // nc)
+    return imgs, np.array([s[0] for s in shapes], np.int32), np.array([s[1] for s in shapes], np.int32)
+
+
 def make_projector(K, rows, cols, min_distance=0.01, max_distance=6.0):
     p = Projector()
     p.K[:] = colmajor(K).tolist()
@@ -564,17 +595,8 @@ class Context:
         """n rig frames -> n clouds (nicp_multi_raw_depth_to_cloud_batch).  frames: n sequences of mp.num_cameras raw uint16
         images in sensor orientation (camera i: (height_i * step) x (width_i * step), the same shape in every frame), numpy
         arrays or numpy views of pinned buffers.  Asynchronous like raw_depth_to_cloud_batch."""
-        n, nc = len(frames), mp.num_cameras
-        imgs = []
-        for fr in frames:
-            assert len(fr) == nc, "a frame needs one raw image per camera"
-            imgs += [r if (isinstance(r, np.ndarray) and r.dtype == np.uint16 and r.flags.c_contiguous)
-                     else np.ascontiguousarray(r, np.uint16) for r in fr]
-        shapes = [imgs[i].shape for i in range(nc)] if n else []
-        for k, im in enumerate(imgs):
-            assert im.shape == shapes[k % nc], "camera %d has a different raw size in frame %d" % (k % nc, k // nc)
-        rr = np.array([s[0] for s in shapes] or [0], np.int32)
-        rc = np.array([s[1] for s in shapes] or [0], np.int32)
+        n = len(frames)
+        imgs, rr, rc = _rig_frames(frames, mp.num_cameras)
         rows, cols = multi_image_size(mp, self.verify)
         clouds = clouds or [self.new_cloud(rows * cols) for _ in range(n)]
         so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
@@ -595,25 +617,14 @@ class Context:
         eye = np.eye(4, dtype=np.float32)
         ro = colmajor(eye if ref_offset is None else ref_offset)
         co = colmajor(eye if cur_offset is None else cur_offset)
-        if guesses is None:
-            g = np.tile(colmajor(eye), (n, 1))
-        else:
-            g = np.asarray(guesses, np.float32).transpose(0, 2, 1).reshape(n, 16)
-        g = np.ascontiguousarray(g, np.float32)
         RA = (C.c_void_p * max(n, 1))(*[r.handle for r in refs])
         CA = (C.c_void_p * max(n, 1))(*[c.handle for c in curs])
         if results is None:
             results = np.zeros(n, RESULT_DTYPE)
-        parr, offs = None, None
-        if priors is not None:
-            assert len(priors) == n
-            flat = [p for ps in priors for p in ps]
-            offs = np.zeros(n + 1, np.int32)
-            offs[1:] = np.cumsum([len(ps) for ps in priors])
-            parr = (Prior * max(len(flat), 1))(*flat)
+        parr, offs = _priors(priors, n)
         _check(self.L, self.L.nicp_multi_align_batch(self.handle, n, RA, CA, C.byref(mp), C.byref(ap), _fptr(ro), _fptr(co),
-                                                     _fptr(g), parr, None if offs is None else _iptr(offs),
-                                                     C.c_float(img_threshold), results.ctypes.data_as(C.POINTER(AlignResult))))
+                                                     _guesses(guesses, n), parr, offs, C.c_float(img_threshold),
+                                                     results.ctypes.data_as(C.POINTER(AlignResult))))
         return results
 
     def align_state(self, rows, cols, max_corr=None):
@@ -644,28 +655,14 @@ class Context:
         eye = np.eye(4, dtype=np.float32)
         ro = colmajor(eye if ref_offset is None else ref_offset)
         co = colmajor(eye if cur_offset is None else cur_offset)
-        if guesses is None:
-            g = np.tile(colmajor(eye), (n, 1))
-        else:
-            g = np.ascontiguousarray(np.asarray(guesses, np.float32).transpose(0, 2, 1)).reshape(n, 16)
-        g = np.ascontiguousarray(g, np.float32)
         RA = (C.c_void_p * n)(*[r.handle for r in refs])
         CA = (C.c_void_p * n)(*[c.handle for c in curs])
         if results is None:
             results = np.zeros(n, RESULT_DTYPE)
-        if priors is not None:
-            assert len(priors) == n
-            flat = [p for ps in priors for p in ps]
-            offs = np.zeros(n + 1, np.int32)
-            offs[1:] = np.cumsum([len(ps) for ps in priors])
-            parr = (Prior * max(len(flat), 1))(*flat)
-            _check(self.L, self.L.nicp_align_batch_priors(self.handle, n, RA, CA, C.byref(proj), C.byref(ap), _fptr(ro),
-                                                          _fptr(co), _fptr(g), parr, _iptr(offs), C.c_float(img_threshold),
-                                                          results.ctypes.data_as(C.POINTER(AlignResult))))
-            return results
-        _check(self.L, self.L.nicp_align_batch(self.handle, n, RA, CA, C.byref(proj), C.byref(ap), _fptr(ro), _fptr(co),
-                                               _fptr(g), C.c_float(img_threshold),
-                                               results.ctypes.data_as(C.POINTER(AlignResult))))
+        parr, offs = _priors(priors, n)
+        _check(self.L, self.L.nicp_align_batch_priors(self.handle, n, RA, CA, C.byref(proj), C.byref(ap), _fptr(ro), _fptr(co),
+                                                      _guesses(guesses, n), parr, offs, C.c_float(img_threshold),
+                                                      results.ctypes.data_as(C.POINTER(AlignResult))))
         return results
 
 
@@ -709,12 +706,12 @@ class ShardPool:
         RA = (C.c_void_p * len(frames))(*[f.ctypes.data for f in frames])
         rf = np.ascontiguousarray(ref_frame, np.int32)
         cf = np.ascontiguousarray(cur_frame, np.int32)
-        g = np.ascontiguousarray(np.asarray(guesses, np.float32).transpose(0, 2, 1)).reshape(n, 16)
         so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
         results = np.zeros(n, RESULT_DTYPE)
         _check(self.L, self.L.nicp_align_frames_sharded(self.handle, len(frames), RA, rows, cols, C.c_float(depth_scale), int(step),
                                                         C.c_float(max_depth_cov), C.byref(proj), C.byref(sp), _fptr(so), n,
-                                                        _iptr(rf), _iptr(cf), _fptr(g), C.byref(ap), C.c_float(img_threshold),
+                                                        _iptr(rf), _iptr(cf), _guesses(guesses, n), C.byref(ap),
+                                                        C.c_float(img_threshold),
                                                         results.ctypes.data_as(C.POINTER(AlignResult))))
         return results
 
@@ -723,39 +720,19 @@ class ShardPool:
         """rig frames in, records out (nicp_multi_align_frames_sharded).  frames: n sequences of mp.num_cameras raw uint16
         images, as in Context.multi_raw_depth_to_cloud_batch; pair i = (ref_frame[i], cur_frame[i]) with guesses[i] (None:
         identity); priors: None or one list of Prior per pair.  Returns RESULT_DTYPE records."""
-        nc = mp.num_cameras
-        imgs = []
-        for fr in frames:
-            assert len(fr) == nc, "a frame needs one raw image per camera"
-            imgs += [r if (isinstance(r, np.ndarray) and r.dtype == np.uint16 and r.flags.c_contiguous)
-                     else np.ascontiguousarray(r, np.uint16) for r in fr]
-        shapes = [imgs[i].shape for i in range(nc)] if frames else [(0, 0)] * nc
-        for k, im in enumerate(imgs):
-            assert im.shape == shapes[k % nc], "camera %d has a different raw size in frame %d" % (k % nc, k // nc)
-        rr = np.array([s[0] for s in shapes], np.int32)
-        rc = np.array([s[1] for s in shapes], np.int32)
+        imgs, rr, rc = _rig_frames(frames, mp.num_cameras)
         n = len(ref_frame)
         assert len(cur_frame) == n
         RA = (C.c_void_p * max(len(imgs), 1))(*[im.ctypes.data for im in imgs])
         rf = np.ascontiguousarray(ref_frame, np.int32)
         cf = np.ascontiguousarray(cur_frame, np.int32)
-        g = None
-        if guesses is not None:
-            g = np.ascontiguousarray(np.asarray(guesses, np.float32).transpose(0, 2, 1)).reshape(n, 16)
         so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
-        parr, offs = None, None
-        if priors is not None:
-            assert len(priors) == n
-            flat = [p for ps in priors for p in ps]
-            offs = np.zeros(n + 1, np.int32)
-            offs[1:] = np.cumsum([len(ps) for ps in priors])
-            parr = (Prior * max(len(flat), 1))(*flat)
+        parr, offs = _priors(priors, n)
         results = np.zeros(n, RESULT_DTYPE)
         _check(self.L, self.L.nicp_multi_align_frames_sharded(
             self.handle, len(frames), RA, _iptr(rr), _iptr(rc), C.c_float(depth_scale), int(step), C.c_float(max_depth_cov),
-            C.byref(mp), C.byref(sp), _fptr(so), n, _iptr(rf), _iptr(cf), None if g is None else _fptr(g), parr,
-            None if offs is None else _iptr(offs), C.byref(ap), C.c_float(img_threshold),
-            results.ctypes.data_as(C.POINTER(AlignResult))))
+            C.byref(mp), C.byref(sp), _fptr(so), n, _iptr(rf), _iptr(cf), _guesses(guesses, n), parr, offs, C.byref(ap),
+            C.c_float(img_threshold), results.ctypes.data_as(C.POINTER(AlignResult))))
         return results
 
     def close(self):

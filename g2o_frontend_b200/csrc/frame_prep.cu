@@ -758,11 +758,13 @@ int launch_frame_prep(nicp_context *ctx, const float *d_depth, const nicp_projec
   return NICP_OK;
 }
 
-// n raw 16-bit frames already on the device (d_raw[f]) -> n clouds: depth conversion + the launch set above, in
-// sub-batches of at most kMaxPrepBatch frames whose scratch (depth + integral image, 44 B/pixel/frame) stays L2 resident
-int launch_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw, int rawRows, int rawCols, float scale, int step,
-                          float maxCov, const nicp_projector *proj, const nicp_stats_params *sp, const float sensorOffset[16],
-                          int keepStats, nicp_cloud *const *clouds) {
+// n raw 16-bit frames of fs already on the device (d_raw[f * fs.cams.n + i] = camera i of frame f) -> n clouds: one depth
+// conversion launch for every camera of every frame, then the launch set above.  n <= kMaxPrepBatch frames, whose scratch
+// (depth + integral image, 44 B/pixel/frame) stays L2 resident.
+int launch_raw_prep_batch(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *d_raw,
+                          const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds) {
+  const nicp_projector *proj = &fs.proj;
+  const CamSet &cams = fs.cams;
   const size_t px = (size_t)proj->rows * proj->cols;
   if (n > ctx->batchSlots || px > ctx->batchPixels) {
     set_error("internal: batch prep scratch too small");
@@ -770,49 +772,35 @@ int launch_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw
   }
   PrepBatch B;
   memset(&B, 0, sizeof B);
-  for (int f = 0; f < n; f++) {
+  for (int f = 0; f < n; f++)
     prep_batch_add(B, ctx->d_bDepth + (size_t)f * ctx->batchPixels, ctx->d_bIntegral + (size_t)f * ctx->batchPixels * kIntegralCh,
                    clouds[f], keepStats != 0);
-    B.raw[f] = d_raw[f];
+  if (cams.multi) {
+    // composite image: rows = max width, cols = sum of heights
+    RigFrames R;
+    memset(&R, 0, sizeof R);
+    R.nCams = cams.n;
+    int maxHeight = 0;
+    for (int i = 0; i < cams.n; i++) {
+      R.rawRows[i] = fs.rawRows[i];
+      R.rawCols[i] = fs.rawCols[i];
+      R.width[i] = cams.width[i];
+      R.height[i] = cams.height[i];
+      R.colOff[i] = cams.colOff[i];
+      if (cams.height[i] > maxHeight) maxHeight = cams.height[i];
+    }
+    for (int f = 0; f < n; f++) {
+      R.depth[f] = B.depth[f];
+      for (int i = 0; i < cams.n; i++) R.raw[f * cams.n + i] = d_raw[f * cams.n + i];
+    }
+    k_rig_depth_convert<<<dim3((maxHeight + 31) / 32, (proj->rows + 31) / 32, n * cams.n), dim3(32, 8), 0, ctx->stream>>>(
+        R, proj->rows, proj->cols, fs.depthScale, fs.step, fs.maxDepthCov);
+  } else {
+    for (int f = 0; f < n; f++) B.raw[f] = d_raw[f];
+    const int outPx = (fs.rawRows[0] / fs.step) * (fs.rawCols[0] / fs.step);
+    k_depth_convert<<<dim3((outPx + 255) / 256, n), 256, 0, ctx->stream>>>(B, fs.rawRows[0], fs.rawCols[0], fs.depthScale,
+                                                                           fs.step, fs.maxDepthCov);
   }
-  const int outPx = (rawRows / step) * (rawCols / step);
-  k_depth_convert<<<dim3((outPx + 255) / 256, n), 256, 0, ctx->stream>>>(B, rawRows, rawCols, scale, step, maxCov);
-  NICP_CHECK_LAUNCH(ctx);
-  return launch_prep_set(ctx, B, proj, sp, sensorOffset, nullptr, nullptr, nullptr);
-}
-
-// the same for n rig frames: d_raw[f * cams.n + i] = camera i of frame f on the device (rawRows[i] x rawCols[i]), proj = the
-// composite image (rows = max width, cols = sum of heights); one conversion launch for every camera of every frame
-int launch_rig_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw, const int *rawRows, const int *rawCols,
-                              float scale, int step, float maxCov, const nicp_projector *proj, const CamSet &cams,
-                              const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds) {
-  const size_t px = (size_t)proj->rows * proj->cols;
-  if (n > ctx->batchSlots || px > ctx->batchPixels) {
-    set_error("internal: batch prep scratch too small");
-    return NICP_ERR_INVALID;
-  }
-  PrepBatch B;
-  memset(&B, 0, sizeof B);
-  RigFrames R;
-  memset(&R, 0, sizeof R);
-  R.nCams = cams.n;
-  int maxHeight = 0;
-  for (int i = 0; i < cams.n; i++) {
-    R.rawRows[i] = rawRows[i];
-    R.rawCols[i] = rawCols[i];
-    R.width[i] = cams.width[i];
-    R.height[i] = cams.height[i];
-    R.colOff[i] = cams.colOff[i];
-    if (cams.height[i] > maxHeight) maxHeight = cams.height[i];
-  }
-  for (int f = 0; f < n; f++) {
-    prep_batch_add(B, ctx->d_bDepth + (size_t)f * ctx->batchPixels, ctx->d_bIntegral + (size_t)f * ctx->batchPixels * kIntegralCh,
-                   clouds[f], keepStats != 0);
-    R.depth[f] = B.depth[f];
-    for (int i = 0; i < cams.n; i++) R.raw[f * cams.n + i] = d_raw[f * cams.n + i];
-  }
-  k_rig_depth_convert<<<dim3((maxHeight + 31) / 32, (proj->rows + 31) / 32, n * cams.n), dim3(32, 8), 0, ctx->stream>>>(
-      R, proj->rows, proj->cols, scale, step, maxCov);
   NICP_CHECK_LAUNCH(ctx);
   return launch_prep_set(ctx, B, proj, sp, sensorOffset, nullptr, nullptr, &cams);
 }

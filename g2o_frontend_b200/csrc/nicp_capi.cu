@@ -226,7 +226,7 @@ static CamSet camset_pinhole(const nicp_projector *proj) {
 static int camset_multi(const nicp_multi_projector *mp, CamSet &c, int &rows, int &cols) {
   memset(&c, 0, sizeof c);
   if (!mp || mp->num_cameras < 1 || mp->num_cameras > kMaxCams) {
-    set_error("multi projector needs 1..%d cameras", kMaxCams);
+    set_error("multi projector needs 1..%d cameras of positive size", kMaxCams);
     return NICP_ERR_INVALID;
   }
   c.n = mp->num_cameras;
@@ -236,7 +236,10 @@ static int camset_multi(const nicp_multi_projector *mp, CamSet &c, int &rows, in
   for (int i = 0; i < c.n; i++) {
     c.width[i] = mp->camera[i].rows;
     c.height[i] = mp->camera[i].cols;
-    if (c.width[i] <= 0 || c.height[i] <= 0) return NICP_ERR_INVALID;
+    if (c.width[i] <= 0 || c.height[i] <= 0) {
+      set_error("multi projector needs 1..%d cameras of positive size", kMaxCams);
+      return NICP_ERR_INVALID;
+    }
     c.colOff[i] = cols;
     cols += c.height[i];
     if (c.width[i] > rows) rows = c.width[i];
@@ -251,6 +254,142 @@ static int camset_multi(const nicp_multi_projector *mp, CamSet &c, int &rows, in
 static int upload_cams(nicp_context *ctx, const CamSet &c) {
   ctx->h_cams = c;
   NICP_CUDA(cudaMemcpyAsync(&ctx->d_cams->set, &ctx->h_cams, sizeof(CamSet), cudaMemcpyHostToDevice, ctx->stream));
+  return NICP_OK;
+}
+
+// ---- frame sets: the raw frames of the batched prep and of the sharded closer ------------------------------------------
+int frames_pinhole(const nicp_projector *proj, int rawRows, int rawCols, float depthScale, int step, float maxDepthCov,
+                   FrameSet &fs) {
+  if (step < 1) step = 1;
+  if (proj->rows != rawRows / step || proj->cols != rawCols / step) {
+    set_error("projector image size %dx%d does not match the scaled raw image %dx%d", proj->rows, proj->cols,
+              rawRows / step, rawCols / step);
+    return NICP_ERR_INVALID;
+  }
+  memset(&fs, 0, sizeof fs);
+  fs.cams = camset_pinhole(proj);
+  fs.proj = *proj;
+  fs.rawRows[0] = rawRows;
+  fs.rawCols[0] = rawCols;
+  fs.rawPixels = (size_t)rawRows * rawCols;
+  fs.depthScale = depthScale;
+  fs.maxDepthCov = maxDepthCov;
+  fs.step = step;
+  fs.prepFrames = kMaxPrepBatch;
+  fs.slotCap = INT_MAX;
+  return NICP_OK;
+}
+
+// frames per launch set of a rig for a composite image of px pixels: a set's scratch (depth + integral image, 44 B per
+// pixel and frame) stays within that of a full pinhole set (kMaxPrepBatch frames of 640x480, 108 MB), at least one frame.
+// Frames are batched so that their row and column chains fill the GPU; a composite of 1280 x 3840 already brings 1280 row
+// passes and 38 400 column chains on its own, so it runs one frame per set (216 MB) instead of 1.7 GB for eight.
+static int rig_prep_frames(size_t px) {
+  const size_t f = (size_t)kMaxPrepBatch * 640 * 480 / px;
+  return f < 1 ? 1 : (f > (size_t)kMaxPrepBatch ? kMaxPrepBatch : (int)f);
+}
+
+// the camera set, composite projector and batching limits of a rig: a frame set without raw frames
+static int rig_geometry(const nicp_multi_projector *mp, FrameSet &fs) {
+  memset(&fs, 0, sizeof fs);
+  int rows, cols, rc;
+  if ((rc = camset_multi(mp, fs.cams, rows, cols))) return rc;
+  fs.proj = mp->camera[0];
+  fs.proj.rows = rows;
+  fs.proj.cols = cols;
+  const size_t px = (size_t)rows * cols;
+  fs.prepFrames = rig_prep_frames(px);
+  // a slot holds 32 B per pixel of z-buffers and index images: a chunk gets at most the memory of 256 pinhole 640x480 slots
+  // (2.5 GB; 16 slots at 1280x3840)
+  fs.slotCap = (int)std::max<size_t>(1, (size_t)256 * 640 * 480 / px);
+  return NICP_OK;
+}
+
+int frames_rig(const nicp_multi_projector *mp, const int *rawRows, const int *rawCols, float depthScale, int step,
+               float maxDepthCov, FrameSet &fs) {
+  if (!rawRows || !rawCols) return NICP_ERR_INVALID;
+  int rc;
+  if ((rc = rig_geometry(mp, fs))) return rc;
+  if (step < 1) step = 1;
+  const CamSet &c = fs.cams;
+  for (int i = 0; i < c.n; i++) {
+    if (rawRows[i] <= 0 || rawCols[i] <= 0 || rawRows[i] / step != c.height[i] || rawCols[i] / step != c.width[i]) {
+      set_error("camera %d: raw image %dx%d at step %d does not scale to the projector's %dx%d (rows x cols = height x width)",
+                i, rawRows[i], rawCols[i], step, c.height[i], c.width[i]);
+      return NICP_ERR_INVALID;
+    }
+    fs.rawRows[i] = rawRows[i];
+    fs.rawCols[i] = rawCols[i];
+    fs.rawPixels += (size_t)rawRows[i] * rawCols[i];
+  }
+  fs.depthScale = depthScale;
+  fs.maxDepthCov = maxDepthCov;
+  fs.step = step;
+  return NICP_OK;
+}
+
+// n raw frames of fs -> clouds[0 .. n), asynchronously: raws[f * fs.cams.n + i] = camera i of frame f
+int prep_frames(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *raws, const nicp_stats_params *sp,
+                const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds) {
+  if (!raws || !clouds) return NICP_ERR_INVALID;
+  const int nc = fs.cams.n;
+  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
+  for (int f = 0; f < n; f++) {
+    for (int i = 0; i < nc; i++)
+      if (!raws[(size_t)f * nc + i]) {
+        set_error("null raw image of camera %d in frame %d", i, f);
+        return NICP_ERR_INVALID;
+      }
+    if (!clouds[f]) {
+      set_error("null cloud at index %d", f);
+      return NICP_ERR_INVALID;
+    }
+    if ((size_t)clouds[f]->capacity < px) {
+      set_error("cloud %d: capacity %d smaller than the image (%zu pixels)", f, clouds[f]->capacity, px);
+      return NICP_ERR_INVALID;
+    }
+    if (clouds[f]->device != ctx->device) {
+      set_error("cloud %d lives on GPU %d, the context on GPU %d", f, clouds[f]->device, ctx->device);
+      return NICP_ERR_INVALID;
+    }
+    for (int j = 0; j < f; j++)
+      if (clouds[j] == clouds[f]) {
+        set_error("cloud %d and cloud %d are the same object", j, f);
+        return NICP_ERR_INVALID;
+      }
+  }
+  const int sub = std::min({env_int("NICP_PREP_BATCH", kMaxPrepBatch), fs.prepFrames, n});
+  int rc;
+  if ((rc = ensure_batch_prep(ctx, sub, px, fs.rawPixels))) return rc;
+  float eye[16];
+  mat4_identity(eye);
+  for (int base = 0; base < n; base += sub) {
+    const int m = n - base < sub ? n - base : sub;
+    // raw frames of sub-batch k are uploaded on the copy stream into staging set k & 1 while sub-batch k - 1 computes; the
+    // cameras of a frame sit back to back in its staging slot
+    const int b = (ctx->bRawToggle ^= 1);
+    uint16_t *stage = ctx->d_bRaw + (size_t)b * ctx->batchSlots * ctx->batchRawPixels;
+    const uint16_t *d_raw[kMaxPrepBatch * kMaxCams];
+    NICP_CUDA(cudaStreamWaitEvent(ctx->copyStream, ctx->evBRawUsed[b], 0));
+    for (int f = 0; f < m; f++) {
+      uint16_t *dst = stage + (size_t)f * ctx->batchRawPixels;
+      for (int i = 0; i < nc; i++) {
+        const size_t cpx = (size_t)fs.rawRows[i] * fs.rawCols[i];
+        NICP_CUDA(cudaMemcpyAsync(dst, raws[(size_t)(base + f) * nc + i], cpx * sizeof(uint16_t), cudaMemcpyHostToDevice,
+                                  ctx->copyStream));
+        d_raw[f * nc + i] = dst;
+        dst += cpx;
+      }
+    }
+    NICP_CUDA(cudaEventRecord(ctx->evBRawCopied[b], ctx->copyStream));
+    NICP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evBRawCopied[b], 0));
+    for (int f = 0; f < m; f++)
+      if (keepStats && (rc = ensure_stats(clouds[base + f]))) return rc;
+    if ((rc = launch_raw_prep_batch(ctx, fs, m, d_raw, sp, sensorOffset ? sensorOffset : eye, keepStats, clouds + base)))
+      return rc;
+    NICP_CUDA(cudaEventRecord(ctx->evBRawUsed[b], ctx->stream));
+  }
+  ctx->lastRows = 0;  // the single-frame test hooks (integral / interval image) describe no frame of a batch
   return NICP_OK;
 }
 
@@ -905,73 +1044,9 @@ int nicp_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *cons
   if (!ctx || n < 0 || !proj || !sp || raw_rows <= 0 || raw_cols <= 0) return NICP_ERR_INVALID;
   NICP_CUDA(cudaSetDevice(ctx->device));
   if (n == 0) return NICP_OK;
-  if (!raws || !clouds) return NICP_ERR_INVALID;
-  if (step < 1) step = 1;
-  if (proj->rows != raw_rows / step || proj->cols != raw_cols / step) {
-    set_error("projector image size %dx%d does not match the scaled raw image %dx%d", proj->rows, proj->cols,
-              raw_rows / step, raw_cols / step);
-    return NICP_ERR_INVALID;
-  }
-  const size_t rpx = (size_t)raw_rows * raw_cols, px = (size_t)proj->rows * proj->cols;
-  for (int i = 0; i < n; i++) {
-    if (!raws[i] || !clouds[i]) {
-      set_error("null frame or cloud at index %d", i);
-      return NICP_ERR_INVALID;
-    }
-    if ((size_t)clouds[i]->capacity < px) {
-      set_error("cloud %d: capacity %d smaller than the image (%zu pixels)", i, clouds[i]->capacity, px);
-      return NICP_ERR_INVALID;
-    }
-    if (clouds[i]->device != ctx->device) {
-      set_error("cloud %d lives on GPU %d, the context on GPU %d", i, clouds[i]->device, ctx->device);
-      return NICP_ERR_INVALID;
-    }
-    for (int j = 0; j < i; j++)
-      if (clouds[j] == clouds[i]) {
-        set_error("cloud %d and cloud %d are the same object", j, i);
-        return NICP_ERR_INVALID;
-      }
-  }
-  int sub = env_int("NICP_PREP_BATCH", kMaxPrepBatch);
-  if (sub > kMaxPrepBatch) sub = kMaxPrepBatch;
-  if (sub > n) sub = n;
-  int rc;
-  if ((rc = ensure_batch_prep(ctx, sub, px, rpx))) return rc;
-  float eye[16];
-  mat4_identity(eye);
-  for (int base = 0; base < n; base += sub) {
-    const int m = n - base < sub ? n - base : sub;
-    // raw frames of sub-batch k are uploaded on the copy stream into staging set k & 1 while sub-batch k - 1 computes
-    const int b = (ctx->bRawToggle ^= 1);
-    uint16_t *stage = ctx->d_bRaw + (size_t)b * ctx->batchSlots * ctx->batchRawPixels;
-    const uint16_t *d_raw[kMaxPrepBatch];
-    NICP_CUDA(cudaStreamWaitEvent(ctx->copyStream, ctx->evBRawUsed[b], 0));
-    for (int f = 0; f < m; f++) {
-      uint16_t *dst = stage + (size_t)f * ctx->batchRawPixels;
-      NICP_CUDA(cudaMemcpyAsync(dst, raws[base + f], rpx * sizeof(uint16_t), cudaMemcpyHostToDevice, ctx->copyStream));
-      d_raw[f] = dst;
-    }
-    NICP_CUDA(cudaEventRecord(ctx->evBRawCopied[b], ctx->copyStream));
-    NICP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evBRawCopied[b], 0));
-    for (int f = 0; f < m; f++)
-      if (keep_stats && (rc = ensure_stats(clouds[base + f]))) return rc;
-    if ((rc = launch_raw_prep_batch(ctx, m, d_raw, raw_rows, raw_cols, depth_scale, step, max_depth_cov, proj, sp,
-                                    sensor_offset ? sensor_offset : eye, keep_stats, clouds + base)))
-      return rc;
-    NICP_CUDA(cudaEventRecord(ctx->evBRawUsed[b], ctx->stream));
-  }
-  ctx->lastRows = 0;  // the single-frame test hooks (integral / interval image) describe no frame of a batch
-  return NICP_OK;
-}
-
-// frames per launch set of nicp_multi_raw_depth_to_cloud_batch for a composite image of px pixels: a set's scratch (depth +
-// integral image, 44 B per pixel and frame) stays within that of a full pinhole set (kMaxPrepBatch frames of 640x480,
-// 108 MB), at least one frame.  Frames are batched so that their row and column chains fill the GPU; a composite of
-// 1280 x 3840 already brings 1280 row passes and 38 400 column chains on its own, so it runs one frame per set (216 MB)
-// instead of 1.7 GB for eight.
-static int rig_prep_frames(size_t px) {
-  const size_t f = (size_t)kMaxPrepBatch * 640 * 480 / px;
-  return f < 1 ? 1 : (f > (size_t)kMaxPrepBatch ? kMaxPrepBatch : (int)f);
+  FrameSet fs;
+  int rc = frames_pinhole(proj, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs);
+  return rc ? rc : prep_frames(ctx, fs, n, raws, sp, sensor_offset, keep_stats, clouds);
 }
 
 int nicp_multi_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *const *raws, const int *raw_rows,
@@ -981,85 +1056,9 @@ int nicp_multi_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t
   if (!ctx || n < 0 || !mp || !sp) return NICP_ERR_INVALID;
   NICP_CUDA(cudaSetDevice(ctx->device));
   if (n == 0) return NICP_OK;
-  if (!raws || !clouds || !raw_rows || !raw_cols) return NICP_ERR_INVALID;
-  if (step < 1) step = 1;
-  CamSet cams;
-  int rows, cols, rc;
-  if ((rc = camset_multi(mp, cams, rows, cols))) return rc;
-  const int nc = cams.n;
-  size_t rpx = 0;
-  for (int i = 0; i < nc; i++) {
-    if (raw_rows[i] <= 0 || raw_cols[i] <= 0 || raw_rows[i] / step != cams.height[i] || raw_cols[i] / step != cams.width[i]) {
-      set_error("camera %d: raw image %dx%d at step %d does not scale to the projector's %dx%d (rows x cols = height x width)",
-                i, raw_rows[i], raw_cols[i], step, cams.height[i], cams.width[i]);
-      return NICP_ERR_INVALID;
-    }
-    rpx += (size_t)raw_rows[i] * raw_cols[i];
-  }
-  const size_t px = (size_t)rows * cols;
-  for (int f = 0; f < n; f++) {
-    for (int i = 0; i < nc; i++)
-      if (!raws[f * nc + i]) {
-        set_error("null raw image of camera %d in frame %d", i, f);
-        return NICP_ERR_INVALID;
-      }
-    if (!clouds[f]) {
-      set_error("null cloud at index %d", f);
-      return NICP_ERR_INVALID;
-    }
-    if ((size_t)clouds[f]->capacity < px) {
-      set_error("cloud %d: capacity %d smaller than the composite image (%zu pixels)", f, clouds[f]->capacity, px);
-      return NICP_ERR_INVALID;
-    }
-    if (clouds[f]->device != ctx->device) {
-      set_error("cloud %d lives on GPU %d, the context on GPU %d", f, clouds[f]->device, ctx->device);
-      return NICP_ERR_INVALID;
-    }
-    for (int j = 0; j < f; j++)
-      if (clouds[j] == clouds[f]) {
-        set_error("cloud %d and cloud %d are the same object", j, f);
-        return NICP_ERR_INVALID;
-      }
-  }
-  int sub = env_int("NICP_PREP_BATCH", kMaxPrepBatch);
-  if (sub > rig_prep_frames(px)) sub = rig_prep_frames(px);
-  if (sub < 1) sub = 1;
-  if (sub > n) sub = n;
-  if ((rc = ensure_batch_prep(ctx, sub, px, rpx))) return rc;
-  float eye[16];
-  mat4_identity(eye);
-  for (int base = 0; base < n; base += sub) {
-    const int m = n - base < sub ? n - base : sub;
-    // as in nicp_raw_depth_to_cloud_batch: sub-batch k is uploaded into staging set k & 1 while sub-batch k - 1 computes;
-    // the cameras of a frame sit back to back in its staging slot
-    const int b = (ctx->bRawToggle ^= 1);
-    uint16_t *stage = ctx->d_bRaw + (size_t)b * ctx->batchSlots * ctx->batchRawPixels;
-    const uint16_t *d_raw[kMaxPrepBatch * kMaxCams];
-    NICP_CUDA(cudaStreamWaitEvent(ctx->copyStream, ctx->evBRawUsed[b], 0));
-    for (int f = 0; f < m; f++) {
-      uint16_t *dst = stage + (size_t)f * ctx->batchRawPixels;
-      for (int i = 0; i < nc; i++) {
-        const size_t cpx = (size_t)raw_rows[i] * raw_cols[i];
-        NICP_CUDA(cudaMemcpyAsync(dst, raws[(size_t)(base + f) * nc + i], cpx * sizeof(uint16_t), cudaMemcpyHostToDevice,
-                                  ctx->copyStream));
-        d_raw[f * nc + i] = dst;
-        dst += cpx;
-      }
-    }
-    NICP_CUDA(cudaEventRecord(ctx->evBRawCopied[b], ctx->copyStream));
-    NICP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evBRawCopied[b], 0));
-    for (int f = 0; f < m; f++)
-      if (keep_stats && (rc = ensure_stats(clouds[base + f]))) return rc;
-    nicp_projector proj = mp->camera[0];
-    proj.rows = rows;
-    proj.cols = cols;
-    if ((rc = launch_rig_raw_prep_batch(ctx, m, d_raw, raw_rows, raw_cols, depth_scale, step, max_depth_cov, &proj, cams, sp,
-                                        sensor_offset ? sensor_offset : eye, keep_stats, clouds + base)))
-      return rc;
-    NICP_CUDA(cudaEventRecord(ctx->evBRawUsed[b], ctx->stream));
-  }
-  ctx->lastRows = 0;
-  return NICP_OK;
+  FrameSet fs;
+  int rc = frames_rig(mp, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs);
+  return rc ? rc : prep_frames(ctx, fs, n, raws, sp, sensor_offset, keep_stats, clouds);
 }
 
 // ---- stage-level statistics / information matrices (host buffers in, host buffers out) -----------------------------
@@ -1471,6 +1470,19 @@ static int align_common(nicp_context *ctx, int n, const nicp_cloud *const *refs,
   return NICP_OK;
 }
 
+}  // extern "C"
+
+// a batch of pairs of clouds built from the frames of fs (nicp_multi_align_batch, and the align step of a sharded worker)
+int nicp::align_frame_pairs(nicp_context *ctx, const FrameSet &fs, int n, const nicp_cloud *const *refs,
+                            const nicp_cloud *const *curs, const nicp_align_params *ap, const float refOffset[16],
+                            const float curOffset[16], const float *guesses, const nicp_prior *priors,
+                            const int *priorOffsets, float imgThr, nicp_align_result *results) {
+  return align_common(ctx, n, refs, curs, &fs.proj, ap, refOffset, curOffset, guesses, imgThr, results, false, priors, 0,
+                      &fs.cams, priorOffsets, fs.slotCap);
+}
+
+extern "C" {
+
 int nicp_align(nicp_context *ctx, const nicp_cloud *reference, const nicp_cloud *current, const nicp_projector *proj,
                const nicp_align_params *ap, const float reference_sensor_offset[16], const float current_sensor_offset[16],
                const float initial_guess[16], const nicp_prior *priors, int num_priors, float frame_inlier_depth_threshold,
@@ -1486,12 +1498,8 @@ int nicp_align_batch(nicp_context *ctx, int n, const nicp_cloud *const *referenc
                      const nicp_projector *proj, const nicp_align_params *ap, const float reference_sensor_offset[16],
                      const float current_sensor_offset[16], const float *initial_guesses, float frame_inlier_depth_threshold,
                      nicp_align_result *results) {
-  if (!ctx || n < 0 || !proj || !ap || proj->rows <= 0 || proj->cols <= 0) return NICP_ERR_INVALID;
-  NICP_CUDA(cudaSetDevice(ctx->device));
-  if (n == 0) return NICP_OK;
-  if (!references || !currents || !results) return NICP_ERR_INVALID;
-  return align_common(ctx, n, references, currents, proj, ap, reference_sensor_offset, current_sensor_offset, initial_guesses,
-                      frame_inlier_depth_threshold, results, false);
+  return nicp_align_batch_priors(ctx, n, references, currents, proj, ap, reference_sensor_offset, current_sensor_offset,
+                                 initial_guesses, nullptr, nullptr, frame_inlier_depth_threshold, results);
 }
 
 int nicp_align_batch_priors(nicp_context *ctx, int n, const nicp_cloud *const *references, const nicp_cloud *const *currents,
@@ -1502,7 +1510,8 @@ int nicp_align_batch_priors(nicp_context *ctx, int n, const nicp_cloud *const *r
   NICP_CUDA(cudaSetDevice(ctx->device));
   if (n == 0) return NICP_OK;
   if (!references || !currents || !results) return NICP_ERR_INVALID;
-  if (!prior_offsets_valid(n, priors, prior_offsets)) return NICP_ERR_INVALID;
+  int rc;
+  if ((rc = check_prior_offsets(n, priors, prior_offsets))) return rc;
   return align_common(ctx, n, references, currents, proj, ap, reference_sensor_offset, current_sensor_offset, initial_guesses,
                       frame_inlier_depth_threshold, results, false, priors, 0, nullptr, prior_offsets);
 }
@@ -1519,25 +1528,22 @@ int nicp_multi_depth_to_cloud(nicp_context *ctx, const float *depth, const nicp_
                               const float sensor_offset[16], int keep_stats, nicp_cloud *cloud, int *index) {
   if (!ctx || !depth || !mp || !sp || !cloud) return NICP_ERR_INVALID;
   NICP_CUDA(cudaSetDevice(ctx->device));
-  CamSet cams;
-  int rows, cols, rc;
-  if ((rc = camset_multi(mp, cams, rows, cols))) return rc;
-  size_t px = (size_t)rows * cols;
+  FrameSet fs;
+  int rc;
+  if ((rc = rig_geometry(mp, fs))) return rc;
+  size_t px = (size_t)fs.proj.rows * fs.proj.cols;
   if ((size_t)cloud->capacity < px) {
     set_error("cloud capacity %d smaller than the composite image (%zu pixels)", cloud->capacity, px);
     return NICP_ERR_INVALID;
   }
   if ((rc = ensure_prep(ctx, px))) return rc;
-  if ((rc = upload_cams(ctx, cams))) return rc;
+  if ((rc = upload_cams(ctx, fs.cams))) return rc;
   if (keep_stats && (rc = ensure_stats(cloud))) return rc;
   NICP_CUDA(cudaMemcpyAsync(ctx->d_depth, depth, px * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-  nicp_projector proj = mp->camera[0];
-  proj.rows = rows;
-  proj.cols = cols;
   float eye[16];
   mat4_identity(eye);
-  if ((rc = launch_frame_prep(ctx, ctx->d_depth, &proj, sp, sensor_offset ? sensor_offset : eye, keep_stats, cloud,
-                              ctx->d_index, &cams)))
+  if ((rc = launch_frame_prep(ctx, ctx->d_depth, &fs.proj, sp, sensor_offset ? sensor_offset : eye, keep_stats, cloud,
+                              ctx->d_index, &fs.cams)))
     return rc;
   if (index) NICP_CUDA(cudaMemcpyAsync(index, ctx->d_index, px * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   NICP_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1574,14 +1580,11 @@ int nicp_multi_align(nicp_context *ctx, const nicp_cloud *reference, const nicp_
   if (!ctx || !reference || !current || !mp || !ap || !result) return NICP_ERR_INVALID;
   NICP_CUDA(cudaSetDevice(ctx->device));
   if (num_priors < 0 || (num_priors > 0 && !priors)) return NICP_ERR_INVALID;
-  CamSet cams;
-  int rows, cols, rc;
-  if ((rc = camset_multi(mp, cams, rows, cols))) return rc;
-  nicp_projector proj = mp->camera[0];
-  proj.rows = rows;
-  proj.cols = cols;
-  return align_common(ctx, 1, &reference, &current, &proj, ap, reference_sensor_offset, current_sensor_offset, initial_guess,
-                      frame_inlier_depth_threshold, result, true, priors, num_priors, &cams);
+  FrameSet fs;
+  int rc;
+  if ((rc = rig_geometry(mp, fs))) return rc;
+  return align_common(ctx, 1, &reference, &current, &fs.proj, ap, reference_sensor_offset, current_sensor_offset,
+                      initial_guess, frame_inlier_depth_threshold, result, true, priors, num_priors, &fs.cams);
 }
 
 int nicp_multi_align_batch(nicp_context *ctx, int n, const nicp_cloud *const *references, const nicp_cloud *const *currents,
@@ -1592,19 +1595,11 @@ int nicp_multi_align_batch(nicp_context *ctx, int n, const nicp_cloud *const *re
   NICP_CUDA(cudaSetDevice(ctx->device));
   if (n == 0) return NICP_OK;
   if (!references || !currents || !results) return NICP_ERR_INVALID;
-  if (!prior_offsets_valid(n, priors, prior_offsets)) return NICP_ERR_INVALID;
-  CamSet cams;
-  int rows, cols, rc;
-  if ((rc = camset_multi(mp, cams, rows, cols))) return rc;
-  nicp_projector proj = mp->camera[0];
-  proj.rows = rows;
-  proj.cols = cols;
-  // a slot holds 32 B per pixel of z-buffers and index images: a chunk gets at most the memory of 256 pinhole 640x480 slots
-  // (2.5 GB; 16 slots at 1280x3840)
-  const size_t P = (size_t)rows * cols;
-  const int slotCap = (int)std::max<size_t>(1, (size_t)256 * 640 * 480 / P);
-  return align_common(ctx, n, references, currents, &proj, ap, reference_sensor_offset, current_sensor_offset, initial_guesses,
-                      frame_inlier_depth_threshold, results, false, priors, 0, &cams, prior_offsets, slotCap);
+  FrameSet fs;
+  int rc;
+  if ((rc = check_prior_offsets(n, priors, prior_offsets)) || (rc = rig_geometry(mp, fs))) return rc;
+  return align_frame_pairs(ctx, fs, n, references, currents, ap, reference_sensor_offset, current_sensor_offset,
+                           initial_guesses, priors, prior_offsets, frame_inlier_depth_threshold, results);
 }
 
 int nicp_align_get_state(nicp_context *ctx, int *reference_index, float *reference_depth, int *current_index,

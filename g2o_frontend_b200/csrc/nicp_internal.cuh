@@ -207,6 +207,20 @@ struct DeviceCams {
   PrepCams prep;
 };
 
+// The raw frames of a batched prep or a sharded call and how they become clouds.  A pinhole camera is a set of one camera
+// (cams.multi == 0), a MultiPointProjector rig a set of its children; frames_pinhole / frames_rig (nicp_capi.cu) fill it and
+// validate the raw sizes.
+struct FrameSet {
+  CamSet cams;
+  nicp_projector proj;                       // the image the clouds are built in: the pinhole's or the rig's composite
+  int rawRows[kMaxCams], rawCols[kMaxCams];  // raw image of camera i, as the sensor delivers it
+  size_t rawPixels;                          // raw pixels of one frame, every camera
+  float depthScale, maxDepthCov;
+  int step;                                  // DepthImage_scale factor, >= 1
+  int prepFrames;                            // frames per launch set of the batched prep (NICP_PREP_BATCH can lower it)
+  int slotCap;                               // pairs per lock-step align chunk (NICP_BATCH_SLOTS can lower it)
+};
+
 struct AlignConsts {
   float K[9];
   float refOffset[16];
@@ -348,27 +362,45 @@ struct nicp_context {
 };
 
 namespace nicp {
-// prior_offsets of a batch: n + 1 non-decreasing entries from 0 (or NULL: no priors)
-inline bool prior_offsets_valid(int n, const nicp_prior *priors, const int *prior_offsets) {
-  if (!prior_offsets) return true;
-  if (prior_offsets[0] != 0) return false;
+// prior_offsets of a batch: n + 1 non-decreasing entries from 0 (or NULL: no priors); a bad array is reported by its first
+// bad entry
+inline int check_prior_offsets(int n, const nicp_prior *priors, const int *prior_offsets) {
+  if (!prior_offsets) return NICP_OK;
+  if (prior_offsets[0] != 0) {
+    set_error("prior_offsets[0] is %d, not 0", prior_offsets[0]);
+    return NICP_ERR_INVALID;
+  }
   for (int i = 0; i < n; i++)
-    if (prior_offsets[i + 1] < prior_offsets[i]) return false;
-  return !(prior_offsets[n] > 0 && !priors);
+    if (prior_offsets[i + 1] < prior_offsets[i]) {
+      set_error("prior_offsets decrease at pair %d (%d -> %d)", i, prior_offsets[i], prior_offsets[i + 1]);
+      return NICP_ERR_INVALID;
+    }
+  if (prior_offsets[n] > 0 && !priors) {
+    set_error("prior_offsets name %d priors but priors is null", prior_offsets[n]);
+    return NICP_ERR_INVALID;
+  }
+  return NICP_OK;
 }
 
+// nicp_capi.cu
+int frames_pinhole(const nicp_projector *proj, int rawRows, int rawCols, float depthScale, int step, float maxDepthCov,
+                   FrameSet &fs);
+int frames_rig(const nicp_multi_projector *mp, const int *rawRows, const int *rawCols, float depthScale, int step,
+               float maxDepthCov, FrameSet &fs);
+int prep_frames(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *raws, const nicp_stats_params *sp,
+                const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds);
+int align_frame_pairs(nicp_context *ctx, const FrameSet &fs, int n, const nicp_cloud *const *refs,
+                      const nicp_cloud *const *curs, const nicp_align_params *ap, const float refOffset[16],
+                      const float curOffset[16], const float *guesses, const nicp_prior *priors, const int *priorOffsets,
+                      float imgThr, nicp_align_result *results);
 // frame_prep.cu
 int launch_depth_convert(nicp_context *ctx, const uint16_t *d_raw, int rows, int cols, float scale, int step,
                          float maxCov, float *d_out);
 int launch_frame_prep(nicp_context *ctx, const float *d_depth, const nicp_projector *proj, const nicp_stats_params *sp,
                       const float sensorOffset[16], int keepStats, nicp_cloud *cloud, int *d_index,
                       const CamSet *cams = nullptr);
-int launch_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw, int rawRows, int rawCols, float scale, int step,
-                          float maxCov, const nicp_projector *proj, const nicp_stats_params *sp, const float sensorOffset[16],
-                          int keepStats, nicp_cloud *const *clouds);
-int launch_rig_raw_prep_batch(nicp_context *ctx, int n, const uint16_t *const *d_raw, const int *rawRows, const int *rawCols,
-                              float scale, int step, float maxCov, const nicp_projector *proj, const CamSet &cams,
-                              const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds);
+int launch_raw_prep_batch(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *d_raw,
+                          const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds);
 int launch_stats_stage(nicp_context *ctx, const float4 *d_points, int n, const int *d_index, const int *d_interval, int rows,
                        int cols, const nicp_stats_params *sp, float *d_integral, float4 *d_normals, float *d_stats16,
                        float *d_eigvals, int *d_statsN, float *d_curvature);

@@ -337,7 +337,13 @@ void nicp_shard_pool_destroy(nicp_shard_pool *pool);
 int nicp_shard_pool_size(const nicp_shard_pool *pool);
 /* frames in, records out: raws[f] = raw 16-bit image of frame f (all raw_rows x raw_cols, converted like
  * nicp_raw_depth_to_cloud; sensor_offset is the sensor pose used for the frame preparation and for both sides of every
- * alignment, as PwnMatcherBase does), pair i = (reference_frame[i], current_frame[i]) with initial_guesses + 16 i. */
+ * alignment, as PwnMatcherBase does), pair i = (reference_frame[i], current_frame[i]) with initial_guesses + 16 i (NULL:
+ * identity).  Worker g takes pairs [g n / G, (g + 1) n / G) and walks them in windows: the longest runs of consecutive
+ * pairs whose distinct frames fit in its frame cap, building only the frames a window needs and does not hold yet.  The
+ * cap is max(2, 0.5 * device memory / (112 B * image pixels) / workers on that device), about 2 600 frames at 640 x 480 on
+ * a 180 GB GPU, so a block of a closer's partition is one window; NICP_SHARD_FRAMES, read when the pool is created, lowers
+ * it.  A worker keeps one cloud cache for this entry and nicp_multi_align_frames_sharded, which starts over when the image
+ * size changes.  Arguments are checked before any worker starts (raw size, frame indices, null images); synchronous. */
 int nicp_align_frames_sharded(nicp_shard_pool *pool, int n_frames, const uint16_t *const *raws, int raw_rows, int raw_cols,
                               float depth_scale, int step, float max_depth_cov, const nicp_projector *proj,
                               const nicp_stats_params *sp, const float sensor_offset[16], int n_pairs,
@@ -392,12 +398,9 @@ int nicp_multi_align_batch(nicp_context *ctx, int n, const nicp_cloud *const *re
  * raws[f * num_cameras + i] is camera i of frame f, raw_rows[i] x raw_cols[i] in every frame, as in
  * nicp_multi_raw_depth_to_cloud_batch; pair i = (reference_frame[i], current_frame[i]) with initial_guesses + 16 i (NULL:
  * identity) and priors as in nicp_multi_align_batch (priors / prior_offsets may be NULL); sensor_offset is the rig pose
- * used for the frame preparation and for both sides of every alignment.  Worker g takes pairs [g n / G, (g + 1) n / G)
- * and walks them in windows: the longest runs of consecutive pairs whose distinct frames fit in its frame cap, building
- * only the frames a window needs and does not hold yet (in current-major order the candidates stay resident and only the
- * current frames rotate).  The cap is max(2, 0.5 * device memory / (112 B * composite pixels) / workers on that device),
- * about 160 frames at 1280 x 3840 on a 180 GB GPU; NICP_SHARD_FRAMES, read when the pool is created, lowers it.  Rig
- * clouds are cached per worker apart from the pinhole ones, so rig calls leave nicp_align_frames_sharded as it was.
+ * used for the frame preparation and for both sides of every alignment.  Blocks, windows, frame cap and cloud cache are
+ * those of nicp_align_frames_sharded, with the composite image: the cap is about 160 frames at 1280 x 3840 on a 180 GB
+ * GPU (in current-major order the candidates stay resident and only the current frames rotate).
  * Record i is byte-identical to nicp_multi_align on the clouds nicp_multi_raw_depth_to_cloud_batch builds from its two
  * frames, whatever the device list, the workers per device or the cap.  Arguments are checked before any worker starts
  * (frame indices, null images, raw sizes, prior_offsets); synchronous. */

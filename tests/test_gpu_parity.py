@@ -411,6 +411,21 @@ def test_priors_in_a_batch(ctx):
     assert singles[0] != singles[1]
     plain = ctx.align_batch([ref] * 5, [cur] * 5, s.projector(), s.align_params(), guesses)
     assert plain[0].tobytes() == singles[0] and plain[1].tobytes() != singles[1]
+    # a bad prior_offsets array is rejected with its first bad entry named
+    import ctypes as C
+    L, parr = ctx.L, (capi.Prior * 2)(*lists[3])
+    RA, CA = (C.c_void_p * 3)(*[ref.handle] * 3), (C.c_void_p * 3)(*[cur.handle] * 3)
+    res = np.zeros(3, capi.RESULT_DTYPE)
+    eye = capi.colmajor(np.eye(4))
+
+    def bad(offs, priors=parr):
+        rc = L.nicp_align_batch_priors(ctx.handle, 3, RA, CA, C.byref(s.projector()), C.byref(s.align_params()),
+                                       capi._fptr(eye), capi._fptr(eye), None, priors, capi._iptr(np.array(offs, np.int32)),
+                                       C.c_float(50.0), res.ctypes.data_as(C.POINTER(capi.AlignResult)))
+        return rc, L.nicp_last_error().decode()
+    assert bad([1, 1, 2, 2]) == (1, "prior_offsets[0] is 1, not 0")
+    assert bad([0, 2, 1, 2]) == (1, "prior_offsets decrease at pair 1 (2 -> 1)")
+    assert bad([0, 1, 1, 2], None) == (1, "prior_offsets name 2 priors but priors is null")
 
 
 @pytest.mark.parametrize("width,height,ncam", [(160, 120, 4), (64, 48, 3)])

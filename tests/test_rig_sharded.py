@@ -98,10 +98,13 @@ def test_rig_sharded_equals_single_calls(verify, kind, step):
 @pytest.mark.parametrize("cap", ["2", "3"])
 def test_frame_cap_windows_change_no_record(verify, monkeypatch, cap):
     """NICP_SHARD_FRAMES = 2 and 3 cut the blocks into windows of a few frames: a self-pair, a window boundary inside the
-    pairs of one current frame, frames evicted and built again; the records are those of the default cap"""
+    pairs of one current frame, frames evicted and built again; the records are those of the default cap.  The cap bounds
+    nicp_align_frames_sharded too: its records under it are those of single nicp_align calls."""
     pairs = [(2, 0), (3, 0), (0, 0), (4, 0), (5, 0), (2, 1), (3, 1), (1, 1), (4, 1), (5, 1), (2, 0)]
     case = _rig_case("4cam", 1, pairs)
     singles = _singles(case, verify)
+    pinhole = _pinhole_case()
+    pinhole_singles = _pinhole_singles(pinhole, verify)
     default = []
     for devs in ([0], [0, 0]):
         pool = capi.ShardPool(devs, verify=verify)
@@ -115,6 +118,12 @@ def test_frame_cap_windows_change_no_record(verify, monkeypatch, cap):
         assert _run(pool, case).tobytes() == d, devs
         pool.close()
         for i, s in enumerate(singles):
+            assert recs[i].tobytes() == s, (devs, i)
+        pool = capi.ShardPool(devs, verify=verify)
+        recs = _pinhole_run(pool, pinhole)
+        assert _pinhole_run(pool, pinhole).tobytes() == recs.tobytes(), devs
+        pool.close()
+        for i, s in enumerate(pinhole_singles):
             assert recs[i].tobytes() == s, (devs, i)
 
 
@@ -139,8 +148,23 @@ def _pinhole_case():
     ap = capi.make_align_params(conf["inlierDistanceThreshold"], conf["inlierNormalAngularThreshold"],
                                 conf["flatCurvatureThreshold"], conf["inlierCurvatureRatioThreshold"], conf["inlierMaxChi2"],
                                 True, 10, 1)
-    return lambda pool: pool.align_frames(raws, proj, sp, ref_frame, cur_frame, np.stack(guesses).astype(np.float32), ap,
-                                          step=step)
+    return dict(raws=raws, proj=proj, sp=sp, ref=ref_frame, cur=cur_frame, guesses=np.stack(guesses).astype(np.float32),
+                ap=ap, step=step)
+
+
+def _pinhole_run(pool, case, raws=None):
+    return pool.align_frames(case["raws"] if raws is None else raws, case["proj"], case["sp"], case["ref"], case["cur"],
+                             case["guesses"], case["ap"], step=case["step"])
+
+
+def _pinhole_singles(case, verify):
+    """the records of nicp_align on clouds from single nicp_raw_depth_to_cloud calls on a plain context"""
+    c = capi.Context(0, verify=verify)
+    clouds = [c.raw_depth_to_cloud(r, case["proj"], case["sp"], step=case["step"])[0] for r in case["raws"]]
+    out = [bytes(c.align(clouds[r], clouds[q], case["proj"], case["ap"], guess=g))
+           for r, q, g in zip(case["ref"], case["cur"], case["guesses"])]
+    c.close()
+    return out
 
 
 @pytest.mark.gpu
@@ -148,13 +172,13 @@ def test_rig_calls_leave_the_pinhole_entry_unchanged():
     """pinhole, rig, pinhole on one pool: both pinhole calls give the records of a fresh pool"""
     pinhole = _pinhole_case()
     fresh = capi.ShardPool([0, 0])
-    expect = pinhole(fresh).tobytes()
+    expect = _pinhole_run(fresh, pinhole).tobytes()
     fresh.close()
     pool = capi.ShardPool([0, 0])
-    assert pinhole(pool).tobytes() == expect
+    assert _pinhole_run(pool, pinhole).tobytes() == expect
     case = _rig_case("4cam", 1)
     _run(pool, case)
-    assert pinhole(pool).tobytes() == expect
+    assert _pinhole_run(pool, pinhole).tobytes() == expect
     pool.close()
 
 
@@ -198,6 +222,12 @@ def test_bad_input_is_rejected_before_any_worker(verify):
     assert status == 1 and msg.startswith("camera 2: raw image"), msg
     offs = np.array([0, 0, 1, 2, 2, 1, 1, 2, 2], np.int32)[:n + 1]
     assert call(offs=offs) == (1, "prior_offsets decrease at pair 4 (2 -> 1)")
+    # the pinhole entry checks its raw size in the calling thread as well
+    pinhole = _pinhole_case()
+    wrong = [np.zeros((r.shape[0], r.shape[1] + 4), np.uint16) for r in pinhole["raws"]]
+    with pytest.raises(capi.NicpError) as e:
+        _pinhole_run(pool, pinhole, wrong)
+    assert str(e.value) == "nicp error 1: projector image size 120x160 does not match the scaled raw image 120x161"
     pool.close()
 
 
