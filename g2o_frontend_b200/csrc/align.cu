@@ -706,7 +706,7 @@ static void launch_group(nicp_context *ctx, int nGroups, int tiles, int parity, 
 // butterfly).
 static void launch_corr_lin(nicp_context *ctx, int mode, int nPairs, int nGroups, int nb, int parity, int epoch, int writeCorr,
                             const AlignConsts &ac, int P, int imgStats, float imgThr, int curEpoch = kEpochFresh) {
-  const bool grouped = nPairs >= ctx->groupMinAvg * nGroups;
+  const bool grouped = takes_grouped(ctx, nPairs, nGroups);
   const dim3 grid(nb, nPairs);
   if (mode == 0) {
     if (grouped) launch_group<0>(ctx, nGroups, nb, parity, epoch, writeCorr, ac, P, imgStats, imgThr, curEpoch);

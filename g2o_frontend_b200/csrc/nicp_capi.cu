@@ -414,6 +414,10 @@ static AlignConsts make_consts(const nicp_projector *proj, const nicp_align_para
   ac.flatCurvature = ap->flat_curvature_threshold;
   ac.minRatio = 1.0f / ap->inlier_curvature_ratio_threshold;
   ac.maxRatio = ap->inlier_curvature_ratio_threshold;
+  // A threshold below 1 puts 1 outside [minRatio, maxRatio], so the reference rejects every pair with a finite ratio
+  // (correspondencefinder.cpp:87-99).  The kernels accept equal curvatures without a division (the ratio is exactly 1),
+  // so such a configuration rejects every pair at the normal-angle gate instead, which sees the same pairs.
+  if (ac.minRatio > 1.0f || ac.maxRatio < 1.0f) ac.normalThreshold = INFINITY;
   ac.maxChi2 = ap->inlier_max_chi2;
   ac.robust = ap->robust_kernel;
   ac.one = 1.0f;
@@ -463,8 +467,8 @@ static void fill_desc(nicp_context *ctx, int slot, int curSlot, const nicp_cloud
   D.curPoints = cur->points;
   D.curNormals = cur->normals;
   D.curOmega = cur->omega;
-  D.refPN = ref->pn;  // (null until ensure_pn: the grouped kernel's chunks call it)
-  D.curPN = cur->pn;
+  D.refPN = nullptr;  // set by prepare_pn when the chunk takes the grouped kernel
+  D.curPN = nullptr;
   D.curN = cur->d_n;
   D.refZ[0] = ctx->d_refZ + (size_t)slot * P;
   D.refZ[1] = ctx->d_refZ + ((size_t)ctx->slots + slot) * P;
@@ -483,6 +487,15 @@ static void fill_desc(nicp_context *ctx, int slot, int curSlot, const nicp_cloud
   } else {
     mat4_identity(D.guess);
   }
+}
+// descriptor `slot` of a chunk that takes the grouped kernel (takes_grouped): the kernel gathers the reference and the
+// current points + normals from the clouds' interleaved caches, packed here if they are missing or out of date
+static int prepare_pn(nicp_context *ctx, int slot, const nicp_cloud *ref, const nicp_cloud *cur) {
+  int rc;
+  if ((rc = ensure_pn(ctx, const_cast<nicp_cloud *>(ref))) || (rc = ensure_pn(ctx, const_cast<nicp_cloud *>(cur)))) return rc;
+  ctx->h_desc[slot].refPN = ref->pn;
+  ctx->h_desc[slot].curPN = cur->pn;
+  return NICP_OK;
 }
 
 // ---- Aligner::_computeStatistics tail (aligner.cpp:172-198, unscented.h:23-65): nicp_stats_tail.cuh, shared with the device ----
@@ -1199,6 +1212,7 @@ int nicp_correspond_linearize(nicp_context *ctx, const nicp_cloud *reference, co
   proj.cols = cols;
   AlignConsts ac = make_consts(&proj, ap, nullptr);
   fill_desc(ctx, 0, 0, reference, current, nullptr, nullptr, nullptr);
+  if (takes_grouped(ctx, 1, 1) && (rc = prepare_pn(ctx, 0, reference, current))) return rc;
   std::vector<unsigned long long> z(px);
   for (size_t i = 0; i < px; i++) z[i] = reference_index[i] < 0 ? kEmptyZ : ((unsigned long long)kEpochFresh << 60) | (unsigned int)reference_index[i];
   NICP_CUDA(cudaMemcpyAsync(ctx->d_desc, ctx->h_desc, sizeof(PairDesc), cudaMemcpyHostToDevice, ctx->stream));
@@ -1228,6 +1242,7 @@ int nicp_linearize(nicp_context *ctx, const nicp_cloud *reference, const nicp_cl
   proj.cols = (int)px;
   AlignConsts ac = make_consts(&proj, ap, nullptr);
   fill_desc(ctx, 0, 0, reference, current, nullptr, nullptr, nullptr);
+  if (takes_grouped(ctx, 1, 1) && (rc = prepare_pn(ctx, 0, reference, current))) return rc;
   std::vector<int> ri(px, -1), ci(px, -1);
   for (int i = 0; i < n; i++) {
     ri[i] = correspondences[2 * i];
@@ -1354,11 +1369,6 @@ static int align_common(nicp_context *ctx, int n, const nicp_cloud *const *refs,
         if ((rc = ensure_points3(ctx, const_cast<nicp_cloud *>(r)))) return rc;
         ctx->h_desc[i].refPoints3 = r->points3;
       }
-      if (m >= 3 || ctx->groupMinAvg == 0) {  // chunks that may take the grouped kernel gather from the interleaved point + normal caches
-        if ((rc = ensure_pn(ctx, const_cast<nicp_cloud *>(r))) || (rc = ensure_pn(ctx, const_cast<nicp_cloud *>(c)))) return rc;
-        ctx->h_desc[i].refPN = r->pn;
-        ctx->h_desc[i].curPN = c->pn;
-      }
       if (numPriors > 0) {
         const int p0 = priorOffsets ? priorOffsets[src] : 0, p1 = priorOffsets ? priorOffsets[src + 1] : numPriors;
         ctx->h_desc[i].priors = p1 > p0 ? reinterpret_cast<const HostPrior *>(ctx->d_priors) + p0 : nullptr;
@@ -1366,6 +1376,14 @@ static int align_common(nicp_context *ctx, int n, const nicp_cloud *const *refs,
       }
     }
     const int nGroups = stage_groups(ctx, m, curSlotOf.data());
+    if (takes_grouped(ctx, m, nGroups)) {
+      for (int i = 0; i < m; i++) {
+        const nicp_cloud *r = refs[base + order[i]], *c = curs[base + order[i]];
+        if ((rc = prepare_pn(ctx, i, r, c))) return rc;
+      }
+      PairGroup *g = host_groups(ctx);
+      for (int k = 0; k < nGroups; k++) g[k].curPN = ctx->h_desc[g[k].first].curPN;
+    }
     const bool useGraph = single && ctx->graphsEnabled && !cams.multi && !ctx->timing;
     bool replayed = false;
     cudaStream_t tail = ctx->stream;  // where this chunk's records are finished and copied out

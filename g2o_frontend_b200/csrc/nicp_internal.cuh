@@ -362,6 +362,12 @@ struct nicp_context {
 };
 
 namespace nicp {
+// whether a chunk of nPairs pairs in nGroups pair groups runs the grouped correspondence kernel (k_corr_lin_group) rather
+// than the per-pair one: its groups average at least NICP_GROUP_MIN_AVG pairs.  The grouped kernel gathers from the
+// interleaved point + normal caches (nicp_cloud::pn), so every caller that may launch it asks this of the chunk it has
+// staged and packs the caches (ensure_pn) exactly when the answer is yes.
+inline bool takes_grouped(const nicp_context *ctx, int nPairs, int nGroups) { return nPairs >= ctx->groupMinAvg * nGroups; }
+
 // prior_offsets of a batch: n + 1 non-decreasing entries from 0 (or NULL: no priors); a bad array is reported by its first
 // bad entry
 inline int check_prior_offsets(int n, const nicp_prior *priors, const int *prior_offsets) {
