@@ -671,6 +671,7 @@ static int launch_prep_set(nicp_context *ctx, const PrepBatch &B, const nicp_pro
   mat4_identity(I4);
   compute_iKRt(proj->K, I4, iKRt);
   Affine a = affine_from(iKRt);
+  // cols <= NICP_MAX_PREP_COLS (check_prep_image): smem <= kRowPassSmemMax
   size_t smem = (size_t)kIntegralCh * (cols + 1) * sizeof(float);
   if (smem > 48 * 1024 && smem > ctx->rowsSmemCfg) {
     NICP_CUDA(cudaFuncSetAttribute(k_integral_rows<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -931,11 +932,8 @@ static StatsConsts stage_consts(const nicp_stats_params *sp) {
 int launch_stats_stage(nicp_context *ctx, const float4 *d_points, int n, const int *d_index, const int *d_interval, int rows,
                        int cols, const nicp_stats_params *sp, float *d_integral, float4 *d_normals, float *d_stats16,
                        float *d_eigvals, int *d_statsN, float *d_curvature) {
+  // cols <= NICP_MAX_PREP_COLS (check_prep_image): smem <= kRowPassSmemMax
   const size_t smem = (size_t)kIntegralCh * (cols + 1) * sizeof(float);
-  if (smem > 200 * 1024) {
-    set_error("image too wide for the row pass (%d columns)", cols);
-    return NICP_ERR_INVALID;
-  }
   if (smem > 48 * 1024) NICP_CUDA(cudaFuncSetAttribute(k_integral_rows_indexed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_integral_rows_indexed<<<rows, 256, smem, ctx->stream>>>(d_index, d_points, rows, cols, d_integral);
   NICP_CHECK_LAUNCH(ctx);

@@ -23,6 +23,25 @@ void set_error(const char *fmt, ...) {
   va_end(ap);
 }
 
+// Image sizes frame preparation builds clouds for (NICP_MAX_PREP_COLS / NICP_MAX_PREP_PIXELS, include/nicp_b200.h): the row
+// pass of the integral image stages the 10 channels of one image row in shared memory, and the compacted point index, the
+// cloud size and the window counts are read from channel 0 of the float32 integral image, exact integers up to 2^24.
+// Checked before anything is uploaded, so that a rejected call leaves the context as it was.
+int check_prep_image(int rows, int cols) {
+  if (cols > NICP_MAX_PREP_COLS) {
+    set_error("image of %d columns is too wide for the row pass of the integral image: %zu bytes of shared memory per "
+              "block, at most %d columns (%zu bytes) fit", cols, (size_t)kIntegralCh * (cols + 1) * sizeof(float),
+              NICP_MAX_PREP_COLS, kRowPassSmemMax);
+    return NICP_ERR_INVALID;
+  }
+  if ((size_t)rows * cols > (size_t)NICP_MAX_PREP_PIXELS) {
+    set_error("image of %d x %d = %zu pixels exceeds %d: the float32 integral image counts pixels exactly only up to 2^24",
+              rows, cols, (size_t)rows * cols, NICP_MAX_PREP_PIXELS);
+    return NICP_ERR_INVALID;
+  }
+  return NICP_OK;
+}
+
 static int env_int(const char *name, int def) {
   const char *v = getenv(name);
   if (!v || !*v) return def;
@@ -266,6 +285,8 @@ int frames_pinhole(const nicp_projector *proj, int rawRows, int rawCols, float d
               rawRows / step, rawCols / step);
     return NICP_ERR_INVALID;
   }
+  int rc;
+  if ((rc = check_prep_image(proj->rows, proj->cols))) return rc;
   memset(&fs, 0, sizeof fs);
   fs.cams = camset_pinhole(proj);
   fs.proj = *proj;
@@ -309,7 +330,7 @@ int frames_rig(const nicp_multi_projector *mp, const int *rawRows, const int *ra
                float maxDepthCov, FrameSet &fs) {
   if (!rawRows || !rawCols) return NICP_ERR_INVALID;
   int rc;
-  if ((rc = rig_geometry(mp, fs))) return rc;
+  if ((rc = rig_geometry(mp, fs)) || (rc = check_prep_image(fs.proj.rows, fs.proj.cols))) return rc;
   if (step < 1) step = 1;
   const CamSet &c = fs.cams;
   for (int i = 0; i < c.n; i++) {
@@ -1007,11 +1028,12 @@ int nicp_depth_to_cloud(nicp_context *ctx, const float *depth, const nicp_projec
   if (!ctx || !depth || !proj || !sp || !cloud || proj->rows <= 0 || proj->cols <= 0) return NICP_ERR_INVALID;
   NICP_CUDA(cudaSetDevice(ctx->device));
   size_t px = (size_t)proj->rows * proj->cols;
+  int rc;
+  if ((rc = check_prep_image(proj->rows, proj->cols))) return rc;
   if ((size_t)cloud->capacity < px) {
     set_error("cloud capacity %d smaller than the image (%zu pixels)", cloud->capacity, px);
     return NICP_ERR_INVALID;
   }
-  int rc;
   if ((rc = ensure_prep(ctx, px))) return rc;
   NICP_CUDA(cudaMemcpyAsync(ctx->d_depth, depth, px * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
   return depth_to_cloud_device(ctx, proj, sp, sensor_offset, keep_stats, cloud, index);
@@ -1029,11 +1051,12 @@ int nicp_raw_depth_to_cloud(nicp_context *ctx, const uint16_t *raw, int raw_rows
     return NICP_ERR_INVALID;
   }
   size_t rpx = (size_t)raw_rows * raw_cols, px = (size_t)proj->rows * proj->cols;
+  int rc;
+  if ((rc = check_prep_image(proj->rows, proj->cols))) return rc;
   if ((size_t)cloud->capacity < px) {
     set_error("cloud capacity %d smaller than the image (%zu pixels)", cloud->capacity, px);
     return NICP_ERR_INVALID;
   }
-  int rc;
   if ((rc = ensure_raw(ctx, rpx))) return rc;
   if ((rc = ensure_prep(ctx, px))) return rc;
   // the upload runs on its own stream into one of two staging images, so the copy of this frame overlaps the
@@ -1086,6 +1109,7 @@ int nicp_stats_compute(nicp_context *ctx, const float *points4, int n, const int
   int *d_index, *d_interval, *d_cnt;
   float *d_integral, *d_stats, *d_eig, *d_curv;
   int rc;
+  if ((rc = check_prep_image(rows, cols))) return rc;
   if ((rc = bufs.alloc(&d_points, (size_t)n)) || (rc = bufs.alloc(&d_normals, (size_t)n)) || (rc = bufs.alloc(&d_index, px)) ||
       (rc = bufs.alloc(&d_interval, px)) || (rc = bufs.alloc(&d_cnt, (size_t)n)) || (rc = bufs.alloc(&d_integral, px * kIntegralCh)) ||
       (rc = bufs.alloc(&d_stats, (size_t)n * 16)) || (rc = bufs.alloc(&d_eig, (size_t)n * 3)) || (rc = bufs.alloc(&d_curv, (size_t)n)))
@@ -1548,7 +1572,7 @@ int nicp_multi_depth_to_cloud(nicp_context *ctx, const float *depth, const nicp_
   NICP_CUDA(cudaSetDevice(ctx->device));
   FrameSet fs;
   int rc;
-  if ((rc = rig_geometry(mp, fs))) return rc;
+  if ((rc = rig_geometry(mp, fs)) || (rc = check_prep_image(fs.proj.rows, fs.proj.cols))) return rc;
   size_t px = (size_t)fs.proj.rows * fs.proj.cols;
   if ((size_t)cloud->capacity < px) {
     set_error("cloud capacity %d smaller than the composite image (%zu pixels)", cloud->capacity, px);

@@ -37,6 +37,12 @@ constexpr int kMaxGroup = 16;     // pairs per group of the grouped fused kernel
 constexpr int kMaxPrepBatch = 8;  // frames per frame-preparation launch set (their scratch stays L2 resident)
 constexpr int kAccum = 32;        // accumulator slots per partial (30 used)
 constexpr int kIntegralCh = 10;   // n,x,y,z,xx,xy,xz,yy,yz,zz
+// dynamic shared memory a block of sm_100 may opt into (cudaDevAttrMaxSharedMemoryPerBlockOptin), the bound of the row pass
+// of the integral image, which stages kIntegralCh * (cols + 1) floats: NICP_MAX_PREP_COLS is the widest image that fits
+constexpr size_t kRowPassSmemMax = 227 * 1024;
+static_assert((size_t)kIntegralCh * (NICP_MAX_PREP_COLS + 1) * sizeof(float) <= kRowPassSmemMax &&
+                  (size_t)kIntegralCh * (NICP_MAX_PREP_COLS + 2) * sizeof(float) > kRowPassSmemMax,
+              "NICP_MAX_PREP_COLS is the widest row the row pass can stage");
 constexpr unsigned long long kEmptyZ = 0xFFFFFFFFFFFFFFFFull;
 
 // z-buffer word (one per pixel, filled with 64-bit atomicMin):
@@ -389,6 +395,8 @@ inline int check_prior_offsets(int n, const nicp_prior *priors, const int *prior
 }
 
 // nicp_capi.cu
+// NICP_ERR_INVALID (with a message) for an image frame preparation cannot build a cloud for
+int check_prep_image(int rows, int cols);
 int frames_pinhole(const nicp_projector *proj, int rawRows, int rawCols, float depthScale, int step, float maxDepthCov,
                    FrameSet &fs);
 int frames_rig(const nicp_multi_projector *mp, const int *rawRows, const int *rawCols, float depthScale, int step,

@@ -35,6 +35,17 @@ extern "C" {
 #define NICP_ERR_CUDA 2      /* a CUDA runtime call or kernel failed; see nicp_last_error() */
 #define NICP_ERR_ALLOC 3
 
+/* Largest image frame preparation (nicp_depth_to_cloud, nicp_raw_depth_to_cloud(_batch), nicp_multi_depth_to_cloud,
+ * nicp_multi_raw_depth_to_cloud_batch, nicp_stats_compute, the sharded closers) builds a cloud for; for a
+ * MultiPointProjector the limits apply to the composite image (cols = sum of the cameras' heights).  A larger image is
+ * rejected with NICP_ERR_INVALID before anything is uploaded.
+ *   NICP_MAX_PREP_COLS    the row pass of the integral image stages 10 float channels of one row in the 227 KB of
+ *                         shared memory a block may have (six 1920x1080 cameras, 6480 columns, do not fit)
+ *   NICP_MAX_PREP_PIXELS  2^24: point indices, cloud sizes and window counts come from float32 pixel counts, which are
+ *                         exact integers only up to 2^24 (eight 1920x1200 cameras, 18.4 M pixels, exceed it) */
+#define NICP_MAX_PREP_COLS 5810
+#define NICP_MAX_PREP_PIXELS 16777216
+
 typedef struct nicp_context nicp_context; /* one per host thread / GPU (not thread-safe, like pwn_core) */
 typedef struct nicp_cloud nicp_cloud;     /* device-resident pwn::Cloud (cloud.h:20-187) */
 

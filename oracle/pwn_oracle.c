@@ -318,7 +318,9 @@ static void unit_orthogonal(const float *s, float *o) {
     o[0] = 0.0f; o[1] = -s[2] * invnm; o[2] = s[1] * invnm;
   }
 }
-void orc_eigen3(const float C[9], float evals[3], float evecs[9]) {
+/* devtrig != 0: atan2 / cos / sin evaluated in float64 and rounded to float32, as the CUDA path does (eigen_variant 2);
+ * otherwise the libm float functions of the reference build */
+static void eigen3_32(const float C[9], float evals[3], float evecs[9], int devtrig) {
   const float eps = FLT_EPSILON;
   float scale = 0.0f;
   for (int i = 0; i < 9; i++) { float a = fabsf(C[i]); if (a > scale) scale = a; }
@@ -339,9 +341,16 @@ void orc_eigen3(const float C[9], float evals[3], float evecs[9]) {
   float q = half_b * half_b + a_over_3 * a_over_3 * a_over_3;
   if (q > 0.0f) q = 0.0f;
   float rho = sqrtf(-a_over_3);
-  float theta = atan2f(sqrtf(-q), half_b) * s_inv3;
-  float cos_theta = cosf(theta);
-  float sin_theta = sinf(theta);
+  float theta, cos_theta, sin_theta;
+  if (devtrig) {
+    theta = (float)atan2((double)sqrtf(-q), (double)half_b) * s_inv3;
+    cos_theta = (float)cos((double)theta);
+    sin_theta = (float)sin((double)theta);
+  } else {
+    theta = atan2f(sqrtf(-q), half_b) * s_inv3;
+    cos_theta = cosf(theta);
+    sin_theta = sinf(theta);
+  }
   float r0 = c2_over_3 + 2.0f * rho * cos_theta;
   float r1 = c2_over_3 - rho * (cos_theta + s_sqrt3 * sin_theta);
   float r2 = c2_over_3 - rho * (cos_theta - s_sqrt3 * sin_theta);
@@ -429,6 +438,8 @@ void orc_eigen3(const float C[9], float evals[3], float evecs[9]) {
   }
   for (int i = 0; i < 3; i++) evals[i] = ev[i] * scale;
 }
+void orc_eigen3(const float C[9], float evals[3], float evecs[9]) { eigen3_32(C, evals, evecs, 0); }
+void orc_eigen3_devtrig(const float C[9], float evals[3], float evecs[9]) { eigen3_32(C, evals, evecs, 1); }
 
 /* ------------------------------------------------------------------------------------------
  * The same call as Eigen >= 3.3 implements it (recalled from Eigen/src/Eigenvalues/SelfAdjointEigenSolver.h of 3.3.x,
@@ -522,11 +533,13 @@ void orc_eigen3_v33(const float C[9], float evals[3], float evecs[9]) {
   }
   for (int i = 0; i < 3; i++) evals[i] = ev[i] * scale + shift;
 }
-static int g_eigen_variant = 0; /* 0: Eigen 3.2.x (the variant the CUDA path follows), 1: Eigen >= 3.3 */
+/* 0: Eigen 3.2.x with libm (the reference build; the variant the CUDA path follows), 1: Eigen >= 3.3, 2: Eigen 3.2.x with
+ * the CUDA path's float64 trig (test yardstick: every other operation of the CUDA path is meant to match it bit for bit) */
+static int g_eigen_variant = 0;
 void orc_set_eigen_variant(int v) { g_eigen_variant = v; }
 static void eigen3_dispatch(const float C[9], float evals[3], float evecs[9]) {
   if (g_eigen_variant == 1) orc_eigen3_v33(C, evals, evecs);
-  else orc_eigen3(C, evals, evecs);
+  else eigen3_32(C, evals, evecs, g_eigen_variant == 2);
 }
 
 /* ------------------------------------------------------------------------------------------

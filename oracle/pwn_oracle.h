@@ -65,7 +65,9 @@ typedef struct {
 
 void orc_eigen3(const float C[9], float evals[3], float evecs[9]);      /* Eigen 3.2.x computeDirect */
 void orc_eigen3_v33(const float C[9], float evals[3], float evecs[9]);  /* Eigen >= 3.3 computeDirect (sensitivity study) */
-void orc_set_eigen_variant(int v); /* which of the two orc_stats / orc_depth_to_cloud use: 0 = 3.2 (default), 1 = >= 3.3 */
+void orc_eigen3_devtrig(const float C[9], float evals[3], float evecs[9]); /* 3.2.x, trig in float64 as the CUDA path */
+void orc_set_eigen_variant(int v); /* which orc_stats / orc_depth_to_cloud use: 0 = 3.2 (default), 1 = >= 3.3,
+                                      2 = 3.2 with the CUDA path's float64 atan2 / cos / sin (orc_eigen3_devtrig) */
 
 void orc_stats(const float *integral, const int *index, const int *interval, const float *points,
                int rows, int cols, int n, const orc_stats_params *p,

@@ -585,10 +585,23 @@ def information_stage(normals, statsM, eigvals, curvature, sp):
 
 
 def set_eigen_variant(v, fast=False):
-    """0: Eigen 3.2.x computeDirect (default; what the CUDA path follows), 1: the Eigen >= 3.3 implementation"""
+    """0: Eigen 3.2.x computeDirect (default; what the CUDA path follows), 1: the Eigen >= 3.3 implementation,
+    2: Eigen 3.2.x with atan2 / cos / sin evaluated in float64 and rounded, as the CUDA path evaluates them.
+    The variant is global state of the library: callers that change it restore 0 afterwards."""
     f = lib(fast).orc_set_eigen_variant
     f.restype = None
     f(int(v))
+
+
+def eigen3_devtrig(Cm):
+    """Eigen 3.2.x computeDirect with the CUDA path's float64 trig (eigen variant 2)"""
+    Cm, cp = _f(colmajor(Cm))
+    ev = np.zeros(3, np.float32)
+    U = np.zeros(9, np.float32)
+    f = lib().orc_eigen3_devtrig
+    f.restype = None
+    f(cp, _fp(ev), _fp(U))
+    return ev, from_colmajor(U, 3)
 
 
 def eigen3_v33(Cm):
