@@ -32,6 +32,8 @@ SYMBOLS = [
     "nicp_cloud_upload_gaussians", "nicp_merge", "nicp_voxelize",
     "nicp_shard_pool_create", "nicp_shard_pool_destroy", "nicp_shard_pool_size", "nicp_align_frames_sharded",
     "nicp_multi_align_frames_sharded",
+    "nicp_frame_store_create", "nicp_multi_frame_store_create", "nicp_frame_store_destroy", "nicp_frame_store_add",
+    "nicp_frame_store_remove", "nicp_frame_store_size", "nicp_frame_store_align", "nicp_frame_store_counters",
 ]
 
 GAUSS_FLOATS = 24
@@ -126,6 +128,7 @@ def load(verify=False):
     L.nicp_v2t.restype = None
     L.nicp_t2v.restype = None
     L.nicp_multi_image_size.restype = None
+    L.nicp_frame_store_destroy.restype = None
     for name in SYMBOLS:
         fn = getattr(L, name)
         if fn.restype is C.c_int:
@@ -738,6 +741,105 @@ class ShardPool:
     def close(self):
         if self.handle:
             self.L.nicp_shard_pool_destroy(self.handle)
+            self.handle = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _ids(ids):
+    return np.ascontiguousarray(ids, np.int64)
+
+
+def _llptr(a):
+    return a.ctypes.data_as(C.POINTER(C.c_longlong))
+
+
+class FrameStore:
+    """nicp_frame_store: the raw frames of one pinhole camera or one rig on a shard pool, under caller-chosen int64 ids.
+    Each worker keeps the clouds of the frames it aligned across calls and prepares a frame only when it does not hold it.
+
+    camera is a Projector (pinhole; raw_shape = (rows, cols) of every raw frame) or a MultiProjector (rig; raw_shape = one
+    (rows, cols) per camera, as the sensor delivers it).  The other arguments are those of ShardPool.align_frames /
+    multi_align_frames and are fixed for the store's lifetime."""
+
+    def __init__(self, pool, camera, sp, raw_shape, depth_scale=0.001, step=1, max_depth_cov=0.01, sensor_offset=None):
+        self.pool = pool  # the store's clouds live on the pool's workers
+        self.L = pool.L
+        self.rig = isinstance(camera, MultiProjector)
+        self.num_cameras = camera.num_cameras if self.rig else 1
+        self.handle = C.c_void_p()
+        so = None if sensor_offset is None else _fptr(colmajor(sensor_offset))
+        # the C call copies raw_rows x raw_cols pixels of every camera from whatever pointer it is given, so add() checks
+        # each image against these shapes
+        self.raw_shapes = [tuple(int(x) for x in s) for s in (raw_shape if self.rig else [raw_shape])]
+        if self.rig:
+            shapes = np.array(raw_shape, np.int32).reshape(self.num_cameras, 2)
+            rr, rc = np.ascontiguousarray(shapes[:, 0]), np.ascontiguousarray(shapes[:, 1])
+            _check(self.L, self.L.nicp_multi_frame_store_create(
+                pool.handle, _iptr(rr), _iptr(rc), C.c_float(depth_scale), int(step), C.c_float(max_depth_cov),
+                C.byref(camera), C.byref(sp), so, C.byref(self.handle)))
+        else:
+            rows, cols = raw_shape
+            _check(self.L, self.L.nicp_frame_store_create(pool.handle, int(rows), int(cols), C.c_float(depth_scale), int(step),
+                                                          C.c_float(max_depth_cov), C.byref(camera), C.byref(sp), so,
+                                                          C.byref(self.handle)))
+
+    def add(self, ids, frames):
+        """frames[k] gets id ids[k]: a uint16 image (pinhole) or a sequence of one uint16 image per camera (rig), each of
+        exactly the raw shape the store was created with for its camera; any other shape raises ValueError and adds
+        nothing"""
+        ids = _ids(ids)
+        n = len(ids)
+        if len(frames) != n:
+            raise ValueError("%d ids for %d frames" % (n, len(frames)))
+        nc = self.num_cameras
+        imgs = []
+        for k, fr in enumerate(frames):
+            cams = fr if self.rig else [fr]
+            if len(cams) != nc:
+                raise ValueError("frame %d has %d images for %d cameras" % (k, len(cams), nc))
+            for i, im in enumerate(cams):
+                im = np.ascontiguousarray(im, np.uint16)
+                if im.shape != self.raw_shapes[i]:
+                    raise ValueError("frame %d, camera %d: raw image of shape %s, the store takes %s"
+                                     % (k, i, im.shape, self.raw_shapes[i]))
+                imgs.append(im)
+        RA = (C.c_void_p * max(len(imgs), 1))(*[im.ctypes.data for im in imgs])
+        _check(self.L, self.L.nicp_frame_store_add(self.handle, n, _llptr(ids), RA))
+
+    def remove(self, ids):
+        ids = _ids(ids)
+        _check(self.L, self.L.nicp_frame_store_remove(self.handle, len(ids), _llptr(ids)))
+
+    def size(self):
+        return int(self.L.nicp_frame_store_size(self.handle))
+
+    def align(self, ref_ids, cur_ids, guesses, ap, priors=None, img_threshold=50.0):
+        """pair i = (ref_ids[i], cur_ids[i]) with guesses[i] (None: identity); priors: None or one list of Prior per pair.
+        Returns RESULT_DTYPE records."""
+        rf, cf = _ids(ref_ids), _ids(cur_ids)
+        n = len(rf)
+        assert len(cf) == n
+        parr, offs = _priors(priors, n)
+        results = np.zeros(n, RESULT_DTYPE)
+        _check(self.L, self.L.nicp_frame_store_align(self.handle, n, _llptr(rf), _llptr(cf), _guesses(guesses, n), parr, offs,
+                                                     C.byref(ap), C.c_float(img_threshold),
+                                                     results.ctypes.data_as(C.POINTER(AlignResult))))
+        return results
+
+    def counters(self):
+        """(frames built, frames found resident) since creation, summed over the workers and the windows of every call"""
+        b, r = C.c_longlong(0), C.c_longlong(0)
+        _check(self.L, self.L.nicp_frame_store_counters(self.handle, C.byref(b), C.byref(r)))
+        return b.value, r.value
+
+    def close(self):
+        if self.handle:
+            self.L.nicp_frame_store_destroy(self.handle)
             self.handle = C.c_void_p()
 
     def __del__(self):

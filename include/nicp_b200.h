@@ -354,7 +354,8 @@ int nicp_shard_pool_size(const nicp_shard_pool *pool);
  * cap is max(2, 0.5 * device memory / (112 B * image pixels) / workers on that device), about 2 600 frames at 640 x 480 on
  * a 180 GB GPU, so a block of a closer's partition is one window; NICP_SHARD_FRAMES, read when the pool is created, lowers
  * it.  A worker keeps one cloud cache for this entry and nicp_multi_align_frames_sharded, which starts over when the image
- * size changes.  Arguments are checked before any worker starts (raw size, frame indices, null images); synchronous. */
+ * size changes; its clouds are reused as storage only, every call prepares the frames it references again (a frame store,
+ * below, keeps them across calls).  Arguments are checked before any worker starts (raw size, frame indices, null images); synchronous. */
 int nicp_align_frames_sharded(nicp_shard_pool *pool, int n_frames, const uint16_t *const *raws, int raw_rows, int raw_cols,
                               float depth_scale, int step, float max_depth_cov, const nicp_projector *proj,
                               const nicp_stats_params *sp, const float sensor_offset[16], int n_pairs,
@@ -423,6 +424,61 @@ int nicp_multi_align_frames_sharded(nicp_shard_pool *pool, int n_frames, const u
                                     const nicp_prior *priors, const int *prior_offsets,
                                     const nicp_align_params *ap, float frame_inlier_depth_threshold,
                                     nicp_align_result *results);
+
+/* ---- frame store: loop-closure frames resident on a shard pool across calls -------------------------------------------
+ * An incremental closer matches each new map node against candidates that earlier steps already used
+ * (MapCloser::process -> PwnCloser::processPartition, pwn_tracker2/pwn_closer.cpp:83-182) and keeps their clouds between
+ * steps (PwnCloudCache, pwn_tracker2/pwn_cloud_cache.cpp:60-102).  A frame store holds the raw frames of one pinhole camera
+ * or one rig under caller-chosen 64-bit ids (e.g. BOSS node ids); each worker of the pool keeps the clouds of the frames its
+ * pairs used, and a later call finds them there.
+ *   - Records: record i of nicp_frame_store_align is byte-identical to nicp_align / nicp_multi_align, with the pair's guess
+ *     and priors, on the clouds nicp_raw_depth_to_cloud_batch / nicp_multi_raw_depth_to_cloud_batch build from its two
+ *     frames, whatever the device list, the workers per device, the frame cap, the store's history or what is resident.
+ *   - Placement and windows: those of nicp_align_frames_sharded (worker g takes pairs [g n / G, (g + 1) n / G)), but each
+ *     worker's slot table is keyed by frame id and persists across calls.  A window keeps the resident clouds it uses;
+ *     missing frames go to empty slots first, then to new clouds while the worker holds fewer than its frame cap, then to
+ *     the least recently used slots the window does not use.  The cap is that of the sharded entries (NICP_SHARD_FRAMES
+ *     lowers it), applied per store and per worker.  The cloud cache of the sharded entries is separate: a worker holds up
+ *     to the cap for those entries and up to the cap for each store, so several full caches on one GPU add up.
+ *   - Lazily built: nicp_frame_store_add only copies the raw images to host memory; a frame is prepared the first time a
+ *     window on some worker needs it, and again only after it was evicted there.  Keep the candidates of one current frame
+ *     in the same order (e.g. by id) from call to call so that each worker keeps seeing the same slice of them.
+ *   - Every argument is checked in the calling thread before any worker starts, and a rejected call changes nothing: null
+ *     handles or arrays, an id added twice (in one call or already in the store), remove / align naming an id that is not
+ *     in the store, bad prior_offsets.  A worker that fails mid-call leaves no slot claiming a frame it did not finish.
+ *   - nicp_shard_pool_destroy releases the device clouds of the pool's stores; every later call on such a store except
+ *     nicp_frame_store_destroy returns NICP_ERR_INVALID (nicp_frame_store_size returns -1).
+ *   - A pool and its stores are used from one host thread at a time, like a context.  Calls are synchronous. */
+typedef struct nicp_frame_store nicp_frame_store;
+/* the frame description, fixed for the store's lifetime and validated like nicp_align_frames_sharded /
+ * nicp_multi_align_frames_sharded validate theirs: raw size, depth_scale, step, max_depth_cov, projector (or rig),
+ * statistics parameters and the sensor offset (NULL: identity) used for the preparation and both sides of every alignment */
+int nicp_frame_store_create(nicp_shard_pool *pool, int raw_rows, int raw_cols, float depth_scale, int step,
+                            float max_depth_cov, const nicp_projector *proj, const nicp_stats_params *sp,
+                            const float sensor_offset[16], nicp_frame_store **store);
+int nicp_multi_frame_store_create(nicp_shard_pool *pool, const int *raw_rows, const int *raw_cols, float depth_scale,
+                                  int step, float max_depth_cov, const nicp_multi_projector *mp,
+                                  const nicp_stats_params *sp, const float sensor_offset[16], nicp_frame_store **store);
+void nicp_frame_store_destroy(nicp_frame_store *store);
+/* copies n frames: frame f has id ids[f] and raw images raws[f * num_cameras + i] (one camera for a pinhole store), as in
+ * nicp_multi_align_frames_sharded; the caller may free them on return.  Every image must be exactly raw_rows[i] x
+ * raw_cols[i] (raw_rows x raw_cols for a pinhole store) as given when the store was created: the call copies that many
+ * pixels from each pointer and cannot see the caller's size (capi.FrameStore.add checks the shapes) */
+int nicp_frame_store_add(nicp_frame_store *store, int n, const long long *ids, const uint16_t *const *raws);
+/* forgets n frames: their raw copies are freed and no worker serves their clouds again (an id added again later is
+ * prepared from its new images) */
+int nicp_frame_store_remove(nicp_frame_store *store, int n, const long long *ids);
+/* frames in the store, -1 for a null store or one whose pool was destroyed */
+int nicp_frame_store_size(const nicp_frame_store *store);
+/* pair i = (reference_ids[i], current_ids[i]) with initial_guesses + 16 i (NULL: identity); priors / prior_offsets as in
+ * nicp_multi_align_batch (may be NULL), for pinhole and rig stores alike */
+int nicp_frame_store_align(nicp_frame_store *store, int n_pairs, const long long *reference_ids,
+                           const long long *current_ids, const float *initial_guesses, const nicp_prior *priors,
+                           const int *prior_offsets, const nicp_align_params *ap, float frame_inlier_depth_threshold,
+                           nicp_align_result *results);
+/* since the store was created, summed over the workers and over the windows of every call: frames a window prepared,
+ * and frames a window found resident (either output may be NULL) */
+int nicp_frame_store_counters(const nicp_frame_store *store, long long *frames_built, long long *frames_reused);
 
 #ifdef __cplusplus
 }
