@@ -29,7 +29,7 @@ SYMBOLS = [
     "nicp_multi_image_size", "nicp_multi_depth_to_cloud", "nicp_multi_project", "nicp_multi_align",
     "nicp_multi_raw_depth_to_cloud_batch", "nicp_multi_align_batch",
     "nicp_cloud_compute_gaussians", "nicp_cloud_has_gaussians", "nicp_cloud_download_gaussians",
-    "nicp_cloud_upload_gaussians", "nicp_merge", "nicp_voxelize",
+    "nicp_cloud_upload_gaussians", "nicp_merge", "nicp_voxelize", "nicp_raw_depth_to_local_map",
     "nicp_shard_pool_create", "nicp_shard_pool_destroy", "nicp_shard_pool_size", "nicp_align_frames_sharded",
     "nicp_multi_align_frames_sharded",
     "nicp_frame_store_create", "nicp_multi_frame_store_create", "nicp_frame_store_destroy", "nicp_frame_store_add",
@@ -479,6 +479,46 @@ class Context:
                                                             int(keep_stats), CA))
         self._keepalive = frames  # the copies are asynchronous: keep the host frames alive until the next call
         return clouds
+
+    def raw_depth_to_local_map(self, raws, proj, sp, poses, map_cloud, depth_scale=0.001, step=1, max_depth_cov=0.01,
+                               sensor_offset=None, baseline=0.075, alpha=0.1, merge_params=None, merge_transform=None,
+                               voxel_resolution=0.0):
+        """n raw frames (uint16 arrays of one shape) with n (4, 4) poses -> appended to map_cloud with their sensor-model
+        gaussians, then Merger::merge(merge_params, merge_transform; identity if None) if merge_params is given, then
+        VoxelCalculator::compute(voxel_resolution) if it is > 0 (nicp_raw_depth_to_local_map).  Synchronous.  Returns
+        (appended points, new size, collapsed indices of the merged points or None, voxel representatives or None).  A map
+        too small raises NicpError with `needed_size` (the size the map would need); the map is left as it was."""
+        n = len(raws)
+        frames = [r if (isinstance(r, np.ndarray) and r.dtype == np.uint16 and r.flags.c_contiguous)
+                  else np.ascontiguousarray(r, np.uint16) for r in raws]
+        rows, cols = frames[0].shape
+        assert all(f.shape == (rows, cols) for f in frames), "every raw frame needs the same shape"
+        P = np.asarray(poses, np.float32)
+        assert P.shape == (n, 4, 4), "one (4, 4) pose per frame"
+        pp = np.ascontiguousarray(P.transpose(0, 2, 1)).reshape(n, 16)
+        so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
+        mt = colmajor(np.eye(4) if merge_transform is None else merge_transform)
+        before = map_cloud.size()
+        collapsed = np.zeros(map_cloud.capacity, np.int32) if merge_params is not None else None
+        reps = np.zeros(map_cloud.capacity, np.int32) if voxel_resolution > 0 else None
+        RA = (C.c_void_p * max(n, 1))(*[f.ctypes.data for f in frames])
+        appended, new_size = C.c_int(0), C.c_int(0)
+        rc = self.L.nicp_raw_depth_to_local_map(
+            self.handle, n, RA, rows, cols, C.c_float(depth_scale), int(step), C.c_float(max_depth_cov), C.byref(proj),
+            C.byref(sp), _fptr(so), C.c_float(baseline), C.c_float(alpha), _fptr(pp),
+            C.byref(merge_params) if merge_params is not None else None, _fptr(mt), C.c_float(voxel_resolution),
+            map_cloud.handle, C.byref(appended), C.byref(new_size), _iptr(collapsed) if collapsed is not None else None,
+            _iptr(reps) if reps is not None else None)
+        if rc != NICP_OK:
+            err = NicpError("nicp error %d: %s" % (rc, self.L.nicp_last_error().decode()))
+            err.needed_size = new_size.value
+            raise err
+        merged = before + appended.value
+        if collapsed is not None:
+            collapsed = collapsed[:merged].copy()
+        if reps is not None:
+            reps = reps[:new_size.value].copy()
+        return appended.value, new_size.value, collapsed, reps
 
     def stats_compute(self, points, index, interval, sp):
         """StatsCalculatorIntegralImage::compute(normals, stats, points, indexImage) with its interval image"""

@@ -370,17 +370,6 @@ struct StatsConsts {
 
 __device__ __forceinline__ int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
-// R * Om * R^T for the 3x3 blocks (InformationMatrixVector::transformInPlace, informationmatrix.h:111-121)
-__device__ __forceinline__ void rotate_sym(const float *M, const float *Om /*3x3 col-major*/, float *out) {
-  float t[9];
-  for (int r = 0; r < 3; r++)
-    for (int c = 0; c < 3; c++)
-      NM3(t, r, c) = dot3(NM4(M, r, 0), NM4(M, r, 1), NM4(M, r, 2), NM3(Om, 0, c), NM3(Om, 1, c), NM3(Om, 2, c));
-  for (int r = 0; r < 3; r++)
-    for (int c = 0; c < 3; c++)
-      NM3(out, r, c) = dot3(NM3(t, r, 0), NM3(t, r, 1), NM3(t, r, 2), NM4(M, c, 0), NM4(M, c, 1), NM4(M, c, 2));
-}
-
 // StatsCalculatorIntegralImage::compute for one pixel (statscalculatorintegralimage.cpp:41-78): region sums of the window
 // of radius clamp(k), mean / covariance (pointaccumulator.h:65-86), computeDirect, curvature, normal orientation.
 // Returns false when the window holds fewer than minPoints points (outputs untouched).
@@ -475,10 +464,7 @@ __global__ void __launch_bounds__(256, 4) k_stats(PrepBatch B, int rows, int col
   // compacted index from channel 0 of the integral image (exact integer counts in float32)
   int idx;
   if (!MULTI) {
-    // raster order: valid pixels in the rows above + valid pixels of this row up to c
-    float above = r > 0 ? I[(size_t)(r - 1) * cols + cols - 1] : 0.0f;
-    float upto = I[pix] - (r > 0 ? I[pix - cols] : 0.0f);
-    idx = (int)above + (int)upto - 1;
+    idx = raster_rank(I, r, c, cols);
   } else {
     // MultiPointProjector::unProject concatenates the children's clouds (multipointprojector.cpp:59-90):
     // points of the earlier column blocks, then raster order inside this camera's block
@@ -1119,30 +1105,7 @@ __global__ void k_cloud_append(int srcCapacity, const int *__restrict__ srcN, co
   if (o >= (size_t)dstCapacity) return;
   float4 p = sp[i], nn = sn[i];
   float4 o0 = so[3 * (size_t)i], o1 = so[3 * (size_t)i + 1], o2 = so[3 * (size_t)i + 2];
-  if (!identity) {
-    float M16[16];
-    mat4_identity(M16);
-    for (int r = 0; r < 3; r++)
-      for (int c = 0; c < 4; c++) NM4(M16, r, c) = M.r[r][c];
-    float x, y, z;
-    xform_point(M, p.x, p.y, p.z, x, y, z);
-    p = make_float4(x, y, z, 1.0f);
-    xform_normal(M, nn.x, nn.y, nn.z, x, y, z);
-    nn = make_float4(x, y, z, nn.w);
-    float P6[6], N6[6];
-    omega_unpack(o0, o1, o2, P6, N6);
-    float OP[9] = {P6[0], P6[1], P6[2], P6[1], P6[3], P6[4], P6[2], P6[4], P6[5]};
-    float ON[9] = {N6[0], N6[1], N6[2], N6[1], N6[3], N6[4], N6[2], N6[4], N6[5]};
-    float tp[9], tn[9];
-    rotate_sym(M16, OP, tp);
-    rotate_sym(M16, ON, tn);
-    const float Q6[6] = {NM3(tp, 0, 0), NM3(tp, 0, 1), NM3(tp, 0, 2), NM3(tp, 1, 1), NM3(tp, 1, 2), NM3(tp, 2, 2)};
-    const float R6[6] = {NM3(tn, 0, 0), NM3(tn, 0, 1), NM3(tn, 0, 2), NM3(tn, 1, 1), NM3(tn, 1, 2), NM3(tn, 2, 2)};
-    const Omega3 w = omega_pack(Q6, R6);
-    o0 = w.o0;
-    o1 = w.o1;
-    o2 = w.o2;
-  }
+  if (!identity) xform_record(M, p, nn, o0, o1, o2);
   dp[o] = p;
   dn[o] = nn;
   dom[3 * o] = o0;

@@ -191,7 +191,36 @@ __global__ void k_valid_flags(const float *__restrict__ depth, int n, float minD
 }
 
 struct Mat3 { float m[9]; };
-// pinholepointprojector.cpp:104-123 for the valid pixels; slot = raster rank of the pixel
+// pinholepointprojector.cpp:104-123 for the valid pixel (r, c) of depth z: g = the gaussian in the moments form
+__device__ __forceinline__ void gauss_sensor_model(int r, int c, float z, const Mat3 &iK, const Affine &iKRt, float fB,
+                                                   float alpha, float *g) {
+#pragma unroll
+  for (int k = 0; k < kGF; k++) g[k] = 0.0f;
+  xform_point(iKRt, fmul((float)c, z), fmul((float)r, z), z, g[0], g[1], g[2]);
+  const float zVariation = fdiv(fmul(fmul(alpha, z), z), fadd(fB, fmul(z, alpha)));
+  float J0[9] = {z, 0.0f, 0.0f, 0.0f, z, 0.0f, (float)c, (float)r, 1.0f}, J[9], JD[9];
+  mat3_mul(iK.m, J0, J);
+  const float dg[3] = {3.0f, 3.0f, zVariation};
+  for (int j = 0; j < 3; j++)
+    for (int i = 0; i < 3; i++) NM3(JD, i, j) = fmul(NM3(J, i, j), dg[j]);
+  mat3_mul_bt(JD, J, g + 3);
+}
+// gaussian3.h:26-36 for one gaussian whose moments are up to date: mean' = R mean + t, cov' = (R cov) R^T
+__device__ __forceinline__ void gauss_xform_moments(const Affine &M, float *g) {
+  float R[9];
+  for (int r = 0; r < 3; r++)
+    for (int c = 0; c < 3; c++) NM3(R, r, c) = M.r[r][c];
+  float mean[3], RC[9], cov[9];
+  mat3_vec(R, g, mean);
+  g[0] = fadd(mean[0], M.r[0][3]);
+  g[1] = fadd(mean[1], M.r[1][3]);
+  g[2] = fadd(mean[2], M.r[2][3]);
+  mat3_mul(R, g + 3, RC);
+  mat3_mul_bt(RC, R, cov);
+  for (int k = 0; k < 9; k++) g[3 + k] = cov[k];
+}
+
+// the valid pixels of one depth image; slot = raster rank of the pixel
 __global__ void k_gaussians(const float *__restrict__ depth, const int *__restrict__ rank, int rows, int cols, float minD,
                             float maxD, Mat3 iK, Affine iKRt, float fB, float alpha, int capacity,
                             float *__restrict__ gauss, int *__restrict__ gflags) {
@@ -203,16 +232,7 @@ __global__ void k_gaussians(const float *__restrict__ depth, const int *__restri
   if (slot >= capacity) return;
   const int r = pix / cols, c = pix - r * cols;
   float g[kGF];
-#pragma unroll
-  for (int k = 0; k < kGF; k++) g[k] = 0.0f;
-  xform_point(iKRt, fmul((float)c, z), fmul((float)r, z), z, g[0], g[1], g[2]);
-  const float zVariation = fdiv(fmul(fmul(alpha, z), z), fadd(fB, fmul(z, alpha)));
-  float J0[9] = {z, 0.0f, 0.0f, 0.0f, z, 0.0f, (float)c, (float)r, 1.0f}, J[9], JD[9];
-  mat3_mul(iK.m, J0, J);
-  const float dg[3] = {3.0f, 3.0f, zVariation};
-  for (int j = 0; j < 3; j++)
-    for (int i = 0; i < 3; i++) NM3(JD, i, j) = fmul(NM3(J, i, j), dg[j]);
-  mat3_mul_bt(JD, J, g + 3);
+  gauss_sensor_model(r, c, z, iK, iKRt, fB, alpha, g);
   gauss_store(gauss + (size_t)kGF * slot, g);
   gflags[slot] = NICP_GAUSS_MOMENTS;
 }
@@ -229,17 +249,7 @@ __global__ void k_gauss_transform(float *__restrict__ gauss, int *__restrict__ g
   gauss_load(gauss + (size_t)kGF * i, g);
   int f = gflags[i];
   gauss_update_moments(g, f);
-  float R[9];
-  for (int r = 0; r < 3; r++)
-    for (int c = 0; c < 3; c++) NM3(R, r, c) = M.r[r][c];
-  float mean[3], RC[9], cov[9];
-  mat3_vec(R, g, mean);
-  g[0] = fadd(mean[0], M.r[0][3]);
-  g[1] = fadd(mean[1], M.r[1][3]);
-  g[2] = fadd(mean[2], M.r[2][3]);
-  mat3_mul(R, g + 3, RC);
-  mat3_mul_bt(RC, R, cov);
-  for (int k = 0; k < 9; k++) g[3 + k] = cov[k];
+  gauss_xform_moments(M, g);
   gauss_store(gauss + (size_t)kGF * i, g);
   gflags[i] = NICP_GAUSS_MOMENTS;
 }
@@ -288,17 +298,7 @@ __global__ void k_gauss_append(const float *__restrict__ sg, const int *__restri
   int f = sf[i];
   if (!identity) {
     gauss_update_moments(g, f);
-    float R[9];
-    for (int r = 0; r < 3; r++)
-      for (int c = 0; c < 3; c++) NM3(R, r, c) = M.r[r][c];
-    float mean[3], RC[9], cov[9];
-    mat3_vec(R, g, mean);
-    g[0] = fadd(mean[0], M.r[0][3]);
-    g[1] = fadd(mean[1], M.r[1][3]);
-    g[2] = fadd(mean[2], M.r[2][3]);
-    mat3_mul(R, g + 3, RC);
-    mat3_mul_bt(RC, R, cov);
-    for (int k = 0; k < 9; k++) g[3 + k] = cov[k];
+    gauss_xform_moments(M, g);
     f = NICP_GAUSS_MOMENTS;
   }
   gauss_store(dg + kGF * o, g);
@@ -324,6 +324,23 @@ int launch_gauss_append(nicp_context *ctx, nicp_cloud *dst, const nicp_cloud *sr
   return NICP_OK;
 }
 
+// host-side constants of the sensor model: unProject matrix with the projector at identity, K^-1, baseline * fx
+struct SensorModel {
+  Affine iKRt;
+  Mat3 iK;
+  float fB;
+};
+static SensorModel sensor_model(const nicp_projector *proj, float baseline) {
+  SensorModel s;
+  float I4[16], iKRt[16];
+  mat4_identity(I4);
+  compute_iKRt(proj->K, I4, iKRt);
+  s.iKRt = affine_from(iKRt);
+  mat3_inverse(proj->K, s.iK.m);
+  s.fB = fmul(baseline, NM3(proj->K, 0, 0));
+  return s;
+}
+
 // depth: host image.  The cloud must have been built from the same image, projector and sensor offset.
 int run_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *depth, const nicp_projector *proj,
                           float baseline, float alpha, const float sensorOffset[16]) {
@@ -339,14 +356,9 @@ int run_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *dep
   k_valid_flags<<<(P + 255) / 256, 256, 0, ctx->stream>>>(d_depth, P, proj->min_distance, proj->max_distance, d_flags);
   NICP_CHECK_LAUNCH(ctx);
   if ((rc = exclusive_scan(ctx, d_flags, d_rank, P, d_scan, d_total))) return rc;
-  float I4[16], iKRt[16];
-  mat4_identity(I4);
-  compute_iKRt(proj->K, I4, iKRt);
-  Mat3 iK;
-  mat3_inverse(proj->K, iK.m);
-  const float fB = fmul(baseline, NM3(proj->K, 0, 0));
+  const SensorModel sm = sensor_model(proj, baseline);
   k_gaussians<<<(P + 127) / 128, 128, 0, ctx->stream>>>(d_depth, d_rank, proj->rows, proj->cols, proj->min_distance,
-                                                        proj->max_distance, iK, affine_from(iKRt), fB, alpha, cloud->capacity,
+                                                        proj->max_distance, sm.iK, sm.iKRt, sm.fB, alpha, cloud->capacity,
                                                         cloud->gauss, cloud->gflags);
   NICP_CHECK_LAUNCH(ctx);
   int total = 0;
@@ -360,6 +372,155 @@ int run_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *dep
   }
   if ((rc = launch_gauss_transform(ctx, cloud, nullptr, 0, cloud->d_n, n, sensorOffset))) return rc;
   cloud->has_gauss = true;
+  return NICP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// local map from one launch set of the batched frame preparation (nicp_raw_depth_to_local_map)
+// ---------------------------------------------------------------------------------------------
+// The frame clouds of the set (frame f = blockIdx.y), the poses they are appended with and the sensor offset of their
+// gaussians: a kernel parameter, like PrepBatch.
+struct LocalMapSet {
+  const float4 *points[kMaxPrepBatch], *normals[kMaxPrepBatch], *omega[kMaxPrepBatch];
+  float *gauss[kMaxPrepBatch];
+  int *gflags[kMaxPrepBatch];
+  const int *count[kMaxPrepBatch];
+  Affine pose[kMaxPrepBatch];
+  int poseIdentity[kMaxPrepBatch];
+  Affine offset;
+  int offsetIdentity;
+};
+
+// nicp_cloud_compute_gaussians for every frame of the set, from the depth and integral images the set's preparation left
+// in the batch scratch: the slot of a valid pixel is its raster rank from channel 0 of the integral image (the compacted
+// index k_stats wrote the point to), then the sensor offset as a second rounded step (k_gauss_transform).
+__global__ void k_local_map_gaussians(LocalMapSet S, const float *__restrict__ depth0, const float *__restrict__ integral0,
+                                      size_t framePixels, int rows, int cols, float minD, float maxD, Mat3 iK, Affine iKRt,
+                                      float fB, float alpha) {
+  const int f = blockIdx.y;
+  const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pix >= rows * cols) return;
+  const float z = depth0[(size_t)f * framePixels + pix];
+  if (z < minD || z > maxD) return;
+  const int r = pix / cols, c = pix - r * cols;
+  const int slot = raster_rank(integral0 + (size_t)f * framePixels * kIntegralCh, r, c, cols);
+  float g[kGF];
+  gauss_sensor_model(r, c, z, iK, iKRt, fB, alpha, g);
+  if (!S.offsetIdentity) gauss_xform_moments(S.offset, g);
+  gauss_store(S.gauss[f] + (size_t)kGF * slot, g);
+  S.gflags[f][slot] = NICP_GAUSS_MOMENTS;
+}
+
+// Cloud::add (cloud.cpp:145-171) of every frame cloud of the set, in frame order, behind *run points: point record and
+// gaussian of point i of frame f moved by pose f (k_cloud_append, k_gauss_append).  A set that does not fit below
+// dstCapacity writes nothing; *run advances regardless (k_local_map_advance), so the final count is the size the map needs.
+__global__ void __launch_bounds__(256) k_local_map_append(LocalMapSet S, int m, const long long *__restrict__ run,
+                                                          int dstCapacity, float4 *__restrict__ dp, float4 *__restrict__ dn,
+                                                          float4 *__restrict__ dom, float *__restrict__ dg,
+                                                          int *__restrict__ df) {
+  const int f = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int n = *S.count[f];
+  if (i >= n) return;
+  long long before = 0, total = 0;
+  for (int k = 0; k < m; k++) {
+    const int nk = *S.count[k];
+    if (k < f) before += nk;
+    total += nk;
+  }
+  const long long base = *run;
+  if (base + total > dstCapacity) return;
+  const size_t o = (size_t)(base + before + i);
+  float4 p = S.points[f][i], nn = S.normals[f][i];
+  const float4 *so = S.omega[f] + 3 * (size_t)i;
+  float4 o0 = so[0], o1 = so[1], o2 = so[2];
+  float g[kGF];
+  gauss_load(S.gauss[f] + (size_t)kGF * i, g);
+  int gf = S.gflags[f][i];
+  if (!S.poseIdentity[f]) {
+    xform_record(S.pose[f], p, nn, o0, o1, o2);
+    gauss_update_moments(g, gf);
+    gauss_xform_moments(S.pose[f], g);
+    gf = NICP_GAUSS_MOMENTS;
+  }
+  dp[o] = p;
+  dn[o] = nn;
+  dom[3 * o] = o0;
+  dom[3 * o + 1] = o1;
+  dom[3 * o + 2] = o2;
+  gauss_store(dg + kGF * o, g);
+  df[o] = gf;
+}
+__global__ void k_local_map_advance(LocalMapSet S, int m, long long *run) {
+  long long total = 0;
+  for (int k = 0; k < m; k++) total += *S.count[k];
+  *run += total;
+}
+__global__ void k_local_map_begin(long long *run, const int *mapN) { *run = *mapN; }
+__global__ void k_local_map_commit(int *mapN, const long long *run) { *mapN = (int)*run; }
+
+int launch_local_map_begin(nicp_context *ctx, nicp_cloud *map, long long *d_run) {
+  if (!map->has_gauss) {  // points the map already holds get default (all-zero) gaussians, as in launch_gauss_append
+    int rc = cloud_ensure_gaussians(ctx, map);
+    if (rc) return rc;
+    NICP_CUDA(cudaMemsetAsync(map->gauss, 0, sizeof(float) * kGF * (size_t)map->capacity, ctx->stream));
+    NICP_CUDA(cudaMemsetAsync(map->gflags, 0, sizeof(int) * (size_t)map->capacity, ctx->stream));
+  }
+  k_local_map_begin<<<1, 1, 0, ctx->stream>>>(d_run, map->d_n);
+  NICP_CHECK_LAUNCH(ctx);
+  return NICP_OK;
+}
+
+// the m frame clouds of the launch set that launch_raw_prep_batch has just queued (its depth and integral images are still
+// in the batch scratch): gaussians, then one append launch behind *d_run
+int launch_local_map_set(nicp_context *ctx, const nicp_projector *proj, int m, nicp_cloud *const *frames, const float *poses,
+                         float baseline, float alpha, const float sensorOffset[16], nicp_cloud *map, long long *d_run) {
+  const int P = proj->rows * proj->cols;
+  LocalMapSet S;
+  memset(&S, 0, sizeof S);
+  for (int f = 0; f < m; f++) {
+    int rc = cloud_ensure_gaussians(ctx, frames[f]);
+    if (rc) return rc;
+    S.points[f] = frames[f]->points;
+    S.normals[f] = frames[f]->normals;
+    S.omega[f] = frames[f]->omega;
+    S.gauss[f] = frames[f]->gauss;
+    S.gflags[f] = frames[f]->gflags;
+    S.count[f] = frames[f]->d_n;
+    float T[16];
+    for (int k = 0; k < 16; k++) T[k] = poses[16 * f + k];
+    fix_last_row(T);
+    S.pose[f] = affine_from(T);
+    S.poseIdentity[f] = is_identity16(T) ? 1 : 0;
+    frames[f]->has_gauss = true;
+  }
+  float M[16];
+  for (int k = 0; k < 16; k++) M[k] = sensorOffset[k];
+  fix_last_row(M);
+  S.offset = affine_from(M);
+  S.offsetIdentity = is_identity16(M) ? 1 : 0;
+  const SensorModel sm = sensor_model(proj, baseline);
+  k_local_map_gaussians<<<dim3((P + 127) / 128, m), 128, 0, ctx->stream>>>(S, ctx->d_bDepth, ctx->d_bIntegral, ctx->batchPixels,
+                                                                          proj->rows, proj->cols, proj->min_distance,
+                                                                          proj->max_distance, sm.iK, sm.iKRt, sm.fB, alpha);
+  NICP_CHECK_LAUNCH(ctx);
+  k_local_map_append<<<dim3((P + 255) / 256, m), 256, 0, ctx->stream>>>(S, m, d_run, map->capacity, map->points, map->normals,
+                                                                        map->omega, map->gauss, map->gflags);
+  NICP_CHECK_LAUNCH(ctx);
+  k_local_map_advance<<<1, 1, 0, ctx->stream>>>(S, m, d_run);
+  NICP_CHECK_LAUNCH(ctx);
+  return NICP_OK;
+}
+
+// the map takes the appended points: count from the device, flags and caches like nicp_cloud_append
+int launch_local_map_commit(nicp_context *ctx, nicp_cloud *map, const long long *d_run, int newSize) {
+  k_local_map_commit<<<1, 1, 0, ctx->stream>>>(map->d_n, d_run);
+  NICP_CHECK_LAUNCH(ctx);
+  map->points3_valid = false; map->pn_valid = false;
+  map->has_stats = false;
+  map->has_gauss = true;
+  map->n_host = newSize;
+  map->n_known = true;
   return NICP_OK;
 }
 

@@ -349,6 +349,43 @@ int frames_rig(const nicp_multi_projector *mp, const int *rawRows, const int *ra
   return NICP_OK;
 }
 
+// frames per launch set of the batched prep for n frames of fs
+static int prep_set_frames(const FrameSet &fs, int n) {
+  return std::min({env_int("NICP_PREP_BATCH", kMaxPrepBatch), fs.prepFrames, n});
+}
+
+// one launch set: m <= ctx->batchSlots raw frames (raws[f * fs.cams.n + i] = camera i of frame f) -> clouds[0 .. m).  The raw
+// frames of set k are uploaded on the copy stream into staging set k & 1 while set k - 1 computes; the cameras of a frame
+// sit back to back in its staging slot.
+static int prep_set(nicp_context *ctx, const FrameSet &fs, int m, const uint16_t *const *raws, const nicp_stats_params *sp,
+                    const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds) {
+  const int nc = fs.cams.n;
+  const int b = (ctx->bRawToggle ^= 1);
+  uint16_t *stage = ctx->d_bRaw + (size_t)b * ctx->batchSlots * ctx->batchRawPixels;
+  const uint16_t *d_raw[kMaxPrepBatch * kMaxCams];
+  NICP_CUDA(cudaStreamWaitEvent(ctx->copyStream, ctx->evBRawUsed[b], 0));
+  for (int f = 0; f < m; f++) {
+    uint16_t *dst = stage + (size_t)f * ctx->batchRawPixels;
+    for (int i = 0; i < nc; i++) {
+      const size_t cpx = (size_t)fs.rawRows[i] * fs.rawCols[i];
+      NICP_CUDA(cudaMemcpyAsync(dst, raws[(size_t)f * nc + i], cpx * sizeof(uint16_t), cudaMemcpyHostToDevice,
+                                ctx->copyStream));
+      d_raw[f * nc + i] = dst;
+      dst += cpx;
+    }
+  }
+  NICP_CUDA(cudaEventRecord(ctx->evBRawCopied[b], ctx->copyStream));
+  NICP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evBRawCopied[b], 0));
+  int rc;
+  for (int f = 0; f < m; f++)
+    if (keepStats && (rc = ensure_stats(clouds[f]))) return rc;
+  float eye[16];
+  mat4_identity(eye);
+  if ((rc = launch_raw_prep_batch(ctx, fs, m, d_raw, sp, sensorOffset ? sensorOffset : eye, keepStats, clouds))) return rc;
+  NICP_CUDA(cudaEventRecord(ctx->evBRawUsed[b], ctx->stream));
+  return NICP_OK;
+}
+
 // n raw frames of fs -> clouds[0 .. n), asynchronously: raws[f * fs.cams.n + i] = camera i of frame f
 int prep_frames(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *raws, const nicp_stats_params *sp,
                 const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds) {
@@ -379,37 +416,12 @@ int prep_frames(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *co
         return NICP_ERR_INVALID;
       }
   }
-  const int sub = std::min({env_int("NICP_PREP_BATCH", kMaxPrepBatch), fs.prepFrames, n});
+  const int sub = prep_set_frames(fs, n);
   int rc;
   if ((rc = ensure_batch_prep(ctx, sub, px, fs.rawPixels))) return rc;
-  float eye[16];
-  mat4_identity(eye);
-  for (int base = 0; base < n; base += sub) {
-    const int m = n - base < sub ? n - base : sub;
-    // raw frames of sub-batch k are uploaded on the copy stream into staging set k & 1 while sub-batch k - 1 computes; the
-    // cameras of a frame sit back to back in its staging slot
-    const int b = (ctx->bRawToggle ^= 1);
-    uint16_t *stage = ctx->d_bRaw + (size_t)b * ctx->batchSlots * ctx->batchRawPixels;
-    const uint16_t *d_raw[kMaxPrepBatch * kMaxCams];
-    NICP_CUDA(cudaStreamWaitEvent(ctx->copyStream, ctx->evBRawUsed[b], 0));
-    for (int f = 0; f < m; f++) {
-      uint16_t *dst = stage + (size_t)f * ctx->batchRawPixels;
-      for (int i = 0; i < nc; i++) {
-        const size_t cpx = (size_t)fs.rawRows[i] * fs.rawCols[i];
-        NICP_CUDA(cudaMemcpyAsync(dst, raws[(size_t)(base + f) * nc + i], cpx * sizeof(uint16_t), cudaMemcpyHostToDevice,
-                                  ctx->copyStream));
-        d_raw[f * nc + i] = dst;
-        dst += cpx;
-      }
-    }
-    NICP_CUDA(cudaEventRecord(ctx->evBRawCopied[b], ctx->copyStream));
-    NICP_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->evBRawCopied[b], 0));
-    for (int f = 0; f < m; f++)
-      if (keepStats && (rc = ensure_stats(clouds[base + f]))) return rc;
-    if ((rc = launch_raw_prep_batch(ctx, fs, m, d_raw, sp, sensorOffset ? sensorOffset : eye, keepStats, clouds + base)))
+  for (int base = 0; base < n; base += sub)
+    if ((rc = prep_set(ctx, fs, std::min(sub, n - base), raws + (size_t)base * nc, sp, sensorOffset, keepStats, clouds + base)))
       return rc;
-    NICP_CUDA(cudaEventRecord(ctx->evBRawUsed[b], ctx->stream));
-  }
   ctx->lastRows = 0;  // the single-frame test hooks (integral / interval image) describe no frame of a batch
   return NICP_OK;
 }
@@ -672,6 +684,11 @@ void nicp_destroy(nicp_context *ctx) {
   if (ctx->d_priors) cudaFree(ctx->d_priors);
   if (ctx->d_cams) cudaFree(ctx->d_cams);
   if (ctx->d_mapScratch) cudaFree(ctx->d_mapScratch);
+  for (nicp_cloud *&c : ctx->lmFrames) {
+    nicp_cloud_destroy(c);
+    c = nullptr;
+  }
+  dev_free(ctx->d_lmRun);
   dev_free(ctx->d_results);
   dev_free(ctx->d_statHb);
   if (ctx->h_results) cudaFreeHost(ctx->h_results);
@@ -1083,6 +1100,79 @@ int nicp_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *cons
   FrameSet fs;
   int rc = frames_pinhole(proj, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs);
   return rc ? rc : prep_frames(ctx, fs, n, raws, sp, sensor_offset, keep_stats, clouds);
+}
+
+// the frame clouds of one launch set of `sub` frames of px pixels, and the running count of the map being built
+static int ensure_local_map_frames(nicp_context *ctx, int sub, size_t px) {
+  for (int f = 0; f < sub; f++) {
+    nicp_cloud *&c = ctx->lmFrames[f];
+    if (c && (size_t)c->capacity < px) {
+      nicp_cloud_destroy(c);
+      c = nullptr;
+    }
+    int rc;
+    if (!c && (rc = nicp_cloud_create(ctx, (int)px, &c))) return rc;
+  }
+  return ctx->d_lmRun ? NICP_OK : dev_alloc(&ctx->d_lmRun, 1);
+}
+
+int nicp_raw_depth_to_local_map(nicp_context *ctx, int n, const uint16_t *const *raws, int raw_rows, int raw_cols,
+                                float depth_scale, int step, float max_depth_cov, const nicp_projector *proj,
+                                const nicp_stats_params *sp, const float sensor_offset[16], float baseline, float alpha,
+                                const float *poses, const nicp_merge_params *merge_params, const float merge_transform[16],
+                                float voxel_resolution, nicp_cloud *map, int *appended_size, int *new_size, int *collapsed,
+                                int *representatives) {
+  if (!ctx || n <= 0 || !raws || !proj || !sp || !sensor_offset || !poses || !map || raw_rows <= 0 || raw_cols <= 0 ||
+      proj->rows <= 0 || proj->cols <= 0)
+    return NICP_ERR_INVALID;
+  if (merge_params && !merge_transform) {
+    set_error("nicp_raw_depth_to_local_map: merge_params without merge_transform");
+    return NICP_ERR_INVALID;
+  }
+  for (int f = 0; f < n; f++)
+    if (!raws[f]) {
+      set_error("null raw image of frame %d", f);
+      return NICP_ERR_INVALID;
+    }
+  if (map->device != ctx->device) {
+    set_error("the map lives on GPU %d, the context on GPU %d", map->device, ctx->device);
+    return NICP_ERR_INVALID;
+  }
+  FrameSet fs;
+  int rc;
+  if ((rc = frames_pinhole(proj, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs))) return rc;
+  NICP_CUDA(cudaSetDevice(ctx->device));
+  const size_t px = (size_t)proj->rows * proj->cols;
+  const int sub = prep_set_frames(fs, n);
+  if ((rc = ensure_batch_prep(ctx, sub, px, fs.rawPixels)) || (rc = ensure_local_map_frames(ctx, sub, px))) return rc;
+  if ((rc = launch_local_map_begin(ctx, map, ctx->d_lmRun))) return rc;
+  for (int base = 0; base < n; base += sub) {
+    const int m = std::min(sub, n - base);
+    if ((rc = prep_set(ctx, fs, m, raws + base, sp, sensor_offset, 0, ctx->lmFrames)) ||
+        (rc = launch_local_map_set(ctx, proj, m, ctx->lmFrames, poses + 16 * (size_t)base, baseline, alpha, sensor_offset,
+                                   map, ctx->d_lmRun)))
+      return rc;
+  }
+  ctx->lastRows = 0;
+  long long run = 0;
+  int before = 0;
+  NICP_CUDA(cudaMemcpyAsync(&run, ctx->d_lmRun, sizeof run, cudaMemcpyDeviceToHost, ctx->stream));
+  NICP_CUDA(cudaMemcpyAsync(&before, map->d_n, sizeof before, cudaMemcpyDeviceToHost, ctx->stream));
+  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (appended_size) *appended_size = (int)std::min<long long>(run - before, INT_MAX);
+  if (run > map->capacity) {
+    if (new_size) *new_size = (int)std::min<long long>(run, INT_MAX);
+    set_error("nicp_raw_depth_to_local_map: %d + %lld points exceed the map's capacity %d", before, run - before,
+              map->capacity);
+    return NICP_ERR_INVALID;
+  }
+  if ((rc = launch_local_map_commit(ctx, map, ctx->d_lmRun, (int)run))) return rc;
+  int size = (int)run;
+  if (merge_params && (rc = nicp_merge(ctx, map, proj, merge_transform, merge_params, collapsed, &size))) return rc;
+  if (voxel_resolution > 0.0f && (rc = nicp_voxelize(ctx, map, voxel_resolution, representatives, &size))) return rc;
+  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (new_size) *new_size = size;
+  return NICP_OK;
 }
 
 int nicp_multi_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *const *raws, const int *raw_rows,

@@ -94,6 +94,42 @@ __host__ __device__ inline void omega_unpack(const float4 &o0, const float4 &o1,
   P6[2] = o1.x; N6[2] = o1.y; P6[3] = o1.z; N6[3] = o1.w;
   P6[4] = o2.x; N6[4] = o2.y; P6[5] = o2.z; N6[5] = o2.w;
 }
+#if defined(__CUDACC__)
+// Cloud::add (cloud.cpp:145-171) of one point record: point, normal (w = curvature kept) and both information matrices
+// (Omega3 layout) moved by M
+__device__ __forceinline__ void xform_record(const Affine &M, float4 &p, float4 &nn, float4 &o0, float4 &o1, float4 &o2) {
+  float M16[16];
+  mat4_identity(M16);
+  for (int r = 0; r < 3; r++)
+    for (int c = 0; c < 4; c++) NM4(M16, r, c) = M.r[r][c];
+  float x, y, z;
+  xform_point(M, p.x, p.y, p.z, x, y, z);
+  p = make_float4(x, y, z, 1.0f);
+  xform_normal(M, nn.x, nn.y, nn.z, x, y, z);
+  nn = make_float4(x, y, z, nn.w);
+  float P6[6], N6[6];
+  omega_unpack(o0, o1, o2, P6, N6);
+  float OP[9] = {P6[0], P6[1], P6[2], P6[1], P6[3], P6[4], P6[2], P6[4], P6[5]};
+  float ON[9] = {N6[0], N6[1], N6[2], N6[1], N6[3], N6[4], N6[2], N6[4], N6[5]};
+  float tp[9], tn[9];
+  rotate_sym(M16, OP, tp);
+  rotate_sym(M16, ON, tn);
+  const float Q6[6] = {NM3(tp, 0, 0), NM3(tp, 0, 1), NM3(tp, 0, 2), NM3(tp, 1, 1), NM3(tp, 1, 2), NM3(tp, 2, 2)};
+  const float R6[6] = {NM3(tn, 0, 0), NM3(tn, 0, 1), NM3(tn, 0, 2), NM3(tn, 1, 1), NM3(tn, 1, 2), NM3(tn, 2, 2)};
+  const Omega3 w = omega_pack(Q6, R6);
+  o0 = w.o0;
+  o1 = w.o1;
+  o2 = w.o2;
+}
+// Compacted (raster-order) index of a valid pixel (r, c) of a pinhole image, read from channel 0 of its float32 integral
+// image I (exact integer counts): valid pixels in the rows above + valid pixels of this row up to c
+__device__ __forceinline__ int raster_rank(const float *__restrict__ I, int r, int c, int cols) {
+  const size_t pix = (size_t)r * cols + c;
+  const float above = r > 0 ? I[(size_t)(r - 1) * cols + cols - 1] : 0.0f;
+  const float upto = I[pix] - (r > 0 ? I[pix - cols] : 0.0f);
+  return (int)above + (int)upto - 1;
+}
+#endif
 
 // accumulator slot layout of the fused correspondence+linearise reduction
 enum {
@@ -360,6 +396,10 @@ struct nicp_context {
   // local-map maintenance scratch (map_ops.cu), grow-only
   void *d_mapScratch;
   size_t mapScratchBytes;
+  // nicp_raw_depth_to_local_map: the frame clouds of one prep launch set (reused set to set and call to call) and the
+  // running point count of the map being built
+  nicp_cloud *lmFrames[nicp::kMaxPrepBatch];
+  long long *d_lmRun;
 
   // last single-align bookkeeping
   int lastAlignRows, lastAlignCols, lastAlignIters, lastAlignParity, lastAlignEpoch;
@@ -451,6 +491,10 @@ int launch_gauss_transform(nicp_context *ctx, nicp_cloud *cloud, const int *d_fi
 int launch_gauss_append(nicp_context *ctx, nicp_cloud *dst, const nicp_cloud *src, const float T[16]);
 int run_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *depth, const nicp_projector *proj,
                           float baseline, float alpha, const float sensorOffset[16]);
+int launch_local_map_begin(nicp_context *ctx, nicp_cloud *map, long long *d_run);
+int launch_local_map_set(nicp_context *ctx, const nicp_projector *proj, int m, nicp_cloud *const *frames, const float *poses,
+                         float baseline, float alpha, const float sensorOffset[16], nicp_cloud *map, long long *d_run);
+int launch_local_map_commit(nicp_context *ctx, nicp_cloud *map, const long long *d_run, int newSize);
 int run_merge(nicp_context *ctx, nicp_cloud *cloud, const nicp_projector *proj, const float transform[16],
               const nicp_merge_params *mp, int n, int *collapsedHost, int *newSize);
 int run_voxelize(nicp_context *ctx, nicp_cloud *cloud, float resolution, int n, int *repHost, int *newSize);

@@ -162,6 +162,18 @@ NICP_HD void iso_mul(const float *A, const float *B, float *C) {
   for (int i = 0; i < 16; i++) C[i] = o[i];
 }
 
+// R * Om * R^T for the 3x3 blocks, R = the rotation of the 4x4 M (InformationMatrixVector::transformInPlace,
+// informationmatrix.h:111-121)
+NICP_HD void rotate_sym(const float *M, const float *Om /*3x3 col-major*/, float *out) {
+  float t[9];
+  for (int r = 0; r < 3; r++)
+    for (int c = 0; c < 3; c++)
+      NM3(t, r, c) = dot3(NM4(M, r, 0), NM4(M, r, 1), NM4(M, r, 2), NM3(Om, 0, c), NM3(Om, 1, c), NM3(Om, 2, c));
+  for (int r = 0; r < 3; r++)
+    for (int c = 0; c < 3; c++)
+      NM3(out, r, c) = dot3(NM3(t, r, 0), NM3(t, r, 1), NM3(t, r, 2), NM4(M, c, 0), NM4(M, c, 1), NM4(M, c, 2));
+}
+
 // ---- PinholePointProjector::_updateMatrices (pinholepointprojector.cpp:17-31) ---------------
 NICP_HD float cof3(const float *m, int i, int j) {
   int i1 = (i + 1) % 3, i2 = (i + 2) % 3, j1 = (j + 1) % 3, j2 = (j + 2) % 3;

@@ -257,6 +257,24 @@ int nicp_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *cons
                                   float depth_scale, int step, float max_depth_cov, const nicp_projector *proj,
                                   const nicp_stats_params *sp, const float sensor_offset[16], int keep_stats,
                                   nicp_cloud *const *clouds);
+/* Local map from n raw pinhole frames in one call.  Frame i is prepared like nicp_raw_depth_to_cloud (keep_stats 0), gets
+ * the sensor-model gaussians of nicp_cloud_compute_gaussians (baseline, alpha, sensor_offset) and is appended to `map` with
+ * poses + 16 * i (column-major 4x4) like nicp_cloud_append, in frame order, behind the points the map already holds (with
+ * or without gaussians).  Then, if merge_params != NULL, nicp_merge(map, proj, merge_transform, merge_params); then, if
+ * voxel_resolution > 0, nicp_voxelize(map, voxel_resolution).  The map is byte-identical to that chain of calls.  Frames
+ * are prepared in launch sets of up to 8 as in nicp_raw_depth_to_cloud_batch; the gaussians come from the set's device
+ * depth images and each set is appended by one launch, with no host round trip per frame.  The frame clouds of one set
+ * are scratch of the context, reused by the next set and the next call.
+ * Outputs (each may be NULL): appended_size = points the frames added; new_size = the map's final size; collapsed
+ * (nicp_merge) and representatives (nicp_voxelize) need room for map->capacity ints.  If the appended points do not fit,
+ * the call returns NICP_ERR_INVALID with new_size = the size the map would need, and the map keeps its size and its points.
+ * Synchronous. */
+int nicp_raw_depth_to_local_map(nicp_context *ctx, int n, const uint16_t *const *raws, int raw_rows, int raw_cols,
+                                float depth_scale, int step, float max_depth_cov, const nicp_projector *proj,
+                                const nicp_stats_params *sp, const float sensor_offset[16], float baseline, float alpha,
+                                const float *poses, const nicp_merge_params *merge_params,
+                                const float merge_transform[16], float voxel_resolution, nicp_cloud *map,
+                                int *appended_size, int *new_size, int *collapsed, int *representatives);
 /* ---- stage-level virtuals of the converter (SURVEY.md section 8b) ------------------------------------------------
  * StatsCalculatorIntegralImage::compute(normals, statsVector, points, indexImage) with the calculator's _intervalImage
  * (statscalculator.h:36, statscalculatorintegralimage.h:37 / .cpp:14-82): PointIntegralImage::compute over
