@@ -28,8 +28,9 @@ SYMBOLS = [
     "nicp_align", "nicp_align_get_state", "nicp_align_get_trace", "nicp_align_batch", "nicp_align_batch_priors",
     "nicp_multi_image_size", "nicp_multi_depth_to_cloud", "nicp_multi_project", "nicp_multi_align",
     "nicp_multi_raw_depth_to_cloud_batch", "nicp_multi_align_batch",
-    "nicp_cloud_compute_gaussians", "nicp_cloud_has_gaussians", "nicp_cloud_download_gaussians",
-    "nicp_cloud_upload_gaussians", "nicp_merge", "nicp_voxelize", "nicp_raw_depth_to_local_map",
+    "nicp_cloud_compute_gaussians", "nicp_multi_cloud_compute_gaussians", "nicp_cloud_has_gaussians",
+    "nicp_cloud_download_gaussians", "nicp_cloud_upload_gaussians", "nicp_merge", "nicp_voxelize",
+    "nicp_raw_depth_to_local_map", "nicp_multi_raw_depth_to_local_map",
     "nicp_shard_pool_create", "nicp_shard_pool_destroy", "nicp_shard_pool_size", "nicp_align_frames_sharded",
     "nicp_multi_align_frames_sharded",
     "nicp_frame_store_create", "nicp_multi_frame_store_create", "nicp_frame_store_destroy", "nicp_frame_store_add",
@@ -193,6 +194,14 @@ def _rig_frames(frames, nc):
     return imgs, np.array([s[0] for s in shapes], np.int32), np.array([s[1] for s in shapes], np.int32)
 
 
+def _per_camera(v, mp):
+    """a scalar for every camera of the rig, or one value per camera -> mp.num_cameras float32"""
+    a = np.asarray(v, np.float32)
+    a = np.full(mp.num_cameras, a, np.float32) if a.ndim == 0 else np.ascontiguousarray(a)
+    assert a.shape == (mp.num_cameras,), "one value per camera"
+    return a
+
+
 def make_projector(K, rows, cols, min_distance=0.01, max_distance=6.0):
     p = Projector()
     p.K[:] = colmajor(K).tolist()
@@ -323,6 +332,15 @@ class Cloud:
         so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
         _check(self.ctx.L, self.ctx.L.nicp_cloud_compute_gaussians(self.ctx.handle, self.handle, _fptr(d), C.byref(proj),
                                                                     C.c_float(baseline), C.c_float(alpha), _fptr(so)))
+
+    def multi_compute_gaussians(self, depth, mp, baseline=0.075, alpha=0.1, sensor_offset=None):
+        """the rig gaussians (nicp_multi_cloud_compute_gaussians) for the composite depth image this cloud was built from;
+        baseline / alpha: a scalar for every camera or one value per camera"""
+        d = np.ascontiguousarray(depth, np.float32)
+        so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
+        b, a = _per_camera(baseline, mp), _per_camera(alpha, mp)
+        _check(self.ctx.L, self.ctx.L.nicp_multi_cloud_compute_gaussians(self.ctx.handle, self.handle, _fptr(d), C.byref(mp),
+                                                                          _fptr(b), _fptr(a), _fptr(so)))
 
     def has_gaussians(self):
         return bool(self.ctx.L.nicp_cloud_has_gaussians(self.handle))
@@ -498,17 +516,48 @@ class Context:
         pp = np.ascontiguousarray(P.transpose(0, 2, 1)).reshape(n, 16)
         so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
         mt = colmajor(np.eye(4) if merge_transform is None else merge_transform)
+        RA = (C.c_void_p * max(n, 1))(*[f.ctypes.data for f in frames])
+        return self._local_map_call(
+            map_cloud, merge_params, voxel_resolution,
+            lambda outs: self.L.nicp_raw_depth_to_local_map(
+                self.handle, n, RA, rows, cols, C.c_float(depth_scale), int(step), C.c_float(max_depth_cov), C.byref(proj),
+                C.byref(sp), _fptr(so), C.c_float(baseline), C.c_float(alpha), _fptr(pp),
+                C.byref(merge_params) if merge_params is not None else None, _fptr(mt), C.c_float(voxel_resolution),
+                map_cloud.handle, *outs))
+
+    def multi_raw_depth_to_local_map(self, frames, mp, sp, poses, map_cloud, depth_scale=0.001, step=1, max_depth_cov=0.01,
+                                     sensor_offset=None, baseline=0.075, alpha=0.1, merge_proj=None, merge_params=None,
+                                     merge_transform=None, voxel_resolution=0.0):
+        """raw_depth_to_local_map for rig frames (nicp_multi_raw_depth_to_local_map): frames as in
+        multi_raw_depth_to_cloud_batch, baseline / alpha a scalar or one value per camera; the merge runs through the
+        pinhole view merge_proj, which merge_params needs.  Returns what raw_depth_to_local_map returns."""
+        n = len(frames)
+        imgs, rr, rc = _rig_frames(frames, mp.num_cameras)
+        P = np.asarray(poses, np.float32)
+        assert P.shape == (n, 4, 4), "one (4, 4) pose per frame"
+        assert merge_params is None or merge_proj is not None, "a merge needs merge_proj (a pinhole merge view)"
+        pp = np.ascontiguousarray(P.transpose(0, 2, 1)).reshape(n, 16)
+        so = colmajor(np.eye(4) if sensor_offset is None else sensor_offset)
+        mt = colmajor(np.eye(4) if merge_transform is None else merge_transform)
+        b, a = _per_camera(baseline, mp), _per_camera(alpha, mp)
+        RA = (C.c_void_p * max(len(imgs), 1))(*[im.ctypes.data for im in imgs])
+        return self._local_map_call(
+            map_cloud, merge_params, voxel_resolution,
+            lambda outs: self.L.nicp_multi_raw_depth_to_local_map(
+                self.handle, n, RA, _iptr(rr), _iptr(rc), C.c_float(depth_scale), int(step), C.c_float(max_depth_cov),
+                C.byref(mp), C.byref(sp), _fptr(so), _fptr(b), _fptr(a), _fptr(pp),
+                C.byref(merge_proj) if merge_proj is not None else None,
+                C.byref(merge_params) if merge_params is not None else None, _fptr(mt), C.c_float(voxel_resolution),
+                map_cloud.handle, *outs))
+
+    def _local_map_call(self, map_cloud, merge_params, voxel_resolution, call):
+        """runs call((appended_size, new_size, collapsed, representatives)) of a local-map entry -> its Python results"""
         before = map_cloud.size()
         collapsed = np.zeros(map_cloud.capacity, np.int32) if merge_params is not None else None
         reps = np.zeros(map_cloud.capacity, np.int32) if voxel_resolution > 0 else None
-        RA = (C.c_void_p * max(n, 1))(*[f.ctypes.data for f in frames])
         appended, new_size = C.c_int(0), C.c_int(0)
-        rc = self.L.nicp_raw_depth_to_local_map(
-            self.handle, n, RA, rows, cols, C.c_float(depth_scale), int(step), C.c_float(max_depth_cov), C.byref(proj),
-            C.byref(sp), _fptr(so), C.c_float(baseline), C.c_float(alpha), _fptr(pp),
-            C.byref(merge_params) if merge_params is not None else None, _fptr(mt), C.c_float(voxel_resolution),
-            map_cloud.handle, C.byref(appended), C.byref(new_size), _iptr(collapsed) if collapsed is not None else None,
-            _iptr(reps) if reps is not None else None)
+        rc = call((C.byref(appended), C.byref(new_size), _iptr(collapsed) if collapsed is not None else None,
+                   _iptr(reps) if reps is not None else None))
         if rc != NICP_OK:
             err = NicpError("nicp error %d: %s" % (rc, self.L.nicp_last_error().decode()))
             err.needed_size = new_size.value

@@ -466,15 +466,7 @@ __global__ void __launch_bounds__(256, 4) k_stats(PrepBatch B, int rows, int col
   if (!MULTI) {
     idx = raster_rank(I, r, c, cols);
   } else {
-    // MultiPointProjector::unProject concatenates the children's clouds (multipointprojector.cpp:59-90):
-    // points of the earlier column blocks, then raster order inside this camera's block
-    const int off = pc->g.colOff[cam], last = off + pc->g.height[cam] - 1;
-    const float *Ir = I + (size_t)r * cols;
-    const float *Ip = r > 0 ? Ir - cols : nullptr;
-    float before = off > 0 ? I[(size_t)(rows - 1) * cols + off - 1] : 0.0f;
-    float aboveBlock = Ip ? Ip[last] - (off > 0 ? Ip[off - 1] : 0.0f) : 0.0f;
-    float rowUpTo = (Ir[c] - (Ip ? Ip[c] : 0.0f)) - (off > 0 ? (Ir[off - 1] - (Ip ? Ip[off - 1] : 0.0f)) : 0.0f);
-    idx = (int)before + (int)aboveBlock + (int)rowUpTo - 1;
+    idx = rig_rank(I, r, c, rows, cols, pc->g.colOff[cam], pc->g.height[cam]);
   }
   if (index) index[pix] = idx;
 

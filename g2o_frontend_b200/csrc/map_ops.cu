@@ -191,33 +191,39 @@ __global__ void k_valid_flags(const float *__restrict__ depth, int n, float minD
 }
 
 struct Mat3 { float m[9]; };
-// pinholepointprojector.cpp:104-123 for the valid pixel (r, c) of depth z: g = the gaussian in the moments form
-__device__ __forceinline__ void gauss_sensor_model(int r, int c, float z, const Mat3 &iK, const Affine &iKRt, float fB,
+// pinholepointprojector.cpp:104-123 for the valid pixel of image coordinates (x, y) and depth z (a pinhole image: x = c,
+// y = r): g = the gaussian in the moments form
+__device__ __forceinline__ void gauss_sensor_model(float x, float y, float z, const Mat3 &iK, const Affine &iKRt, float fB,
                                                    float alpha, float *g) {
 #pragma unroll
   for (int k = 0; k < kGF; k++) g[k] = 0.0f;
-  xform_point(iKRt, fmul((float)c, z), fmul((float)r, z), z, g[0], g[1], g[2]);
+  xform_point(iKRt, fmul(x, z), fmul(y, z), z, g[0], g[1], g[2]);
   const float zVariation = fdiv(fmul(fmul(alpha, z), z), fadd(fB, fmul(z, alpha)));
-  float J0[9] = {z, 0.0f, 0.0f, 0.0f, z, 0.0f, (float)c, (float)r, 1.0f}, J[9], JD[9];
+  float J0[9] = {z, 0.0f, 0.0f, 0.0f, z, 0.0f, x, y, 1.0f}, J[9], JD[9];
   mat3_mul(iK.m, J0, J);
   const float dg[3] = {3.0f, 3.0f, zVariation};
   for (int j = 0; j < 3; j++)
     for (int i = 0; i < 3; i++) NM3(JD, i, j) = fmul(NM3(J, i, j), dg[j]);
   mat3_mul_bt(JD, J, g + 3);
 }
+// cov' = (R cov) R^T in place
+__device__ __forceinline__ void gauss_rotate_cov(const float *R, float *cov) {
+  float RC[9], out[9];
+  mat3_mul(R, cov, RC);
+  mat3_mul_bt(RC, R, out);
+  for (int k = 0; k < 9; k++) cov[k] = out[k];
+}
 // gaussian3.h:26-36 for one gaussian whose moments are up to date: mean' = R mean + t, cov' = (R cov) R^T
 __device__ __forceinline__ void gauss_xform_moments(const Affine &M, float *g) {
   float R[9];
   for (int r = 0; r < 3; r++)
     for (int c = 0; c < 3; c++) NM3(R, r, c) = M.r[r][c];
-  float mean[3], RC[9], cov[9];
+  float mean[3];
   mat3_vec(R, g, mean);
   g[0] = fadd(mean[0], M.r[0][3]);
   g[1] = fadd(mean[1], M.r[1][3]);
   g[2] = fadd(mean[2], M.r[2][3]);
-  mat3_mul(R, g + 3, RC);
-  mat3_mul_bt(RC, R, cov);
-  for (int k = 0; k < 9; k++) g[3 + k] = cov[k];
+  gauss_rotate_cov(R, g + 3);
 }
 
 // the valid pixels of one depth image; slot = raster rank of the pixel
@@ -232,7 +238,7 @@ __global__ void k_gaussians(const float *__restrict__ depth, const int *__restri
   if (slot >= capacity) return;
   const int r = pix / cols, c = pix - r * cols;
   float g[kGF];
-  gauss_sensor_model(r, c, z, iK, iKRt, fB, alpha, g);
+  gauss_sensor_model((float)c, (float)r, z, iK, iKRt, fB, alpha, g);
   gauss_store(gauss + (size_t)kGF * slot, g);
   gflags[slot] = NICP_GAUSS_MOMENTS;
 }
@@ -376,6 +382,114 @@ int run_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *dep
 }
 
 // ---------------------------------------------------------------------------------------------
+// sensor-model gaussians of a MultiPointProjector rig (DESIGN.md, known deviations): the gaussian of a point of camera i
+// is child i's PinholePointProjector model at its pixel (u, v) = (r, c - colOff_i) of the composite image, its mean is the
+// rig point itself (pixel_point<true>) and its covariance is rotated into the rig frame by the rotation of offset_i
+// ---------------------------------------------------------------------------------------------
+// per camera: unProject matrix with the rig at identity (PrepCams::iKRt), K_i^-1, baseline_i * fx_i, alpha_i, the rotation
+// of offset_i and whether it applies (0: offset_i is exactly the identity)
+struct RigSensor {
+  CamGeom g;
+  Affine iKRt[kMaxCams];
+  Mat3 iK[kMaxCams], R[kMaxCams];
+  float fB[kMaxCams], alpha[kMaxCams];
+  int rotate[kMaxCams];
+};
+static RigSensor rig_sensor(const CamSet &cams, const float *baseline, const float *alpha) {
+  RigSensor s;
+  memset(&s, 0, sizeof s);
+  s.g = geom_of(cams);
+  for (int i = 0; i < cams.n; i++) {
+    float iKRt[16];
+    compute_iKRt(cams.K[i], cams.offset[i], iKRt);
+    s.iKRt[i] = affine_from(iKRt);
+    mat3_inverse(cams.K[i], s.iK[i].m);
+    s.fB[i] = fmul(baseline[i], NM3(cams.K[i], 0, 0));
+    s.alpha[i] = alpha[i];
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 3; c++) NM3(s.R[i].m, r, c) = NM4(cams.offset[i], r, c);
+    s.rotate[i] = is_identity16(cams.offset[i]) ? 0 : 1;
+  }
+  return s;
+}
+// the camera whose column block holds composite column c (the blocks tile the columns; pixel_point<true>)
+__device__ __forceinline__ int rig_block(const CamGeom &g, int c) {
+  int cam = 0;
+  for (int i = 0; i < g.n; i++)
+    if (c >= g.colOff[i] && c < g.colOff[i] + g.height[i]) cam = i;
+  return cam;
+}
+__device__ __forceinline__ bool rig_valid(const CamGeom &g, int cam, int r, float z) {
+  return r < g.width[cam] && !(z < g.minD[cam] || z > g.maxD[cam]);
+}
+// the gaussian of the valid pixel (r, c) of camera cam, depth z, in the rig frame before the rig's sensor offset
+__device__ __forceinline__ void rig_gaussian(const RigSensor &S, int cam, int r, int c, float z, float *g) {
+  gauss_sensor_model((float)r, (float)(c - S.g.colOff[cam]), z, S.iK[cam], S.iKRt[cam], S.fB[cam], S.alpha[cam], g);
+  if (S.rotate[cam]) gauss_rotate_cov(S.R[cam].m, g + 3);
+}
+// position of composite pixel (r, c) of camera cam in the rig's point order (camera by camera, raster order inside the
+// camera's rows x height_i block): an exclusive scan of valid flags stored there is the compacted index of every valid pixel
+__device__ __forceinline__ size_t rig_order(const CamGeom &g, int cam, int r, int c, int rows) {
+  return (size_t)rows * g.colOff[cam] + (size_t)r * g.height[cam] + (c - g.colOff[cam]);
+}
+__global__ void k_rig_valid_flags(const float *__restrict__ depth, int rows, int cols, CamGeom g, int *__restrict__ flags) {
+  const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pix >= rows * cols) return;
+  const int r = pix / cols, c = pix - r * cols;
+  const int cam = rig_block(g, c);
+  flags[rig_order(g, cam, r, c, rows)] = rig_valid(g, cam, r, depth[pix]) ? 1 : 0;
+}
+__global__ void k_rig_gaussians(const float *__restrict__ depth, const int *__restrict__ rank, int rows, int cols, RigSensor S,
+                                int capacity, float *__restrict__ gauss, int *__restrict__ gflags) {
+  const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pix >= rows * cols) return;
+  const float z = depth[pix];
+  const int r = pix / cols, c = pix - r * cols;
+  const int cam = rig_block(S.g, c);
+  if (!rig_valid(S.g, cam, r, z)) return;
+  const int slot = rank[rig_order(S.g, cam, r, c, rows)];
+  if (slot >= capacity) return;
+  float g[kGF];
+  rig_gaussian(S, cam, r, c, z, g);
+  gauss_store(gauss + (size_t)kGF * slot, g);
+  gflags[slot] = NICP_GAUSS_MOMENTS;
+}
+
+// depth: host composite image (rows x cols) the cloud was built from with the same rig and sensor offset; baseline, alpha:
+// one per camera
+int run_multi_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *depth, const CamSet &cams, int rows,
+                                int cols, const float *baseline, const float *alpha, const float sensorOffset[16]) {
+  const int P = rows * cols;
+  int rc = cloud_ensure_gaussians(ctx, cloud);
+  if (rc) return rc;
+  Bump b;
+  const size_t need = pad256(sizeof(float) * P) + 2 * pad256(sizeof(int) * P) + pad256(sizeof(int) * scan_scratch_ints(P)) + 1024;
+  if ((rc = map_scratch(ctx, need, &b))) return rc;
+  float *d_depth = b.take<float>(P);
+  int *d_flags = b.take<int>(P), *d_rank = b.take<int>(P), *d_scan = b.take<int>(scan_scratch_ints(P)), *d_total = b.take<int>(1);
+  NICP_CUDA(cudaMemcpyAsync(d_depth, depth, sizeof(float) * P, cudaMemcpyHostToDevice, ctx->stream));
+  const RigSensor S = rig_sensor(cams, baseline, alpha);
+  k_rig_valid_flags<<<(P + 255) / 256, 256, 0, ctx->stream>>>(d_depth, rows, cols, S.g, d_flags);
+  NICP_CHECK_LAUNCH(ctx);
+  if ((rc = exclusive_scan(ctx, d_flags, d_rank, P, d_scan, d_total))) return rc;
+  k_rig_gaussians<<<(P + 127) / 128, 128, 0, ctx->stream>>>(d_depth, d_rank, rows, cols, S, cloud->capacity, cloud->gauss,
+                                                            cloud->gflags);
+  NICP_CHECK_LAUNCH(ctx);
+  int total = 0;
+  NICP_CUDA(cudaMemcpyAsync(&total, d_total, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
+  int n = 0;
+  NICP_CUDA(cudaMemcpy(&n, cloud->d_n, sizeof(int), cudaMemcpyDeviceToHost));
+  if (total != n) {
+    set_error("nicp_multi_cloud_compute_gaussians: the depth image has %d valid pixels but the cloud holds %d points", total, n);
+    return NICP_ERR_INVALID;
+  }
+  if ((rc = launch_gauss_transform(ctx, cloud, nullptr, 0, cloud->d_n, n, sensorOffset))) return rc;
+  cloud->has_gauss = true;
+  return NICP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
 // local map from one launch set of the batched frame preparation (nicp_raw_depth_to_local_map)
 // ---------------------------------------------------------------------------------------------
 // The frame clouds of the set (frame f = blockIdx.y), the poses they are appended with and the sensor offset of their
@@ -405,7 +519,24 @@ __global__ void k_local_map_gaussians(LocalMapSet S, const float *__restrict__ d
   const int r = pix / cols, c = pix - r * cols;
   const int slot = raster_rank(integral0 + (size_t)f * framePixels * kIntegralCh, r, c, cols);
   float g[kGF];
-  gauss_sensor_model(r, c, z, iK, iKRt, fB, alpha, g);
+  gauss_sensor_model((float)c, (float)r, z, iK, iKRt, fB, alpha, g);
+  if (!S.offsetIdentity) gauss_xform_moments(S.offset, g);
+  gauss_store(S.gauss[f] + (size_t)kGF * slot, g);
+  S.gflags[f][slot] = NICP_GAUSS_MOMENTS;
+}
+// the same for the rig frames of a set: the slot of a valid pixel is its rig rank (k_stats<true>)
+__global__ void k_local_map_rig_gaussians(LocalMapSet S, const float *__restrict__ depth0, const float *__restrict__ integral0,
+                                          size_t framePixels, int rows, int cols, RigSensor R) {
+  const int f = blockIdx.y;
+  const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pix >= rows * cols) return;
+  const float z = depth0[(size_t)f * framePixels + pix];
+  const int r = pix / cols, c = pix - r * cols;
+  const int cam = rig_block(R.g, c);
+  if (!rig_valid(R.g, cam, r, z)) return;
+  const int slot = rig_rank(integral0 + (size_t)f * framePixels * kIntegralCh, r, c, rows, cols, R.g.colOff[cam], R.g.height[cam]);
+  float g[kGF];
+  rig_gaussian(R, cam, r, c, z, g);
   if (!S.offsetIdentity) gauss_xform_moments(S.offset, g);
   gauss_store(S.gauss[f] + (size_t)kGF * slot, g);
   S.gflags[f][slot] = NICP_GAUSS_MOMENTS;
@@ -472,9 +603,11 @@ int launch_local_map_begin(nicp_context *ctx, nicp_cloud *map, long long *d_run)
 }
 
 // the m frame clouds of the launch set that launch_raw_prep_batch has just queued (its depth and integral images are still
-// in the batch scratch): gaussians, then one append launch behind *d_run
-int launch_local_map_set(nicp_context *ctx, const nicp_projector *proj, int m, nicp_cloud *const *frames, const float *poses,
-                         float baseline, float alpha, const float sensorOffset[16], nicp_cloud *map, long long *d_run) {
+// in the batch scratch): gaussians, then one append launch behind *d_run.  baseline, alpha: one per camera of fs.
+int launch_local_map_set(nicp_context *ctx, const FrameSet &fs, int m, nicp_cloud *const *frames, const float *poses,
+                         const float *baseline, const float *alpha, const float sensorOffset[16], nicp_cloud *map,
+                         long long *d_run) {
+  const nicp_projector *proj = &fs.proj;
   const int P = proj->rows * proj->cols;
   LocalMapSet S;
   memset(&S, 0, sizeof S);
@@ -499,10 +632,16 @@ int launch_local_map_set(nicp_context *ctx, const nicp_projector *proj, int m, n
   fix_last_row(M);
   S.offset = affine_from(M);
   S.offsetIdentity = is_identity16(M) ? 1 : 0;
-  const SensorModel sm = sensor_model(proj, baseline);
-  k_local_map_gaussians<<<dim3((P + 127) / 128, m), 128, 0, ctx->stream>>>(S, ctx->d_bDepth, ctx->d_bIntegral, ctx->batchPixels,
-                                                                          proj->rows, proj->cols, proj->min_distance,
-                                                                          proj->max_distance, sm.iK, sm.iKRt, sm.fB, alpha);
+  if (fs.cams.multi) {
+    k_local_map_rig_gaussians<<<dim3((P + 127) / 128, m), 128, 0, ctx->stream>>>(
+        S, ctx->d_bDepth, ctx->d_bIntegral, ctx->batchPixels, proj->rows, proj->cols, rig_sensor(fs.cams, baseline, alpha));
+  } else {
+    const SensorModel sm = sensor_model(proj, baseline[0]);
+    k_local_map_gaussians<<<dim3((P + 127) / 128, m), 128, 0, ctx->stream>>>(S, ctx->d_bDepth, ctx->d_bIntegral,
+                                                                            ctx->batchPixels, proj->rows, proj->cols,
+                                                                            proj->min_distance, proj->max_distance, sm.iK,
+                                                                            sm.iKRt, sm.fB, alpha[0]);
+  }
   NICP_CHECK_LAUNCH(ctx);
   k_local_map_append<<<dim3((P + 255) / 256, m), 256, 0, ctx->stream>>>(S, m, d_run, map->capacity, map->points, map->normals,
                                                                         map->omega, map->gauss, map->gflags);

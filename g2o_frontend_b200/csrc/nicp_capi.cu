@@ -3,6 +3,7 @@
 // dense statistics of Aligner::_computeStatistics (aligner.cpp:152-199).  No CPU fallback: every
 // compute entry point launches CUDA kernels or fails.
 #include <climits>
+#include <cmath>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstring>
@@ -346,6 +347,20 @@ int frames_rig(const nicp_multi_projector *mp, const int *rawRows, const int *ra
   fs.depthScale = depthScale;
   fs.maxDepthCov = maxDepthCov;
   fs.step = step;
+  return NICP_OK;
+}
+
+// the sensor-model constant of every camera of a rig (baseline, alpha): n finite values > 0
+static int check_per_camera(const char *what, const float *v, int n) {
+  if (!v) {
+    set_error("%s is null: the rig needs one value per camera", what);
+    return NICP_ERR_INVALID;
+  }
+  for (int i = 0; i < n; i++)
+    if (!(v[i] > 0.0f) || !std::isfinite(v[i])) {
+      set_error("%s[%d] = %g: needs a positive value per camera", what, i, (double)v[i]);
+      return NICP_ERR_INVALID;
+    }
   return NICP_OK;
 }
 
@@ -910,6 +925,17 @@ int nicp_cloud_compute_gaussians(nicp_context *ctx, nicp_cloud *c, const float *
   NICP_CUDA(cudaSetDevice(ctx->device));
   return run_compute_gaussians(ctx, c, depth, proj, baseline, alpha, sensor_offset);
 }
+int nicp_multi_cloud_compute_gaussians(nicp_context *ctx, nicp_cloud *c, const float *depth, const nicp_multi_projector *mp,
+                                       const float *baseline, const float *alpha, const float sensor_offset[16]) {
+  if (!ctx || !c || !depth || !mp || !sensor_offset) return NICP_ERR_INVALID;
+  FrameSet fs;
+  int rc;
+  if ((rc = rig_geometry(mp, fs)) || (rc = check_prep_image(fs.proj.rows, fs.proj.cols)) ||
+      (rc = check_per_camera("baseline", baseline, fs.cams.n)) || (rc = check_per_camera("alpha", alpha, fs.cams.n)))
+    return rc;
+  NICP_CUDA(cudaSetDevice(ctx->device));
+  return run_multi_compute_gaussians(ctx, c, depth, fs.cams, fs.proj.rows, fs.proj.cols, baseline, alpha, sensor_offset);
+}
 int nicp_cloud_has_gaussians(const nicp_cloud *c) { return c && c->has_gauss ? 1 : 0; }
 int nicp_cloud_download_gaussians(nicp_context *ctx, const nicp_cloud *c, float *gauss24, int *flags) {
   if (!ctx || !c) return NICP_ERR_INVALID;
@@ -1116,6 +1142,63 @@ static int ensure_local_map_frames(nicp_context *ctx, int sub, size_t px) {
   return ctx->d_lmRun ? NICP_OK : dev_alloc(&ctx->d_lmRun, 1);
 }
 
+// the body of nicp_raw_depth_to_local_map and nicp_multi_raw_depth_to_local_map: n frames of fs (raws[f * fs.cams.n + i] =
+// camera i of frame f; baseline, alpha: one per camera) prepared, given their gaussians and appended to the map, then
+// merged through mergeProj and voxelized on request.  The arguments the entries check are valid.
+static int raw_frames_to_local_map(nicp_context *ctx, const char *who, const FrameSet &fs, int n, const uint16_t *const *raws,
+                                   const nicp_stats_params *sp, const float sensorOffset[16], const float *baseline,
+                                   const float *alpha, const float *poses, const nicp_projector *mergeProj,
+                                   const nicp_merge_params *mergeParams, const float mergeTransform[16],
+                                   float voxelResolution, nicp_cloud *map, int *appendedSize, int *newSize, int *collapsed,
+                                   int *representatives) {
+  const int nc = fs.cams.n;
+  for (int f = 0; f < n; f++)
+    for (int i = 0; i < nc; i++)
+      if (!raws[(size_t)f * nc + i]) {
+        if (fs.cams.multi)
+          set_error("null raw image of camera %d in frame %d", i, f);
+        else
+          set_error("null raw image of frame %d", f);
+        return NICP_ERR_INVALID;
+      }
+  if (map->device != ctx->device) {
+    set_error("the map lives on GPU %d, the context on GPU %d", map->device, ctx->device);
+    return NICP_ERR_INVALID;
+  }
+  NICP_CUDA(cudaSetDevice(ctx->device));
+  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
+  const int sub = prep_set_frames(fs, n);
+  int rc;
+  if ((rc = ensure_batch_prep(ctx, sub, px, fs.rawPixels)) || (rc = ensure_local_map_frames(ctx, sub, px))) return rc;
+  if ((rc = launch_local_map_begin(ctx, map, ctx->d_lmRun))) return rc;
+  for (int base = 0; base < n; base += sub) {
+    const int m = std::min(sub, n - base);
+    if ((rc = prep_set(ctx, fs, m, raws + (size_t)base * nc, sp, sensorOffset, 0, ctx->lmFrames)) ||
+        (rc = launch_local_map_set(ctx, fs, m, ctx->lmFrames, poses + 16 * (size_t)base, baseline, alpha, sensorOffset, map,
+                                   ctx->d_lmRun)))
+      return rc;
+  }
+  ctx->lastRows = 0;
+  long long run = 0;
+  int before = 0;
+  NICP_CUDA(cudaMemcpyAsync(&run, ctx->d_lmRun, sizeof run, cudaMemcpyDeviceToHost, ctx->stream));
+  NICP_CUDA(cudaMemcpyAsync(&before, map->d_n, sizeof before, cudaMemcpyDeviceToHost, ctx->stream));
+  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (appendedSize) *appendedSize = (int)std::min<long long>(run - before, INT_MAX);
+  if (run > map->capacity) {
+    if (newSize) *newSize = (int)std::min<long long>(run, INT_MAX);
+    set_error("%s: %d + %lld points exceed the map's capacity %d", who, before, run - before, map->capacity);
+    return NICP_ERR_INVALID;
+  }
+  if ((rc = launch_local_map_commit(ctx, map, ctx->d_lmRun, (int)run))) return rc;
+  int size = (int)run;
+  if (mergeParams && (rc = nicp_merge(ctx, map, mergeProj, mergeTransform, mergeParams, collapsed, &size))) return rc;
+  if (voxelResolution > 0.0f && (rc = nicp_voxelize(ctx, map, voxelResolution, representatives, &size))) return rc;
+  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (newSize) *newSize = size;
+  return NICP_OK;
+}
+
 int nicp_raw_depth_to_local_map(nicp_context *ctx, int n, const uint16_t *const *raws, int raw_rows, int raw_cols,
                                 float depth_scale, int step, float max_depth_cov, const nicp_projector *proj,
                                 const nicp_stats_params *sp, const float sensor_offset[16], float baseline, float alpha,
@@ -1129,50 +1212,35 @@ int nicp_raw_depth_to_local_map(nicp_context *ctx, int n, const uint16_t *const 
     set_error("nicp_raw_depth_to_local_map: merge_params without merge_transform");
     return NICP_ERR_INVALID;
   }
-  for (int f = 0; f < n; f++)
-    if (!raws[f]) {
-      set_error("null raw image of frame %d", f);
-      return NICP_ERR_INVALID;
-    }
-  if (map->device != ctx->device) {
-    set_error("the map lives on GPU %d, the context on GPU %d", map->device, ctx->device);
+  FrameSet fs;
+  int rc;
+  if ((rc = frames_pinhole(proj, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs))) return rc;
+  return raw_frames_to_local_map(ctx, "nicp_raw_depth_to_local_map", fs, n, raws, sp, sensor_offset, &baseline, &alpha, poses,
+                                 proj, merge_params, merge_transform, voxel_resolution, map, appended_size, new_size,
+                                 collapsed, representatives);
+}
+
+int nicp_multi_raw_depth_to_local_map(nicp_context *ctx, int n, const uint16_t *const *raws, const int *raw_rows,
+                                      const int *raw_cols, float depth_scale, int step, float max_depth_cov,
+                                      const nicp_multi_projector *mp, const nicp_stats_params *sp,
+                                      const float sensor_offset[16], const float *baseline, const float *alpha,
+                                      const float *poses, const nicp_projector *merge_proj,
+                                      const nicp_merge_params *merge_params, const float merge_transform[16],
+                                      float voxel_resolution, nicp_cloud *map, int *appended_size, int *new_size,
+                                      int *collapsed, int *representatives) {
+  if (!ctx || n <= 0 || !raws || !mp || !sp || !sensor_offset || !poses || !map) return NICP_ERR_INVALID;
+  if (merge_params && (!merge_proj || !merge_transform)) {
+    set_error("nicp_multi_raw_depth_to_local_map: merge_params without merge_proj or merge_transform");
     return NICP_ERR_INVALID;
   }
   FrameSet fs;
   int rc;
-  if ((rc = frames_pinhole(proj, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs))) return rc;
-  NICP_CUDA(cudaSetDevice(ctx->device));
-  const size_t px = (size_t)proj->rows * proj->cols;
-  const int sub = prep_set_frames(fs, n);
-  if ((rc = ensure_batch_prep(ctx, sub, px, fs.rawPixels)) || (rc = ensure_local_map_frames(ctx, sub, px))) return rc;
-  if ((rc = launch_local_map_begin(ctx, map, ctx->d_lmRun))) return rc;
-  for (int base = 0; base < n; base += sub) {
-    const int m = std::min(sub, n - base);
-    if ((rc = prep_set(ctx, fs, m, raws + base, sp, sensor_offset, 0, ctx->lmFrames)) ||
-        (rc = launch_local_map_set(ctx, proj, m, ctx->lmFrames, poses + 16 * (size_t)base, baseline, alpha, sensor_offset,
-                                   map, ctx->d_lmRun)))
-      return rc;
-  }
-  ctx->lastRows = 0;
-  long long run = 0;
-  int before = 0;
-  NICP_CUDA(cudaMemcpyAsync(&run, ctx->d_lmRun, sizeof run, cudaMemcpyDeviceToHost, ctx->stream));
-  NICP_CUDA(cudaMemcpyAsync(&before, map->d_n, sizeof before, cudaMemcpyDeviceToHost, ctx->stream));
-  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
-  if (appended_size) *appended_size = (int)std::min<long long>(run - before, INT_MAX);
-  if (run > map->capacity) {
-    if (new_size) *new_size = (int)std::min<long long>(run, INT_MAX);
-    set_error("nicp_raw_depth_to_local_map: %d + %lld points exceed the map's capacity %d", before, run - before,
-              map->capacity);
-    return NICP_ERR_INVALID;
-  }
-  if ((rc = launch_local_map_commit(ctx, map, ctx->d_lmRun, (int)run))) return rc;
-  int size = (int)run;
-  if (merge_params && (rc = nicp_merge(ctx, map, proj, merge_transform, merge_params, collapsed, &size))) return rc;
-  if (voxel_resolution > 0.0f && (rc = nicp_voxelize(ctx, map, voxel_resolution, representatives, &size))) return rc;
-  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
-  if (new_size) *new_size = size;
-  return NICP_OK;
+  if ((rc = frames_rig(mp, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs)) ||
+      (rc = check_per_camera("baseline", baseline, fs.cams.n)) || (rc = check_per_camera("alpha", alpha, fs.cams.n)))
+    return rc;
+  return raw_frames_to_local_map(ctx, "nicp_multi_raw_depth_to_local_map", fs, n, raws, sp, sensor_offset, baseline, alpha,
+                                 poses, merge_proj, merge_params, merge_transform, voxel_resolution, map, appended_size,
+                                 new_size, collapsed, representatives);
 }
 
 int nicp_multi_raw_depth_to_cloud_batch(nicp_context *ctx, int n, const uint16_t *const *raws, const int *raw_rows,

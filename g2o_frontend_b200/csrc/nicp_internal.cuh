@@ -129,6 +129,18 @@ __device__ __forceinline__ int raster_rank(const float *__restrict__ I, int r, i
   const float upto = I[pix] - (r > 0 ? I[pix - cols] : 0.0f);
   return (int)above + (int)upto - 1;
 }
+// The same for a valid pixel (r, c) of the camera whose column block of a MultiPointProjector composite image is
+// [off, off + height): MultiPointProjector::unProject concatenates the children's clouds (multipointprojector.cpp:59-90), so
+// the index counts the points of the earlier column blocks, then raster order inside this camera's block
+__device__ __forceinline__ int rig_rank(const float *__restrict__ I, int r, int c, int rows, int cols, int off, int height) {
+  const int last = off + height - 1;
+  const float *Ir = I + (size_t)r * cols;
+  const float *Ip = r > 0 ? Ir - cols : nullptr;
+  float before = off > 0 ? I[(size_t)(rows - 1) * cols + off - 1] : 0.0f;
+  float aboveBlock = Ip ? Ip[last] - (off > 0 ? Ip[off - 1] : 0.0f) : 0.0f;
+  float rowUpTo = (Ir[c] - (Ip ? Ip[c] : 0.0f)) - (off > 0 ? (Ir[off - 1] - (Ip ? Ip[off - 1] : 0.0f)) : 0.0f);
+  return (int)before + (int)aboveBlock + (int)rowUpTo - 1;
+}
 #endif
 
 // accumulator slot layout of the fused correspondence+linearise reduction
@@ -396,8 +408,8 @@ struct nicp_context {
   // local-map maintenance scratch (map_ops.cu), grow-only
   void *d_mapScratch;
   size_t mapScratchBytes;
-  // nicp_raw_depth_to_local_map: the frame clouds of one prep launch set (reused set to set and call to call) and the
-  // running point count of the map being built
+  // nicp_raw_depth_to_local_map / nicp_multi_raw_depth_to_local_map: the frame clouds of one prep launch set (reused set
+  // to set and call to call) and the running point count of the map being built
   nicp_cloud *lmFrames[nicp::kMaxPrepBatch];
   long long *d_lmRun;
 
@@ -492,8 +504,11 @@ int launch_gauss_append(nicp_context *ctx, nicp_cloud *dst, const nicp_cloud *sr
 int run_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *depth, const nicp_projector *proj,
                           float baseline, float alpha, const float sensorOffset[16]);
 int launch_local_map_begin(nicp_context *ctx, nicp_cloud *map, long long *d_run);
-int launch_local_map_set(nicp_context *ctx, const nicp_projector *proj, int m, nicp_cloud *const *frames, const float *poses,
-                         float baseline, float alpha, const float sensorOffset[16], nicp_cloud *map, long long *d_run);
+int run_multi_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *depth, const CamSet &cams, int rows,
+                                int cols, const float *baseline, const float *alpha, const float sensorOffset[16]);
+int launch_local_map_set(nicp_context *ctx, const FrameSet &fs, int m, nicp_cloud *const *frames, const float *poses,
+                         const float *baseline, const float *alpha, const float sensorOffset[16], nicp_cloud *map,
+                         long long *d_run);
 int launch_local_map_commit(nicp_context *ctx, nicp_cloud *map, const long long *d_run, int newSize);
 int run_merge(nicp_context *ctx, nicp_cloud *cloud, const nicp_projector *proj, const float transform[16],
               const nicp_merge_params *mp, int n, int *collapsedHost, int *newSize);

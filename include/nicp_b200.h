@@ -190,6 +190,18 @@ int nicp_cloud_append(nicp_context *ctx, nicp_cloud *dst, const nicp_cloud *src,
  * order).  PinholePointProjector defaults: baseline 0.075, alpha 0.1 (pinholepointprojector.cpp:5-13). */
 int nicp_cloud_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *depth, const nicp_projector *proj,
                                  float baseline, float alpha, const float sensor_offset[16]);
+/* The rig counterpart of nicp_cloud_compute_gaussians; depth is the composite image the cloud was built from by
+ * nicp_multi_depth_to_cloud / nicp_multi_raw_depth_to_cloud_batch; baseline, alpha: mp->num_cameras floats each (> 0).
+ * The gaussian of a point of camera i at composite pixel (r, c), depth z, is child i's sensor model above at its pixel
+ * (u, v) = (r, c - colOff_i), in the moments form: mean = the rig point (bit-identical to the cloud's point before the
+ * sensor offset), covariance R_i (J diag(3, 3, alpha_i z^2 / (baseline_i fx_i + alpha_i z)) J^T) R_i^T with R_i the
+ * rotation of sensor_offset[i] of the rig (skipped when that offset is the identity); then sensor_offset as above.  One
+ * gaussian per point, in the cloud's point order.  This is the project's definition (DESIGN.md, known deviations), not
+ * pinned to the reference's MultiPointProjector.  A depth image whose valid pixels differ in number from the cloud's
+ * points is rejected with NICP_ERR_INVALID. */
+int nicp_multi_cloud_compute_gaussians(nicp_context *ctx, nicp_cloud *cloud, const float *depth,
+                                       const nicp_multi_projector *mp, const float *baseline, const float *alpha,
+                                       const float sensor_offset[16]);
 /* 1 if the cloud carries gaussians.  nicp_cloud_transform / nicp_cloud_append carry them along (cloud.cpp:145-186). */
 int nicp_cloud_has_gaussians(const nicp_cloud *cloud);
 int nicp_cloud_download_gaussians(nicp_context *ctx, const nicp_cloud *cloud, float *gauss24, int *flags);
@@ -275,6 +287,22 @@ int nicp_raw_depth_to_local_map(nicp_context *ctx, int n, const uint16_t *const 
                                 const float *poses, const nicp_merge_params *merge_params,
                                 const float merge_transform[16], float voxel_resolution, nicp_cloud *map,
                                 int *appended_size, int *new_size, int *collapsed, int *representatives);
+/* The rig counterpart of nicp_raw_depth_to_local_map: raws[f * num_cameras + i] is camera i of frame f, raw_rows /
+ * raw_cols as in nicp_multi_raw_depth_to_cloud_batch; each frame gets the gaussians of nicp_multi_cloud_compute_gaussians
+ * (baseline, alpha: one per camera, > 0).  The merge step (if merge_params != NULL) is nicp_merge(map, merge_proj,
+ * merge_transform, merge_params) with a pinhole merge view (merge_proj and merge_transform are then required).  The map
+ * is byte-identical to the chain of single calls (nicp_multi_raw_depth_to_cloud_batch of one frame,
+ * nicp_multi_cloud_compute_gaussians, nicp_cloud_append, then nicp_merge and nicp_voxelize).  A launch set holds
+ * clamp(8 * 640 * 480 / composite pixels, 1, 8) frames; the frame clouds of one set are scratch of the context.  Outputs,
+ * a map too small and synchronisation as in nicp_raw_depth_to_local_map. */
+int nicp_multi_raw_depth_to_local_map(nicp_context *ctx, int n, const uint16_t *const *raws, const int *raw_rows,
+                                      const int *raw_cols, float depth_scale, int step, float max_depth_cov,
+                                      const nicp_multi_projector *mp, const nicp_stats_params *sp,
+                                      const float sensor_offset[16], const float *baseline, const float *alpha,
+                                      const float *poses, const nicp_projector *merge_proj,
+                                      const nicp_merge_params *merge_params, const float merge_transform[16],
+                                      float voxel_resolution, nicp_cloud *map, int *appended_size, int *new_size,
+                                      int *collapsed, int *representatives);
 /* ---- stage-level virtuals of the converter (SURVEY.md section 8b) ------------------------------------------------
  * StatsCalculatorIntegralImage::compute(normals, statsVector, points, indexImage) with the calculator's _intervalImage
  * (statscalculator.h:36, statscalculatorintegralimage.h:37 / .cpp:14-82): PointIntegralImage::compute over

@@ -582,6 +582,18 @@ class MultiPointProjector : public PointProjector {
   }
   void clearProjectors() { _pointProjectors.clear(); }
   size_t numProjectors() const { return _pointProjectors.size(); }
+  // baseline() / alpha() of every child: the per-camera sensor model of the rig's gaussians
+  // (nicp_multi_cloud_compute_gaussians); every child must be a PinholePointProjector
+  void childSensorModels(std::vector<float> &baseline, std::vector<float> &alpha) const {
+    baseline.clear();
+    alpha.clear();
+    for (size_t i = 0; i < _pointProjectors.size(); i++) {
+      const PinholePointProjector *pp = _pointProjectors[i].pointProjector;
+      if (!pp) throw std::runtime_error("MultiPointProjector: the sensor model needs a PinholePointProjector per child");
+      baseline.push_back(pp->baseline());
+      alpha.push_back(pp->alpha());
+    }
+  }
   // multipointprojector.cpp:7-18
   void computeImageSize(int &rows, int &cols) const {
     nicp_multi_projector mp = abiMultiProjector();
@@ -863,6 +875,13 @@ class DepthImageConverterIntegralImage : public DepthImageConverter {
                                           _keepStats ? 1 : 0, d, _indexImage.data()),
                 "DepthImageConverterIntegralImage::compute (MultiPointProjector)");
       cloud.setHasStats(_keepStats);
+      if (_keepGaussians) {
+        std::vector<float> baseline, alpha;
+        mpp->childSensorModels(baseline, alpha);
+        nicpCheck(nicp_multi_cloud_compute_gaussians(Context::current().handle(), d, depthImage.data(), &mp, baseline.data(),
+                                                     alpha.data(), sensorOffset.data()),
+                  "DepthImageConverterIntegralImage::compute (MultiPointProjector gaussians)");
+      }
       return;
     }
     PinholePointProjector *pp = dynamic_cast<PinholePointProjector *>(_projector);
@@ -908,7 +927,8 @@ class Merger {
   Size2i imageSize() const { Size2i s = {_rows, _cols}; return s; }
   const std::vector<int> &collapsedIndices() const { return _collapsedIndices; }
 
-  // merger.cpp:15-119
+  // merger.cpp:15-119.  The Merger's projector must be a PinholePointProjector: a rig cloud (a MultiPointProjector
+  // converter with setKeepGaussians(true)) is merged through a pinhole view of the Merger's image size.
   void merge(Cloud *cloud, Isometry3f transform = Isometry3f::Identity()) {
     if (_rows <= 0 || _cols <= 0) throw std::runtime_error("Merger: _indexImage has zero size");
     if (!_depthImageConverter || !_depthImageConverter->projector()) throw std::runtime_error("Merger: missing _depthImageConverter / projector");
