@@ -35,6 +35,8 @@ SYMBOLS = [
     "nicp_multi_align_frames_sharded",
     "nicp_frame_store_create", "nicp_multi_frame_store_create", "nicp_frame_store_destroy", "nicp_frame_store_add",
     "nicp_frame_store_remove", "nicp_frame_store_size", "nicp_frame_store_align", "nicp_frame_store_counters",
+    "nicp_tracker_create", "nicp_multi_tracker_create", "nicp_tracker_destroy", "nicp_tracker_size", "nicp_tracker_step",
+    "nicp_tracker_reset",
 ]
 
 GAUSS_FLOATS = 24
@@ -103,6 +105,20 @@ RESULT_DTYPE = np.dtype([("T", np.float32, 16), ("omega", np.float32, 36), ("err
 assert RESULT_DTYPE.itemsize == 256
 
 
+class TrackResult(C.Structure):
+    _fields_ = [("global_T", C.c_float * 16), ("relative_T", C.c_float * 16), ("guess", C.c_float * 16),
+                ("frame", C.c_int), ("aligned", C.c_int), ("keyframe", C.c_int), ("num_keyframes", C.c_int),
+                ("record", AlignResult)]
+
+
+assert C.sizeof(TrackResult) == 464
+
+TRACK_DTYPE = np.dtype([("global_T", np.float32, 16), ("relative_T", np.float32, 16), ("guess", np.float32, 16),
+                        ("frame", np.int32), ("aligned", np.int32), ("keyframe", np.int32), ("num_keyframes", np.int32),
+                        ("record", RESULT_DTYPE)])
+assert TRACK_DTYPE.itemsize == 464
+
+
 def lib_path(verify=False):
     return os.path.join(LIB_DIR, "libnicp_b200_verify.so" if verify else "libnicp_b200.so")
 
@@ -130,6 +146,7 @@ def load(verify=False):
     L.nicp_t2v.restype = None
     L.nicp_multi_image_size.restype = None
     L.nicp_frame_store_destroy.restype = None
+    L.nicp_tracker_destroy.restype = None
     for name in SYMBOLS:
         fn = getattr(L, name)
         if fn.restype is C.c_int:
@@ -929,6 +946,89 @@ class FrameStore:
     def close(self):
         if self.handle:
             self.L.nicp_frame_store_destroy(self.handle)
+            self.handle = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Tracker:
+    """nicp_tracker: S independent depth sequences tracked as pwn::SequentialTracker::processFrame tracks one, with their
+    keyframes resident on the workers of a shard pool (sequence s on worker s * G // S).  One step takes one frame of each
+    listed sequence: one batched prep and one batched alignment per worker.
+
+    camera is a Projector (pinhole, describing the image after scaling; raw_shape = (rows, cols) of every raw frame) or a
+    MultiProjector (rig; raw_shape = one (rows, cols) per camera, as the sensor delivers it), as for FrameStore.  sp and ap
+    are the statistics and alignment parameters, img_threshold the frame inlier depth threshold of every record, and
+    new_frame_inliers_fraction the keyframe threshold of SequentialTracker::setNewFrameInliersFraction.  Every argument is
+    fixed for the tracker's lifetime."""
+
+    def __init__(self, pool, camera, sp, ap, raw_shape, n_sequences, depth_scale=0.001, step=1, max_depth_cov=0.01,
+                 sensor_offset=None, img_threshold=50.0, new_frame_inliers_fraction=0.4):
+        self.pool = pool  # the tracker's clouds live on the pool's workers
+        self.L = pool.L
+        self.rig = isinstance(camera, MultiProjector)
+        self.num_cameras = camera.num_cameras if self.rig else 1
+        self.handle = C.c_void_p()
+        so = None if sensor_offset is None else _fptr(colmajor(sensor_offset))
+        # the C call reads raw_rows x raw_cols pixels of every camera from whatever pointer it is given, so step() checks
+        # each image against these shapes
+        self.raw_shapes = [tuple(int(x) for x in s) for s in (raw_shape if self.rig else [raw_shape])]
+        common = (C.c_float(depth_scale), int(step), C.c_float(max_depth_cov))
+        tail = (C.byref(sp), so, C.byref(ap), C.c_float(img_threshold), C.c_float(new_frame_inliers_fraction),
+                C.byref(self.handle))
+        if self.rig:
+            shapes = np.array(raw_shape, np.int32).reshape(self.num_cameras, 2)
+            rr, rc = np.ascontiguousarray(shapes[:, 0]), np.ascontiguousarray(shapes[:, 1])
+            _check(self.L, self.L.nicp_multi_tracker_create(pool.handle, int(n_sequences), _iptr(rr), _iptr(rc), *common,
+                                                            C.byref(camera), *tail))
+        else:
+            rows, cols = raw_shape
+            _check(self.L, self.L.nicp_tracker_create(pool.handle, int(n_sequences), int(rows), int(cols), *common,
+                                                      C.byref(camera), *tail))
+
+    def step(self, sequences, frames, odometry=None):
+        """frames[k] is the next frame of sequence sequences[k]: a uint16 image (pinhole) or one uint16 image per camera
+        (rig), each of exactly the raw shape given at creation (any other shape raises ValueError and the library is not
+        called).  odometry: None (identity) or one (4, 4) initial guess per frame.  Returns TRACK_DTYPE results."""
+        seqs = np.ascontiguousarray(sequences, np.int32)
+        n = len(seqs)
+        if len(frames) != n:
+            raise ValueError("%d sequences for %d frames" % (n, len(frames)))
+        nc = self.num_cameras
+        imgs = []
+        for k, fr in enumerate(frames):
+            cams = fr if self.rig else [fr]
+            if len(cams) != nc:
+                raise ValueError("frame %d has %d images for %d cameras" % (k, len(cams), nc))
+            for i, im in enumerate(cams):
+                im = np.ascontiguousarray(im, np.uint16)
+                if im.shape != self.raw_shapes[i]:
+                    raise ValueError("frame %d, camera %d: raw image of shape %s, the tracker takes %s"
+                                     % (k, i, im.shape, self.raw_shapes[i]))
+                imgs.append(im)
+        if odometry is not None and len(odometry) != n:
+            raise ValueError("%d odometry guesses for %d frames" % (len(odometry), n))
+        RA = (C.c_void_p * max(len(imgs), 1))(*[im.ctypes.data for im in imgs])
+        results = np.zeros(n, TRACK_DTYPE)
+        _check(self.L, self.L.nicp_tracker_step(self.handle, n, _iptr(seqs), RA, _guesses(odometry, n),
+                                                results.ctypes.data_as(C.POINTER(TrackResult))))
+        return results
+
+    def reset(self, sequences):
+        """the listed sequences start over: no keyframe, global pose identity, counters 0"""
+        seqs = np.ascontiguousarray(sequences, np.int32)
+        _check(self.L, self.L.nicp_tracker_reset(self.handle, len(seqs), _iptr(seqs)))
+
+    def size(self):
+        return int(self.L.nicp_tracker_size(self.handle))
+
+    def close(self):
+        if self.handle:
+            self.L.nicp_tracker_destroy(self.handle)
             self.handle = C.c_void_p()
 
     def __del__(self):

@@ -24,6 +24,10 @@
 // A frame store (nicp_frame_store_*) runs the same walker with frames named by caller-chosen ids instead of the index in
 // one call's array, and with a slot table per worker that outlives the call: the incremental closer's PwnCloudCache
 // (pwn_tracker2/pwn_cloud_cache.cpp:60-102), which rebuilds a node's cloud only after it was evicted.
+//
+// A tracker (nicp_tracker_*) runs SequentialTracker::processFrame (include/pwn/tracker.h) for many independent sequences:
+// each sequence stays on one worker with its keyframe and current cloud, and a step is one batched prep and one batched
+// alignment per worker, the pose bookkeeping being done in the calling thread once every worker has succeeded.
 #include <algorithm>
 #include <climits>
 #include <cstdlib>
@@ -75,6 +79,7 @@ struct nicp_shard_pool {
   std::vector<Worker> workers;
   int frameCap;  // NICP_SHARD_FRAMES (>= 2), 0 = unset
   std::vector<nicp_frame_store *> stores;  // released when the pool is destroyed
+  std::vector<nicp_tracker *> trackers;    // likewise
 };
 
 struct nicp_frame_store {
@@ -85,6 +90,27 @@ struct nicp_frame_store {
   bool hasOffset;
   std::unordered_map<long long, std::vector<uint16_t>> raws;  // id -> raw images of its cameras, back to back
   std::vector<Residency> res;                                  // one per worker of the pool
+};
+
+// The state of one sequence of a tracker: SequentialTracker's members (include/pwn/tracker.h), with the keyframe cloud and
+// the cloud the next frame is prepared into living on the sequence's worker.
+struct TrackSeq {
+  int worker;
+  nicp_cloud *key, *cur;
+  bool hasKey;                  // SequentialTracker::_previousCloud != 0
+  float globalT[16], keyT[16];  // _globalT, _previousCloudTransform (column-major)
+  int counter, numKeyframes;
+};
+
+struct nicp_tracker {
+  nicp_shard_pool *pool;  // null once the pool has been destroyed
+  nicp::FrameSet fs;
+  nicp_stats_params sp;
+  nicp_align_params ap;
+  float imgThr, newFrameInliersFraction;
+  float sensorOffset[16];
+  bool hasOffset;
+  std::vector<TrackSeq> seqs;
 };
 
 using namespace nicp;
@@ -292,6 +318,129 @@ static void store_release(nicp_frame_store *st) {
   for (Residency &r : st->res) r.release();
 }
 
+// ---- trackers -------------------------------------------------------------------------------------------------------------
+
+// The pose bookkeeping of SequentialTracker::processFrame (include/pwn/tracker.h:64-91) after an alignment with relative
+// transform T and `inliers` inliers, in float32 and in the operation order of include/pwn/compat.h: iso_mul / iso_inverse
+// are Isometry3f::operator* / inverse(), the re-orthogonalisation is written with Matrix3f's product (a sum from 0.0f,
+// column index ascending), operator*(float) and operator-.  Returns whether the new cloud becomes the keyframe.
+static bool track_bookkeeping(TrackSeq &s, const float guess[16], const float T[16], int inliers, int pixels,
+                              float newFrameInliersFraction) {
+  if (inliers > 0)
+    iso_mul(s.keyT, T, s.globalT);
+  else
+    iso_mul(s.globalT, guess, s.globalT);
+  if (!(s.counter % 50)) {  // pwn_tracker.cpp:153-158: R -= 0.5 R (R^T R - I)
+    float R[9], E[9], corr[9];
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 3; c++) R[c * 3 + r] = NM4(s.globalT, r, c);
+    for (int r = 0; r < 3; r++)
+      for (int k = 0; k < 3; k++) {
+        float acc = 0.0f;
+        for (int c = 0; c < 3; c++) acc += R[r * 3 + c] * R[k * 3 + c];  // R^T(r, c) * R(c, k)
+        E[k * 3 + r] = acc;
+      }
+    for (int i = 0; i < 3; i++) E[i * 3 + i] -= 1.0f;
+    for (int r = 0; r < 3; r++)
+      for (int k = 0; k < 3; k++) {
+        float acc = 0.0f;
+        for (int c = 0; c < 3; c++) acc += R[c * 3 + r] * E[k * 3 + c];
+        corr[k * 3 + r] = acc;
+      }
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 3; c++) NM4(s.globalT, r, c) = R[c * 3 + r] - corr[c * 3 + r] * 0.5f;
+  }
+  fix_last_row(s.globalT);
+  return (float)inliers / (float)pixels < newFrameInliersFraction;
+}
+
+static void track_restart(TrackSeq &s) {
+  s.hasKey = false;
+  mat4_identity(s.globalT);
+  mat4_identity(s.keyT);
+  s.counter = s.numKeyframes = 0;
+}
+
+static void tracker_release(nicp_tracker *t) {
+  for (TrackSeq &s : t->seqs) {
+    nicp_cloud_destroy(s.key);
+    nicp_cloud_destroy(s.cur);
+    s.key = s.cur = nullptr;
+  }
+}
+
+// NICP_ERR_INVALID (with a message) for a null tracker or one whose pool is gone
+static int tracker_usable(const nicp_tracker *t) {
+  if (!t) return NICP_ERR_INVALID;
+  if (!t->pool) {
+    set_error("the tracker's shard pool has been destroyed: only nicp_tracker_destroy may be called");
+    return NICP_ERR_INVALID;
+  }
+  return NICP_OK;
+}
+
+static int tracker_create(nicp_shard_pool *pool, int S, const FrameSet &fs, const nicp_stats_params *sp,
+                          const float sensor_offset[16], const nicp_align_params *ap, float imgThr, float newFraction,
+                          nicp_tracker **out) {
+  const int G = (int)pool->workers.size();
+  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
+  std::vector<int> worker(S), onWorker(G, 0);
+  for (int s = 0; s < S; s++) onWorker[worker[s] = (int)((long long)s * G / S)]++;
+  for (int g = 0; g < G; g++) {
+    const int cap = frame_cap(pool, pool->workers[g], px);
+    if ((long long)2 * onWorker[g] > cap) {
+      set_error("worker %d (GPU %d) would hold %d sequences at two clouds each, more than its frame cap of %d clouds of "
+                "%zu pixels (NICP_SHARD_FRAMES lowers the cap): use more workers or fewer sequences",
+                g, pool->workers[g].device, onWorker[g], cap, px);
+      return NICP_ERR_INVALID;
+    }
+  }
+  nicp_tracker *t = new nicp_tracker();
+  t->pool = pool;
+  t->fs = fs;
+  t->sp = *sp;
+  t->ap = *ap;
+  t->imgThr = imgThr;
+  t->newFrameInliersFraction = newFraction;
+  t->hasOffset = sensor_offset != nullptr;
+  if (sensor_offset) memcpy(t->sensorOffset, sensor_offset, sizeof t->sensorOffset);
+  t->seqs.resize(S);
+  for (int s = 0; s < S; s++) {
+    TrackSeq &q = t->seqs[s];
+    q.worker = worker[s];
+    q.key = q.cur = nullptr;
+    track_restart(q);
+    nicp_context *ctx = pool->workers[q.worker].ctx;
+    int rc;
+    if ((rc = nicp_cloud_create(ctx, (int)px, &q.key)) || (rc = nicp_cloud_create(ctx, (int)px, &q.cur))) {
+      tracker_release(t);
+      delete t;
+      return rc;
+    }
+  }
+  pool->trackers.push_back(t);
+  *out = t;
+  return NICP_OK;
+}
+
+// n distinct sequences in [0, S)
+static int check_sequences(const nicp_tracker *t, int n, const int *sequences) {
+  std::vector<char> seen(t->seqs.size(), 0);
+  for (int k = 0; k < n; k++) {
+    const int s = sequences[k];
+    if (s < 0 || s >= (int)t->seqs.size()) {
+      set_error("entry %d names sequence %d outside [0, %d)", k, s, (int)t->seqs.size());
+      return NICP_ERR_INVALID;
+    }
+    if (seen[s]) {
+      set_error("sequence %d is listed twice", s);
+      return NICP_ERR_INVALID;
+    }
+    seen[s] = 1;
+  }
+  return NICP_OK;
+}
+
 extern "C" {
 
 int nicp_shard_pool_create(const int *devices, int n_devices, nicp_shard_pool **out) {
@@ -333,6 +482,10 @@ void nicp_shard_pool_destroy(nicp_shard_pool *pool) {
   for (nicp_frame_store *st : pool->stores) {
     store_release(st);
     st->pool = nullptr;
+  }
+  for (nicp_tracker *t : pool->trackers) {
+    tracker_release(t);
+    t->pool = nullptr;
   }
   for (nicp_shard_pool::Worker &w : pool->workers) {
     w.calls.release();
@@ -514,6 +667,198 @@ int nicp_frame_store_counters(const nicp_frame_store *store, long long *frames_b
   }
   if (frames_built) *frames_built = b;
   if (frames_reused) *frames_reused = r;
+  return NICP_OK;
+}
+
+int nicp_tracker_create(nicp_shard_pool *pool, int n_sequences, int raw_rows, int raw_cols, float depth_scale, int step,
+                        float max_depth_cov, const nicp_projector *proj, const nicp_stats_params *sp,
+                        const float sensor_offset[16], const nicp_align_params *ap, float frame_inlier_depth_threshold,
+                        float new_frame_inliers_fraction, nicp_tracker **tracker) {
+  if (!tracker) return NICP_ERR_INVALID;
+  *tracker = nullptr;
+  if (!pool || !proj || !sp || !ap || raw_rows <= 0 || raw_cols <= 0 || n_sequences <= 0) return NICP_ERR_INVALID;
+  FrameSet fs;
+  int rc = frames_pinhole(proj, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs);
+  return rc ? rc
+            : tracker_create(pool, n_sequences, fs, sp, sensor_offset, ap, frame_inlier_depth_threshold,
+                             new_frame_inliers_fraction, tracker);
+}
+
+int nicp_multi_tracker_create(nicp_shard_pool *pool, int n_sequences, const int *raw_rows, const int *raw_cols,
+                              float depth_scale, int step, float max_depth_cov, const nicp_multi_projector *mp,
+                              const nicp_stats_params *sp, const float sensor_offset[16], const nicp_align_params *ap,
+                              float frame_inlier_depth_threshold, float new_frame_inliers_fraction, nicp_tracker **tracker) {
+  if (!tracker) return NICP_ERR_INVALID;
+  *tracker = nullptr;
+  if (!pool || !mp || !sp || !ap || n_sequences <= 0) return NICP_ERR_INVALID;
+  FrameSet fs;
+  int rc = frames_rig(mp, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs);
+  return rc ? rc
+            : tracker_create(pool, n_sequences, fs, sp, sensor_offset, ap, frame_inlier_depth_threshold,
+                             new_frame_inliers_fraction, tracker);
+}
+
+void nicp_tracker_destroy(nicp_tracker *tracker) {
+  if (!tracker) return;
+  if (tracker->pool) {
+    std::vector<nicp_tracker *> &v = tracker->pool->trackers;
+    v.erase(std::remove(v.begin(), v.end(), tracker), v.end());
+    tracker_release(tracker);
+  }
+  delete tracker;
+}
+
+int nicp_tracker_size(const nicp_tracker *tracker) {
+  return tracker_usable(tracker) ? -1 : (int)tracker->seqs.size();
+}
+
+int nicp_tracker_reset(nicp_tracker *tracker, int n, const int *sequences) {
+  int rc;
+  if ((rc = tracker_usable(tracker))) return rc;
+  if (n < 0) return NICP_ERR_INVALID;
+  if (n == 0) return NICP_OK;
+  if (!sequences) return NICP_ERR_INVALID;
+  if ((rc = check_sequences(tracker, n, sequences))) return rc;
+  for (int k = 0; k < n; k++) track_restart(tracker->seqs[sequences[k]]);
+  return NICP_OK;
+}
+
+int nicp_tracker_step(nicp_tracker *tracker, int n, const int *sequences, const uint16_t *const *raws,
+                      const float *odometry, nicp_track_result *results) {
+  int rc;
+  if ((rc = tracker_usable(tracker))) return rc;
+  if (n < 0) return NICP_ERR_INVALID;
+  if (n == 0) return NICP_OK;
+  if (!sequences || !raws || !results) return NICP_ERR_INVALID;
+  if ((rc = check_sequences(tracker, n, sequences))) return rc;
+  const FrameSet &fs = tracker->fs;
+  const int nc = fs.cams.n;
+  for (int k = 0; k < n; k++)
+    for (int i = 0; i < nc; i++)
+      if (!raws[(size_t)k * nc + i]) {
+        set_error("null raw image of camera %d in entry %d (sequence %d)", i, k, sequences[k]);
+        return NICP_ERR_INVALID;
+      }
+  nicp_shard_pool *pool = tracker->pool;
+  const float *so = tracker->hasOffset ? tracker->sensorOffset : nullptr;
+
+  // guess = keyT^-1 * globalT * odometry, from the committed state (SequentialTracker::processFrame, tracker.h:64-65)
+  std::vector<float> guesses((size_t)16 * n);
+  float eye[16];
+  mat4_identity(eye);
+  const int G = (int)pool->workers.size();
+  std::vector<std::vector<int>> entries(G);  // entries of the step on worker g, in listed order
+  for (int k = 0; k < n; k++) {
+    const TrackSeq &s = tracker->seqs[sequences[k]];
+    entries[s.worker].push_back(k);
+    float *g = &guesses[(size_t)16 * k];
+    if (!s.hasKey) {
+      mat4_identity(g);
+      continue;
+    }
+    iso_inverse(s.keyT, g);
+    iso_mul(g, s.globalT, g);
+    iso_mul(g, odometry ? odometry + (size_t)16 * k : eye, g);
+    fix_last_row(g);  // Aligner::setInitialGuess
+  }
+
+  // every worker: one batched prep of its entries' frames, one batched alignment of those that have a keyframe
+  std::vector<nicp_align_result> recs(n);
+  auto work = [&](int g) {
+    nicp_shard_pool::Worker &w = pool->workers[g];
+    const std::vector<int> &mine = entries[g];
+    w.rc = NICP_OK;
+    w.error.clear();
+    if (mine.empty()) return;
+    auto body = [&]() -> int {
+      NICP_CUDA(cudaSetDevice(w.device));
+      std::vector<const uint16_t *> frameRaws;
+      std::vector<nicp_cloud *> clouds;
+      std::vector<const nicp_cloud *> refs, curs;
+      std::vector<float> gs;
+      std::vector<int> aligned;
+      for (int k : mine) {
+        const TrackSeq &s = tracker->seqs[sequences[k]];
+        for (int i = 0; i < nc; i++) frameRaws.push_back(raws[(size_t)k * nc + i]);
+        clouds.push_back(s.hasKey ? s.cur : s.key);
+        if (s.hasKey) {
+          refs.push_back(s.key);
+          curs.push_back(s.cur);
+          gs.insert(gs.end(), &guesses[(size_t)16 * k], &guesses[(size_t)16 * k] + 16);
+          aligned.push_back(k);
+        }
+      }
+      int rc;
+      if ((rc = prep_frames(w.ctx, fs, (int)clouds.size(), frameRaws.data(), &tracker->sp, so, 0, clouds.data())))
+        return rc;
+      if (refs.empty()) return NICP_OK;
+      std::vector<nicp_align_result> out(refs.size());
+      if ((rc = align_frame_pairs(w.ctx, fs, (int)refs.size(), refs.data(), curs.data(), &tracker->ap, so, so, gs.data(),
+                                  nullptr, nullptr, tracker->imgThr, out.data())))
+        return rc;
+      for (size_t i = 0; i < aligned.size(); i++) recs[aligned[i]] = out[i];
+      return NICP_OK;
+    };
+    w.rc = body();
+    if (w.rc) w.error = nicp_last_error();  // this worker thread's message
+    // no upload of this step may still be reading the caller's raw images when the call returns
+    const int sync = nicp_synchronize(w.ctx);
+    if (!w.rc && sync) {
+      w.rc = sync;
+      w.error = nicp_last_error();
+    }
+  };
+  if (G == 1) {
+    work(0);
+  } else {
+    std::vector<std::thread> threads;
+    threads.reserve(G);
+    for (int g = 0; g < G; g++) threads.emplace_back(work, g);
+    for (std::thread &t : threads) t.join();
+  }
+  for (int g = 0; g < G; g++)
+    if (pool->workers[g].rc != NICP_OK) {
+      set_error("device %d (shard %d of %d): %s", pool->workers[g].device, g, G, pool->workers[g].error.c_str());
+      return pool->workers[g].rc;
+    }
+  for (int k = 0; k < n; k++)
+    if (tracker->seqs[sequences[k]].hasKey && recs[k].status != NICP_OK) {
+      set_error("entry %d (sequence %d): the alignment's record has status %d", k, sequences[k], recs[k].status);
+      return recs[k].status;
+    }
+
+  // commit, in the calling thread
+  const int pixels = fs.proj.rows * fs.proj.cols;
+  for (int k = 0; k < n; k++) {
+    TrackSeq &s = tracker->seqs[sequences[k]];
+    nicp_track_result &r = results[k];
+    memset(&r, 0, sizeof r);
+    r.frame = s.counter;
+    r.record.status = NICP_OK;
+    if (!s.hasKey) {  // the first frame: its cloud is the keyframe
+      s.hasKey = true;
+      memcpy(s.keyT, s.globalT, sizeof s.keyT);
+      s.numKeyframes++;
+      r.keyframe = 1;
+      mat4_identity(r.relative_T);
+      mat4_identity(r.guess);
+    } else {
+      const float *guess = &guesses[(size_t)16 * k];
+      r.aligned = 1;
+      r.record = recs[k];
+      memcpy(r.relative_T, recs[k].T, sizeof r.relative_T);
+      memcpy(r.guess, guess, sizeof r.guess);
+      if (track_bookkeeping(s, guess, recs[k].T, recs[k].inliers, pixels, tracker->newFrameInliersFraction)) {
+        std::swap(s.key, s.cur);
+        memcpy(s.keyT, s.globalT, sizeof s.keyT);
+        s.numKeyframes++;
+        r.keyframe = 1;
+      }
+    }
+    s.counter++;
+    memcpy(r.global_T, s.globalT, sizeof r.global_T);
+    r.num_keyframes = s.numKeyframes;
+  }
   return NICP_OK;
 }
 

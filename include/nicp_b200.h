@@ -526,6 +526,67 @@ int nicp_frame_store_align(nicp_frame_store *store, int n_pairs, const long long
  * and frames a window found resident (either output may be NULL) */
 int nicp_frame_store_counters(const nicp_frame_store *store, long long *frames_built, long long *frames_reused);
 
+/* ---- batched keyframe tracking: many independent depth sequences on a shard pool ---------------------------------------
+ * One sequence's poses depend on each other (PwnTracker::processFrame, pwn_tracker/pwn_tracker.cpp:106-282), but separate
+ * sequences (offline odometry over a recorded dataset, many robots, a parameter sweep over one log) do not.  A tracker keeps
+ * the keyframe state of S sequences resident on the workers of a pool; one step takes one frame of each listed sequence.
+ *   - Semantics: each listed sequence does exactly what pwn::SequentialTracker::processFrame (include/pwn/tracker.h) does on
+ *     that frame, with the tracker's sensor offset on every frame and setScale(step).  The cloud is prepared as
+ *     nicp_raw_depth_to_cloud / nicp_multi_raw_depth_to_cloud_batch prepare it (keep_stats 0).  A sequence without a keyframe
+ *     takes the cloud as its keyframe (keyT = globalT) and aligns nothing; its odometry is ignored.  Otherwise
+ *     guess = keyT^-1 * globalT * odometry (then fixLastRow), and the keyframe (reference) is aligned against the new cloud
+ *     (current): the record is byte-identical to nicp_align / nicp_multi_align with that guess, no priors and the sensor
+ *     offset on both sides (except omega when the pair has no inlier at all: the batched alignment reports another Omega
+ *     there than the single call).  Then globalT = keyT * T if inliers > 0, else globalT * guess; the rotation is re-orthogonalised
+ *     when the sequence's frame counter is a multiple of 50; fixLastRow; and the new cloud becomes the keyframe
+ *     (keyT = globalT) when (float)inliers / (float)(rows * cols) < new_frame_inliers_fraction (composite pixels for a rig).
+ *     The pose arithmetic is float32 in the operation order of include/pwn/compat.h, so it matches the C++ class bit for bit.
+ *   - Placement and memory: sequence s lives on worker floor(s * G / S) for the tracker's lifetime and owns two device
+ *     clouds there (keyframe and current frame), allocated at create; a keyframe switch swaps the two, nothing is copied.
+ *     Creation fails with NICP_ERR_INVALID when a worker's sequences need more clouds (two each) than its frame cap (that of
+ *     the sharded entries; NICP_SHARD_FRAMES lowers it).
+ *   - One step: every argument is checked in the calling thread first (null arrays or images, a sequence outside [0, S) or
+ *     listed twice, a destroyed pool).  Each worker with listed sequences makes one batched prep of their frames and one
+ *     batched alignment of those that have a keyframe, in listed order, and is synchronised before the call returns.  The
+ *     sequences' state is committed only after every worker succeeded: a rejected or failed step changes no sequence.  A
+ *     record whose status is not NICP_OK fails the step with that status.
+ *   - nicp_shard_pool_destroy releases the trackers' clouds; every later call on such a tracker except
+ *     nicp_tracker_destroy returns NICP_ERR_INVALID (nicp_tracker_size returns -1).  Calls are synchronous; a pool and its
+ *     trackers are used from one host thread at a time. */
+typedef struct {
+  float global_T[16];        /* SequentialTracker::globalT() after this frame */
+  float relative_T[16];      /* lastRelative(): the aligner's T (identity when aligned = 0) */
+  float guess[16];           /* initial guess the alignment started from, after fixLastRow (identity when aligned = 0) */
+  int frame;                 /* frames this sequence had processed before this one (SequentialTracker::_counter) */
+  int aligned;               /* 0 for a sequence's first frame after create / reset: nothing to align against */
+  int keyframe;              /* lastWasKeyframe() */
+  int num_keyframes;         /* numKeyframes() */
+  nicp_align_result record;  /* the alignment's record; zeroed with status NICP_OK when aligned = 0 */
+} nicp_track_result;
+
+typedef struct nicp_tracker nicp_tracker;
+/* the frame description, fixed for the tracker's lifetime and validated like nicp_frame_store_create /
+ * nicp_multi_frame_store_create validate theirs (proj describes the camera after scaling, as in nicp_raw_depth_to_cloud;
+ * sensor_offset NULL: identity); ap and frame_inlier_depth_threshold are those of every alignment */
+int nicp_tracker_create(nicp_shard_pool *pool, int n_sequences, int raw_rows, int raw_cols, float depth_scale, int step,
+                        float max_depth_cov, const nicp_projector *proj, const nicp_stats_params *sp,
+                        const float sensor_offset[16], const nicp_align_params *ap, float frame_inlier_depth_threshold,
+                        float new_frame_inliers_fraction, nicp_tracker **tracker);
+int nicp_multi_tracker_create(nicp_shard_pool *pool, int n_sequences, const int *raw_rows, const int *raw_cols,
+                              float depth_scale, int step, float max_depth_cov, const nicp_multi_projector *mp,
+                              const nicp_stats_params *sp, const float sensor_offset[16], const nicp_align_params *ap,
+                              float frame_inlier_depth_threshold, float new_frame_inliers_fraction, nicp_tracker **tracker);
+void nicp_tracker_destroy(nicp_tracker *tracker);
+/* n_sequences; -1 for a null tracker or one whose pool was destroyed */
+int nicp_tracker_size(const nicp_tracker *tracker);
+/* one frame for each of n distinct sequences: raws[k * num_cameras + i] is camera i of sequence sequences[k]'s frame (one
+ * camera for a pinhole tracker), exactly the raw size given at create; odometry + 16 k is that frame's initialGuess
+ * (NULL: identity); results[k] receives its result */
+int nicp_tracker_step(nicp_tracker *tracker, int n, const int *sequences, const uint16_t *const *raws,
+                      const float *odometry, nicp_track_result *results);
+/* the listed sequences start over: no keyframe, global pose identity, counters 0 */
+int nicp_tracker_reset(nicp_tracker *tracker, int n, const int *sequences);
+
 #ifdef __cplusplus
 }
 #endif
