@@ -26,6 +26,7 @@ SYMBOLS = [
     "nicp_stats_compute", "nicp_information_compute",
     "nicp_project", "nicp_correspond_linearize", "nicp_linearize",
     "nicp_align", "nicp_align_get_state", "nicp_align_get_trace", "nicp_align_batch", "nicp_align_batch_priors",
+    "nicp_statistics_tail", "nicp_statistics_tail_host",
     "nicp_multi_image_size", "nicp_multi_depth_to_cloud", "nicp_multi_project", "nicp_multi_align",
     "nicp_multi_raw_depth_to_cloud_batch", "nicp_multi_align_batch",
     "nicp_cloud_compute_gaussians", "nicp_multi_cloud_compute_gaussians", "nicp_cloud_has_gaussians",
@@ -755,6 +756,13 @@ class Context:
         _check(self.L, self.L.nicp_align_get_trace(self.handle, _fptr(tr), iters))
         return tr
 
+    def statistics_tail(self, H, T):
+        """the batch's _computeStatistics tail kernel on n caller-given linearisations (test hook): H (n, 36) and T (n, 16)
+        column-major -> omega (n, 36) column-major, ratios (n, 2) = (translational, rotational)"""
+        H, T, omega, ratios = _tail_args(H, T)
+        _check(self.L, self.L.nicp_statistics_tail(self.handle, H.shape[0], _fptr(H), _fptr(T), _fptr(omega), _fptr(ratios)))
+        return omega, ratios
+
     def align_batch(self, refs, curs, proj, ap, guesses=None, ref_offset=None, cur_offset=None, img_threshold=50.0,
                     results=None, priors=None):
         """refs/curs: sequences of Cloud.  guesses: (n,4,4) row/col matrices or None.  priors: None or a sequence of
@@ -782,6 +790,22 @@ def update_matrices(K, T, verify=False):
     KRt, iKRt = np.zeros(16, np.float32), np.zeros(16, np.float32)
     L.nicp_update_matrices(_fptr(k), _fptr(t), _fptr(KRt), _fptr(iKRt))
     return from_colmajor(KRt, 4), from_colmajor(iKRt, 4)
+
+
+def _tail_args(H, T):
+    H = np.ascontiguousarray(H, np.float32).reshape(-1, 36)
+    T = np.ascontiguousarray(T, np.float32).reshape(-1, 16)
+    assert H.shape[0] == T.shape[0]
+    return H, T, np.zeros((H.shape[0], 36), np.float32), np.zeros((H.shape[0], 2), np.float32)
+
+
+def statistics_tail_host(H, T, verify=False):
+    """the host function that finishes a single alignment's record (test hook, no GPU needed): Context.statistics_tail's
+    arguments and results"""
+    L = load(verify)
+    H, T, omega, ratios = _tail_args(H, T)
+    _check(L, L.nicp_statistics_tail_host(H.shape[0], _fptr(H), _fptr(T), _fptr(omega), _fptr(ratios)))
+    return omega, ratios
 
 
 def result_T(res):

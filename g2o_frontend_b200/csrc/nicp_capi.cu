@@ -1857,4 +1857,43 @@ int nicp_align_get_trace(nicp_context *ctx, float *trace61, int max_iterations) 
   return NICP_OK;
 }
 
+// the batch's k_statistics on caller-given H / T: the records and H staging of the context's result slots [0, n) are
+// filled here, so the state of the last nicp_align ends
+int nicp_statistics_tail(nicp_context *ctx, int n, const float *H, const float *T, float *omega, float *ratios) {
+  if (!ctx || n < 0) return NICP_ERR_INVALID;
+  NICP_CUDA(cudaSetDevice(ctx->device));
+  if (n == 0) return NICP_OK;
+  if (!H || !T || !omega || !ratios) return NICP_ERR_INVALID;
+  ctx->lastAlignValid = false;
+  int rc;
+  if ((rc = ensure_results(ctx, n))) return rc;
+  std::vector<nicp_align_result> rec((size_t)n);
+  std::vector<float> Hb((size_t)n * 42, 0.0f);
+  memset(rec.data(), 0, sizeof(nicp_align_result) * n);
+  for (int i = 0; i < n; i++) {
+    memcpy(rec[i].T, T + 16 * (size_t)i, sizeof(float) * 16);
+    memcpy(Hb.data() + 42 * (size_t)i, H + 36 * (size_t)i, sizeof(float) * 36);
+  }
+  NICP_CUDA(cudaMemcpyAsync(ctx->d_results, rec.data(), sizeof(nicp_align_result) * n, cudaMemcpyHostToDevice, ctx->stream));
+  NICP_CUDA(cudaMemcpyAsync(ctx->d_statHb, Hb.data(), sizeof(float) * 42 * n, cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = launch_statistics(ctx, ctx->stream, 0, n))) return rc;
+  NICP_CUDA(cudaMemcpyAsync(rec.data(), ctx->d_results, sizeof(nicp_align_result) * n, cudaMemcpyDeviceToHost, ctx->stream));
+  NICP_CUDA(cudaStreamSynchronize(ctx->stream));
+  for (int i = 0; i < n; i++) {
+    memcpy(omega + 36 * (size_t)i, rec[i].omega, sizeof(float) * 36);
+    ratios[2 * (size_t)i] = rec[i].translational_eigen_ratio;
+    ratios[2 * (size_t)i + 1] = rec[i].rotational_eigen_ratio;
+  }
+  return NICP_OK;
+}
+
+// the host function a single nicp_align finishes its record with (finish_results)
+int nicp_statistics_tail_host(int n, const float *H, const float *T, float *omega, float *ratios) {
+  if (n < 0 || (n > 0 && (!H || !T || !omega || !ratios))) return NICP_ERR_INVALID;
+  for (int i = 0; i < n; i++)
+    compute_statistics(H + 36 * (size_t)i, T + 16 * (size_t)i, omega + 36 * (size_t)i, ratios + 2 * (size_t)i,
+                       ratios + 2 * (size_t)i + 1);
+  return NICP_OK;
+}
+
 }  // extern "C"

@@ -9,6 +9,7 @@
 // JacobiSVD / Matrix6f::inverse() of the reference are replaced by a float64 cyclic Jacobi and a float64 Gauss-Jordan
 // (tolerance-level parity, like the oracle: DESIGN.md section 5).
 #pragma once
+#include <cstring>
 #include "nicp_math.cuh"
 
 namespace nicp {
@@ -128,7 +129,24 @@ NICP_HD float stats_sym_eig_ratio3(const float *O, int off) {
   return (float)ddiv(mx, mn);
 }
 
-// H_lin: the linearisation at the final T (column-major 6x6); T column-major 4x4.  Omega (36), two ratios.
+// x, or the quiet NaN 0x7fc00000 if x is any NaN.  A weak or degenerate H makes NaNs in the tail (a sigma point with
+// |q| > 1 takes sqrt of a negative number in v2t; a direction dropped by the pseudo-inverse makes the Cholesky divide
+// 0 by 0), and x86 and sm_100a arithmetic give those NaNs different sign and payload bits: one NaN for the record keeps
+// the host's single-alignment record and the device's batch record byte-identical.
+NICP_HD float canonical_nan(float x) {
+  if (x == x) return x;
+#if defined(__CUDA_ARCH__)
+  return __int_as_float(0x7fc00000);
+#else
+  const unsigned int q = 0x7fc00000u;
+  float f;
+  memcpy(&f, &q, sizeof f);
+  return f;
+#endif
+}
+
+// H_lin: the linearisation at the final T (column-major 6x6); T column-major 4x4.  Omega (36), two ratios; every NaN
+// among them is canonical_nan's.
 NICP_HD void compute_statistics_tail(const float *H_lin, const float *T, float *Omega, float *tr, float *rr) {
   float H[36], Sigma[36];
   for (int i = 0; i < 36; i++) H[i] = H_lin[i];
@@ -189,8 +207,9 @@ NICP_HD void compute_statistics_tail(const float *H_lin, const float *T, float *
       for (int c = 0; c < 6; c++) NM6(cov, r, c) = fadd(NM6(cov, r, c), (float)dmul(wc[i], (double)fmul(dl[r], dl[c])));
   }
   stats_mat6_inverse(cov, Omega);
-  *tr = stats_sym_eig_ratio3(Omega, 0);
-  *rr = stats_sym_eig_ratio3(Omega, 3);
+  *tr = canonical_nan(stats_sym_eig_ratio3(Omega, 0));
+  *rr = canonical_nan(stats_sym_eig_ratio3(Omega, 3));
+  for (int i = 0; i < 36; i++) Omega[i] = canonical_nan(Omega[i]);
 }
 
 }  // namespace nicp

@@ -358,6 +358,14 @@ int nicp_align_get_state(nicp_context *ctx, int *reference_index, float *referen
 /* per-iteration trace of the last nicp_align: T at the start of each outer iteration (16), H (36),
  * b (6), error, inliers, numCorrespondences = 61 floats per iteration (test hook) */
 int nicp_align_get_trace(nicp_context *ctx, float *trace61, int max_iterations);
+/* The dense tail of Aligner::_computeStatistics (aligner.cpp:172-198) on n caller-given linearisations (test hooks):
+ * H = n x 36 (column-major 6x6), T = n x 16 (column-major 4x4) -> omega = n x 36, ratios = n x 2 (translational,
+ * rotational eigen-ratio).  Every NaN among the outputs is the quiet NaN 0x7fc00000.
+ * nicp_statistics_tail runs the kernel that finishes a batch's records on the device (it ends the state of the last
+ * nicp_align: nicp_align_get_state / _get_trace fail until the next one); nicp_statistics_tail_host needs no context and
+ * runs the host function that finishes a single nicp_align's record.  The two agree bit for bit. */
+int nicp_statistics_tail(nicp_context *ctx, int n, const float *H, const float *T, float *omega, float *ratios);
+int nicp_statistics_tail_host(int n, const float *H, const float *T, float *omega, float *ratios);
 
 /* Batched alignment of n independent pairs (loop-closure candidate verification,
  * pwn_tracker2/pwn_closer.cpp:83-182).  initial_guesses = n x 16 floats.  Results of pair i are
@@ -536,8 +544,7 @@ int nicp_frame_store_counters(const nicp_frame_store *store, long long *frames_b
  *     takes the cloud as its keyframe (keyT = globalT) and aligns nothing; its odometry is ignored.  Otherwise
  *     guess = keyT^-1 * globalT * odometry (then fixLastRow), and the keyframe (reference) is aligned against the new cloud
  *     (current): the record is byte-identical to nicp_align / nicp_multi_align with that guess, no priors and the sensor
- *     offset on both sides (except omega when the pair has no inlier at all: the batched alignment reports another Omega
- *     there than the single call).  Then globalT = keyT * T if inliers > 0, else globalT * guess; the rotation is re-orthogonalised
+ *     offset on both sides.  Then globalT = keyT * T if inliers > 0, else globalT * guess; the rotation is re-orthogonalised
  *     when the sequence's frame counter is a multiple of 50; fixLastRow; and the new cloud becomes the keyframe
  *     (keyT = globalT) when (float)inliers / (float)(rows * cols) < new_frame_inliers_fraction (composite pixels for a rig).
  *     The pose arithmetic is float32 in the operation order of include/pwn/compat.h, so it matches the C++ class bit for bit.

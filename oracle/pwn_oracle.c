@@ -1351,6 +1351,28 @@ static void align_linearize(const int *corr, int numCorr, const float *refPoints
   *err = (float)ed;
 }
 
+/* aligner.cpp:92-111: H + I + 1000 I, the priors at invT, dx = LDLT^-1 (-b), invT = v2t(dx) invT */
+static void gn_solve(const orc_align_params *p, const float *H, const float *b, float *invT) {
+  float Hd[36], nb[6], dx[6], dT[16];
+  memcpy(Hd, H, sizeof Hd);
+  for (int d = 0; d < 6; d++) M6(Hd, d, d) = M6(Hd, d, d) + 1.0f;
+  for (int d = 0; d < 6; d++) M6(Hd, d, d) = M6(Hd, d, d) + 1000.0f;
+  memcpy(nb, b, sizeof nb);
+  if (p->numPriors) add_priors(p, invT, Hd, nb);
+  for (int d = 0; d < 6; d++) nb[d] = -nb[d];
+  orc_ldlt_solve6(Hd, nb, dx);
+  orc_v2t(dx, dT);
+  orc_iso_mul(dT, invT, invT);
+}
+/* aligner.cpp:115-117: T = invT^-1, T = v2t(t2v(T)), fixLastRow */
+static void gn_finish(const float *invT, float *T) {
+  orc_iso_inverse(invT, T);
+  float v[6];
+  orc_t2v(T, v);
+  orc_v2t(v, T);
+  fix_last_row(T);
+}
+
 void orc_align(int nRef, const float *refPoints, const float *refNormals, const float *refCurv,
                int nCur, const float *curPoints, const float *curNormals, const float *curCurv,
                const float *curOmegaP, const float *curOmegaN,
@@ -1393,22 +1415,9 @@ void orc_align(int nRef, const float *refPoints, const float *refNormals, const 
         memcpy(tr + 52, b, 6 * sizeof(float));
         tr[58] = err; tr[59] = (float)inl; tr[60] = (float)numCorr;
       }
-      float Hd[36], nb[6], dx[6], dT[16];
-      memcpy(Hd, H, sizeof Hd);
-      for (int d = 0; d < 6; d++) M6(Hd, d, d) = M6(Hd, d, d) + 1.0f;
-      for (int d = 0; d < 6; d++) M6(Hd, d, d) = M6(Hd, d, d) + 1000.0f;
-      memcpy(nb, b, sizeof nb);
-      if (p->numPriors) add_priors(p, invT, Hd, nb);
-      for (int d = 0; d < 6; d++) nb[d] = -nb[d];
-      orc_ldlt_solve6(Hd, nb, dx);
-      orc_v2t(dx, dT);
-      orc_iso_mul(dT, invT, invT);
+      gn_solve(p, H, b, invT);
     }
-    orc_iso_inverse(invT, T);
-    float v[6];
-    orc_t2v(T, v);
-    orc_v2t(v, T);
-    fix_last_row(T);
+    gn_finish(invT, T);
   }
   res->error = err;
   res->inliers = inl;
@@ -1422,6 +1431,26 @@ void orc_align(int nRef, const float *refPoints, const float *refNormals, const 
   memcpy(res->H, H, sizeof res->H);
   memcpy(res->b, b, sizeof res->b);
   compute_statistics(H, T, res->mean, res->omega, &res->translationalRatio, &res->rotationalRatio);
+}
+
+void orc_compute_statistics(const float H[36], const float T[16], float mean[6], float Omega[36], float *tr, float *rr) {
+  compute_statistics(H, T, mean, Omega, tr, rr);
+}
+
+/* orc_align's outer iteration (inner = 1) from its linearisation on */
+void orc_gn_step(const float H[36], const float b[6], const float T[16], const orc_prior *priors, int numPriors,
+                 float Tnext[16]) {
+  orc_align_params p;
+  memset(&p, 0, sizeof p);
+  p.numPriors = numPriors;
+  p.priors = priors;
+  float Tc[16], invT[16];
+  memcpy(Tc, T, sizeof Tc);
+  fix_last_row(Tc);
+  orc_iso_inverse(Tc, invT);
+  fix_last_row(invT);
+  gn_solve(&p, H, b, invT);
+  gn_finish(invT, Tnext);
 }
 
 /* PwnMatcherBase::matchClouds, pwn_tracker2/pwn_matcher_base.cpp:167-196.  NB: the reference

@@ -188,6 +188,14 @@ void orc_align(int nRef, const float *refPoints, const float *refNormals, const 
                const orc_align_params *p, orc_align_result *res,
                int *refIndex, float *refDepth, int *curIndex, float *curDepth, int *corr,
                float *trace);
+/* the two dense pieces of orc_align on their own (the same static functions, no behaviour of their own):
+ * orc_compute_statistics is the _computeStatistics tail (aligner.cpp:172-198) on the linearisation H at T;
+ * orc_gn_step is one outer iteration with innerIterations = 1 after its linearisation (aligner.cpp:84-118): invT = T^-1
+ * (fixLastRow), H + I + 1000 I and -b with the priors added at invT, LDLT, invT = v2t(dx) invT, T = v2t(t2v(invT^-1)),
+ * fixLastRow -> Tnext.  Matrices column-major. */
+void orc_compute_statistics(const float H[36], const float T[16], float mean[6], float Omega[36], float *tr, float *rr);
+void orc_gn_step(const float H[36], const float b[6], const float T[16], const orc_prior *priors, int numPriors,
+                 float Tnext[16]);
 
 /* test knob: float64 accumulation of the Linearizer sums inside orc_align (0 = reference behaviour) */
 void orc_set_accumulate_f64(int on);

@@ -378,6 +378,30 @@ def ldlt_solve6(H, b):
     return x
 
 
+def compute_statistics(H, T):
+    """_computeStatistics' dense tail (orc_compute_statistics) on the linearisation H (6, 6) at the pose T (4, 4) ->
+    (mean (6,), Omega (6, 6), translational ratio, rotational ratio)"""
+    Hc, hp = _f(colmajor(H))
+    Tc, tp = _f(colmajor(T))
+    mean = np.zeros(6, np.float32)
+    om = np.zeros(36, np.float32)
+    tr, rr = C.c_float(0), C.c_float(0)
+    lib().orc_compute_statistics(hp, tp, _fp(mean), _fp(om), C.byref(tr), C.byref(rr))
+    return mean, from_colmajor(om, 6), np.float32(tr.value), np.float32(rr.value)
+
+
+def gn_step(H, b, T, priors=()):
+    """one outer iteration of align() with inner = 1 after its linearisation (orc_gn_step): H (6, 6), b (6,) at T (4, 4),
+    priors a sequence of Prior (make_prior) -> the next T (4, 4)"""
+    Hc, hp = _f(colmajor(H))
+    bb, bp = _f(b)
+    Tc, tp = _f(colmajor(T))
+    out = np.zeros(16, np.float32)
+    parr = (Prior * len(priors))(*priors) if len(priors) else None
+    lib().orc_gn_step(hp, bp, tp, parr, len(priors), _fp(out))
+    return from_colmajor(out, 4)
+
+
 def make_prior(kind, mean, info, reference=None):
     p = Prior()
     p.kind = kind
@@ -632,7 +656,8 @@ def _declare():
         for name in ("orc_depth_u16_to_f32", "orc_depth_scale", "orc_v2t", "orc_t2v", "orc_update_matrices",
                      "orc_project_intervals", "orc_project", "orc_integral_image", "orc_eigen3", "orc_linearize",
                      "orc_linearize_f64", "orc_ldlt_solve6", "orc_align", "orc_image_stats", "orc_multi_image_size",
-                     "orc_multi_intervals", "orc_multi_project", "orc_set_accumulate_f64", "orc_cloud_transform", "orc_gaussians_transform"):
+                     "orc_multi_intervals", "orc_multi_project", "orc_set_accumulate_f64", "orc_cloud_transform", "orc_gaussians_transform",
+                     "orc_compute_statistics", "orc_gn_step"):
             getattr(l, name).restype = None
 
 

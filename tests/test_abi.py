@@ -116,6 +116,10 @@ def test_null_handles_are_rejected_not_dereferenced(verify):
     assert L.nicp_align(N, N, N, N, N, N, N, N, N, 0, f0, N) == 1
     assert L.nicp_align_get_state(N, N, N, N, N, N, N, N) == 1
     assert L.nicp_align_get_trace(N, N, 0) == 1
+    assert L.nicp_statistics_tail(N, 1, N, N, N, N) == 1
+    assert L.nicp_statistics_tail_host(1, N, N, N, N) == 1
+    assert L.nicp_statistics_tail_host(-1, N, N, N, N) == 1
+    assert L.nicp_statistics_tail_host(0, N, N, N, N) == 0
     assert L.nicp_align_batch(N, 0, N, N, N, N, N, N, N, f0, N) == 1
     assert L.nicp_align_batch_priors(N, 0, N, N, N, N, N, N, N, N, N, f0, N) == 1
     assert L.nicp_multi_depth_to_cloud(N, N, N, N, N, 0, N, N) == 1

@@ -20,9 +20,6 @@ from test_rig_sharded import SP as RIG_SP
 
 POOLS = ([0], [0, 0], [0, 0, 0])
 FRACTION = 0.6  # keyframe threshold that makes the synthetic sweeps switch keyframes (test_sequential_tracker_*)
-# a pair without a single inlier: the batched alignment every tracker step runs (as nicp_align_batch and the sharded
-# entries do) reports another Omega than nicp_align; every other field, and so the tracker's bookkeeping, is identical
-ZERO_INLIER_FIELDS = ("omega",)
 f32 = np.float32
 
 
@@ -240,8 +237,7 @@ def check_sequence(results, q, case, chain):
             want = np.frombuffer(chain.align(q, key, t, capi.from_colmajor(r["guess"], 4)), capi.RESULT_DTYPE)[0]
             got = r["record"]
             differ = [f for f in capi.RESULT_DTYPE.names if got[f].tobytes() != want[f].tobytes()]
-            allowed = ZERO_INLIER_FIELDS if int(got["inliers"]) == 0 else ()
-            assert set(differ) <= set(allowed), (q, t, {f: (got[f], want[f]) for f in differ})
+            assert not differ, (q, t, {f: (got[f], want[f]) for f in differ})
             assert np.array_equal(r["relative_T"].view(np.uint32), r["record"]["T"].view(np.uint32)), (q, t)
             assert r["record"]["status"] == 0
         else:
