@@ -38,6 +38,8 @@ SYMBOLS = [
     "nicp_frame_store_remove", "nicp_frame_store_size", "nicp_frame_store_align", "nicp_frame_store_counters",
     "nicp_tracker_create", "nicp_multi_tracker_create", "nicp_tracker_destroy", "nicp_tracker_size", "nicp_tracker_step",
     "nicp_tracker_reset",
+    "nicp_scene_tracker_create", "nicp_scene_tracker_destroy", "nicp_scene_tracker_size", "nicp_scene_tracker_step",
+    "nicp_scene_tracker_reset", "nicp_scene_tracker_download_map", "nicp_scene_tracker_phase_ms",
 ]
 
 GAUSS_FLOATS = 24
@@ -120,6 +122,19 @@ TRACK_DTYPE = np.dtype([("global_T", np.float32, 16), ("relative_T", np.float32,
 assert TRACK_DTYPE.itemsize == 464
 
 
+class SceneTrackResult(C.Structure):
+    _fields_ = [("global_T", C.c_float * 16), ("scene_T", C.c_float * 16), ("frame", C.c_int), ("aligned", C.c_int),
+                ("new_map", C.c_int), ("added", C.c_int), ("map_points", C.c_int), ("record", AlignResult)]
+
+
+assert C.sizeof(SceneTrackResult) == 404
+
+SCENE_TRACK_DTYPE = np.dtype([("global_T", np.float32, 16), ("scene_T", np.float32, 16), ("frame", np.int32),
+                              ("aligned", np.int32), ("new_map", np.int32), ("added", np.int32), ("map_points", np.int32),
+                              ("record", RESULT_DTYPE)])
+assert SCENE_TRACK_DTYPE.itemsize == 404
+
+
 def lib_path(verify=False):
     return os.path.join(LIB_DIR, "libnicp_b200_verify.so" if verify else "libnicp_b200.so")
 
@@ -148,6 +163,7 @@ def load(verify=False):
     L.nicp_multi_image_size.restype = None
     L.nicp_frame_store_destroy.restype = None
     L.nicp_tracker_destroy.restype = None
+    L.nicp_scene_tracker_destroy.restype = None
     for name in SYMBOLS:
         fn = getattr(L, name)
         if fn.restype is C.c_int:
@@ -1053,6 +1069,106 @@ class Tracker:
     def close(self):
         if self.handle:
             self.L.nicp_tracker_destroy(self.handle)
+            self.handle = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class SceneTracker:
+    """nicp_scene_tracker: S independent pinhole depth sequences, each running the scene-based odometry of
+    pwn_core/pwn_aligner.cpp (align against the local map re-rendered at the predicted pose, add the frame, merge) with its
+    local map resident on the workers of a shard pool (sequence s on worker s * G // S).  One step takes one frame of each
+    listed sequence.
+
+    proj describes the image after scaling (raw_shape = (rows, cols) of every raw frame); sp, ap and mp are the statistics,
+    alignment and merge parameters; baseline and alpha the sensor model of the map's gaussians; chunk_step closes the map
+    after the first alignment and then every chunk_step frames (0: never); map_capacity is the points each map can hold.
+    Every argument is fixed for the tracker's lifetime."""
+
+    def __init__(self, pool, proj, sp, ap, raw_shape, n_sequences, map_capacity, mp=None, depth_scale=0.001, step=1,
+                 max_depth_cov=0.01, sensor_offset=None, baseline=0.075, alpha=0.1, img_threshold=50.0, chunk_step=10):
+        self.pool = pool  # the tracker's clouds live on the pool's workers
+        self.L = pool.L
+        self.handle = C.c_void_p()
+        self.map_capacity = int(map_capacity)
+        so = None if sensor_offset is None else _fptr(colmajor(sensor_offset))
+        # the C call reads raw_rows x raw_cols pixels from whatever pointer it is given, so step() checks each image
+        self.raw_shape = tuple(int(x) for x in raw_shape)
+        mp = make_merge_params() if mp is None else mp
+        rows, cols = self.raw_shape
+        _check(self.L, self.L.nicp_scene_tracker_create(
+            pool.handle, int(n_sequences), rows, cols, C.c_float(depth_scale), int(step), C.c_float(max_depth_cov),
+            C.byref(proj), C.byref(sp), so, C.c_float(baseline), C.c_float(alpha), C.byref(ap), C.c_float(img_threshold),
+            C.byref(mp), int(chunk_step), self.map_capacity, C.byref(self.handle)))
+
+    def step(self, sequences, frames):
+        """frames[k] is the next uint16 frame of sequence sequences[k], of exactly the raw shape given at creation (any
+        other shape raises ValueError and the library is not called).  Returns SCENE_TRACK_DTYPE results."""
+        seqs = np.ascontiguousarray(sequences, np.int32)
+        n = len(seqs)
+        if len(frames) != n:
+            raise ValueError("%d sequences for %d frames" % (n, len(frames)))
+        imgs = []
+        for k, im in enumerate(frames):
+            im = np.ascontiguousarray(im, np.uint16)
+            if im.shape != self.raw_shape:
+                raise ValueError("frame %d: raw image of shape %s, the tracker takes %s" % (k, im.shape, self.raw_shape))
+            imgs.append(im)
+        RA = (C.c_void_p * max(n, 1))(*[im.ctypes.data for im in imgs])
+        results = np.zeros(n, SCENE_TRACK_DTYPE)
+        _check(self.L, self.L.nicp_scene_tracker_step(self.handle, n, _iptr(seqs), RA,
+                                                      results.ctypes.data_as(C.POINTER(SceneTrackResult))))
+        return results
+
+    def reset(self, sequences, initial_poses=None):
+        """the listed sequences start over with an empty map: globalT = sceneT = initial_poses[k] ((4, 4) each; None:
+        identity)"""
+        seqs = np.ascontiguousarray(sequences, np.int32)
+        n = len(seqs)
+        if initial_poses is not None and len(initial_poses) != n:
+            raise ValueError("%d initial poses for %d sequences" % (len(initial_poses), n))
+        _check(self.L, self.L.nicp_scene_tracker_reset(self.handle, n, _iptr(seqs), _guesses(initial_poses, n)))
+
+    def download_map(self, sequence):
+        """the map of one sequence: dict of points (n, 4), normals (n, 4), curvature (n,), omega_p / omega_n (n, 6),
+        gauss (n, 24) and gflags (n,), as Cloud.download and Cloud.download_gaussians give them"""
+        n = C.c_int(-1)
+        nulls = (None,) * 7
+        rc = self.L.nicp_scene_tracker_download_map(self.handle, int(sequence), 0, *nulls, C.byref(n))
+        if n.value < 0:  # not even the size: a bad handle or sequence
+            _check(self.L, rc)
+        cap = max(n.value, 0)
+        pts = np.zeros((cap, 4), np.float32)
+        nrm = np.zeros((cap, 4), np.float32)
+        curv = np.zeros(cap, np.float32)
+        op = np.zeros((cap, 6), np.float32)
+        on = np.zeros((cap, 6), np.float32)
+        g = np.zeros((cap, GAUSS_FLOATS), np.float32)
+        f = np.zeros(cap, np.int32)
+        n = C.c_int(0)
+        _check(self.L, self.L.nicp_scene_tracker_download_map(self.handle, int(sequence), cap, _fptr(pts), _fptr(nrm),
+                                                              _fptr(curv), _fptr(op), _fptr(on), _fptr(g), _iptr(f),
+                                                              C.byref(n)))
+        m = n.value
+        return {"points": pts[:m], "normals": nrm[:m], "curvature": curv[:m], "omega_p": op[:m], "omega_n": on[:m],
+                "gauss": g[:m], "gflags": f[:m]}
+
+    def phase_ms(self):
+        """host milliseconds of phase 1 (prep, render, alignment) and phase 2 (append, merges), summed over every step"""
+        a, b = C.c_double(0.0), C.c_double(0.0)
+        _check(self.L, self.L.nicp_scene_tracker_phase_ms(self.handle, C.byref(a), C.byref(b)))
+        return a.value, b.value
+
+    def size(self):
+        return int(self.L.nicp_scene_tracker_size(self.handle))
+
+    def close(self):
+        if self.handle:
+            self.L.nicp_scene_tracker_destroy(self.handle)
             self.handle = C.c_void_p()
 
     def __del__(self):

@@ -361,6 +361,41 @@ int launch_decode_z(nicp_context *ctx, const unsigned long long *d_z, int n, int
   return NICP_OK;
 }
 
+// nicp_project of the maps of a launch set (map f = blockIdx.y), each with its own KRt, into z-buffers zStride words apart;
+// then their depth images (FLT_MAX where empty) into depth slots depthStride floats apart.  The z pass is k_project_single's
+// (project_point: nearest wins, lowest index wins ties), so each depth image is nicp_project's bit for bit.
+__global__ void __launch_bounds__(256) k_render_maps_z(MapRenderSet R, int rows, int cols, float minD, float maxD,
+                                                       unsigned long long *__restrict__ z0, size_t zStride) {
+  const int f = blockIdx.y;
+  const int n = *R.count[f];
+  const float4 *__restrict__ pts = R.points[f];
+  unsigned long long *z = z0 + (size_t)f * zStride;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    project_point(R.KRt[f], pts[i], i, rows, cols, minD, maxD, z, kEpochFresh);
+}
+__global__ void k_render_maps_depth(const unsigned long long *__restrict__ z0, size_t zStride, int P, float *__restrict__ depth0,
+                                    size_t depthStride) {
+  const int f = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P) return;
+  depth0[(size_t)f * depthStride + i] = z_depth(z0[(size_t)f * zStride + i], kEpochFresh, FLT_MAX);
+}
+
+int launch_render_maps(nicp_context *ctx, const MapRenderSet &R, int m, int maxPoints, const nicp_projector *proj,
+                       unsigned long long *d_z, size_t zStride, float *d_depth, size_t depthStride) {
+  const int P = proj->rows * proj->cols;
+  for (int f = 0; f < m; f++)
+    NICP_CUDA(cudaMemsetAsync(d_z + (size_t)f * zStride, 0xFF, (size_t)P * sizeof(unsigned long long), ctx->stream));
+  // grid-stride over the points: the counts are read on the device, maxPoints (the host's mirror) only sizes the grid
+  const int blocks = std::max(1, std::min((maxPoints + 255) / 256, ctx->smCount * 8));
+  k_render_maps_z<<<dim3(blocks, m), 256, 0, ctx->stream>>>(R, proj->rows, proj->cols, proj->min_distance,
+                                                            proj->max_distance, d_z, zStride);
+  NICP_CHECK_LAUNCH(ctx);
+  k_render_maps_depth<<<dim3((P + 255) / 256, m), 256, 0, ctx->stream>>>(d_z, zStride, P, d_depth, depthStride);
+  NICP_CHECK_LAUNCH(ctx);
+  return NICP_OK;
+}
+
 // ---------------------------------------------------------------------------------------------
 // SE3Prior / SE3RelativePrior / SE3AbsolutePrior (se3_prior.cpp:8-71) and their use in the
 // Gauss-Newton step (aligner.cpp:97-108), evaluated by the solving thread.  Numeric Jacobians with

@@ -737,6 +737,20 @@ int launch_frame_prep(nicp_context *ctx, const float *d_depth, const nicp_projec
   return NICP_OK;
 }
 
+// frame f of a launch set of n <= kMaxPrepBatch frames of fs -> depth and integral slot f of the batch scratch, cloud f
+static int batch_scratch(nicp_context *ctx, const FrameSet &fs, int n, int keepStats, nicp_cloud *const *clouds, PrepBatch &B) {
+  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
+  if (n > ctx->batchSlots || px > ctx->batchPixels) {
+    set_error("internal: batch prep scratch too small");
+    return NICP_ERR_INVALID;
+  }
+  memset(&B, 0, sizeof B);
+  for (int f = 0; f < n; f++)
+    prep_batch_add(B, ctx->d_bDepth + (size_t)f * ctx->batchPixels, ctx->d_bIntegral + (size_t)f * ctx->batchPixels * kIntegralCh,
+                   clouds[f], keepStats != 0);
+  return NICP_OK;
+}
+
 // n raw 16-bit frames of fs already on the device (d_raw[f * fs.cams.n + i] = camera i of frame f) -> n clouds: one depth
 // conversion launch for every camera of every frame, then the launch set above.  n <= kMaxPrepBatch frames, whose scratch
 // (depth + integral image, 44 B/pixel/frame) stays L2 resident.
@@ -744,16 +758,9 @@ int launch_raw_prep_batch(nicp_context *ctx, const FrameSet &fs, int n, const ui
                           const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds) {
   const nicp_projector *proj = &fs.proj;
   const CamSet &cams = fs.cams;
-  const size_t px = (size_t)proj->rows * proj->cols;
-  if (n > ctx->batchSlots || px > ctx->batchPixels) {
-    set_error("internal: batch prep scratch too small");
-    return NICP_ERR_INVALID;
-  }
   PrepBatch B;
-  memset(&B, 0, sizeof B);
-  for (int f = 0; f < n; f++)
-    prep_batch_add(B, ctx->d_bDepth + (size_t)f * ctx->batchPixels, ctx->d_bIntegral + (size_t)f * ctx->batchPixels * kIntegralCh,
-                   clouds[f], keepStats != 0);
+  int rc;
+  if ((rc = batch_scratch(ctx, fs, n, keepStats, clouds, B))) return rc;
   if (cams.multi) {
     // composite image: rows = max width, cols = sum of heights
     RigFrames R;
@@ -782,6 +789,16 @@ int launch_raw_prep_batch(nicp_context *ctx, const FrameSet &fs, int n, const ui
   }
   NICP_CHECK_LAUNCH(ctx);
   return launch_prep_set(ctx, B, proj, sp, sensorOffset, nullptr, nullptr, &cams);
+}
+
+// the launch set above entered from depth images already in the first n depth slots of the batch scratch (a scene
+// tracker renders its maps there): no upload, no conversion
+int launch_depth_prep_batch(nicp_context *ctx, const FrameSet &fs, int n, const nicp_stats_params *sp,
+                            const float sensorOffset[16], nicp_cloud *const *clouds) {
+  PrepBatch B;
+  int rc;
+  if ((rc = batch_scratch(ctx, fs, n, 0, clouds, B))) return rc;
+  return launch_prep_set(ctx, B, &fs.proj, sp, sensorOffset, nullptr, nullptr, &fs.cams);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -542,36 +542,30 @@ __global__ void k_local_map_rig_gaussians(LocalMapSet S, const float *__restrict
   S.gflags[f][slot] = NICP_GAUSS_MOMENTS;
 }
 
-// Cloud::add (cloud.cpp:145-171) of every frame cloud of the set, in frame order, behind *run points: point record and
-// gaussian of point i of frame f moved by pose f (k_cloud_append, k_gauss_append).  A set that does not fit below
-// dstCapacity writes nothing; *run advances regardless (k_local_map_advance), so the final count is the size the map needs.
-__global__ void __launch_bounds__(256) k_local_map_append(LocalMapSet S, int m, const long long *__restrict__ run,
-                                                          int dstCapacity, float4 *__restrict__ dp, float4 *__restrict__ dn,
-                                                          float4 *__restrict__ dom, float *__restrict__ dg,
-                                                          int *__restrict__ df) {
-  const int f = blockIdx.y;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int n = *S.count[f];
-  if (i >= n) return;
-  long long before = 0, total = 0;
-  for (int k = 0; k < m; k++) {
-    const int nk = *S.count[k];
-    if (k < f) before += nk;
-    total += nk;
-  }
-  const long long base = *run;
-  if (base + total > dstCapacity) return;
-  const size_t o = (size_t)(base + before + i);
-  float4 p = S.points[f][i], nn = S.normals[f][i];
-  const float4 *so = S.omega[f] + 3 * (size_t)i;
-  float4 o0 = so[0], o1 = so[1], o2 = so[2];
+// Cloud::add (cloud.cpp:145-171) of one point with its gaussian: source point i moved by M (unless identity) and written at
+// destination slot o.  The per-point body of k_local_map_append and k_scene_append.
+__device__ __forceinline__ void append_point(const float4 *__restrict__ sp, const float4 *__restrict__ sn,
+                                             const float4 *__restrict__ som, const float *__restrict__ sg,
+                                             const int *__restrict__ sf, int i, const Affine &M, int identity,
+                                             float4 *__restrict__ dp, float4 *__restrict__ dn, float4 *__restrict__ dom,
+                                             float *__restrict__ dg, int *__restrict__ df, size_t o) {
+  // the sources are read-only for the whole launch: read them through the non-coherent path (ld.global.nc), which the
+  // restrict qualifiers of an inlined helper do not let the compiler infer on its own
+  float4 p = __ldg(sp + i), nn = __ldg(sn + i);
+  const float4 *so = som + 3 * (size_t)i;
+  float4 o0 = __ldg(so), o1 = __ldg(so + 1), o2 = __ldg(so + 2);
   float g[kGF];
-  gauss_load(S.gauss[f] + (size_t)kGF * i, g);
-  int gf = S.gflags[f][i];
-  if (!S.poseIdentity[f]) {
-    xform_record(S.pose[f], p, nn, o0, o1, o2);
+  const float4 *gs = reinterpret_cast<const float4 *>(sg + (size_t)kGF * i);
+#pragma unroll
+  for (int k = 0; k < kGF / 4; k++) {
+    const float4 v = __ldg(gs + k);
+    g[4 * k] = v.x; g[4 * k + 1] = v.y; g[4 * k + 2] = v.z; g[4 * k + 3] = v.w;
+  }
+  int gf = __ldg(sf + i);
+  if (!identity) {
+    xform_record(M, p, nn, o0, o1, o2);
     gauss_update_moments(g, gf);
-    gauss_xform_moments(S.pose[f], g);
+    gauss_xform_moments(M, g);
     gf = NICP_GAUSS_MOMENTS;
   }
   dp[o] = p;
@@ -581,6 +575,29 @@ __global__ void __launch_bounds__(256) k_local_map_append(LocalMapSet S, int m, 
   dom[3 * o + 2] = o2;
   gauss_store(dg + kGF * o, g);
   df[o] = gf;
+}
+
+// Cloud::add (cloud.cpp:145-171) of every frame cloud of the set, in frame order, behind *run points: point record and
+// gaussian of point i of frame f moved by pose f (k_cloud_append, k_gauss_append).  A set that does not fit below
+// dstCapacity writes nothing; *run advances regardless (k_local_map_advance), so the final count is the size the map needs.
+__global__ void __launch_bounds__(256) k_local_map_append(LocalMapSet S, int m, const long long *__restrict__ run,
+                                                          int dstCapacity, float4 *__restrict__ dp, float4 *__restrict__ dn,
+                                                          float4 *__restrict__ dom, float *__restrict__ dg,
+                                                          int *__restrict__ df) {
+  const int f = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int n = __ldg(S.count[f]);
+  if (i >= n) return;
+  long long before = 0, total = 0;
+  for (int k = 0; k < m; k++) {
+    const int nk = __ldg(S.count[k]);
+    if (k < f) before += nk;
+    total += nk;
+  }
+  const long long base = __ldg(run);
+  if (base + total > dstCapacity) return;
+  append_point(S.points[f], S.normals[f], S.omega[f], S.gauss[f], S.gflags[f], i, S.pose[f], S.poseIdentity[f], dp, dn, dom,
+               dg, df, (size_t)(base + before + i));
 }
 __global__ void k_local_map_advance(LocalMapSet S, int m, long long *run) {
   long long total = 0;
@@ -607,13 +624,12 @@ int launch_local_map_begin(nicp_context *ctx, nicp_cloud *map, long long *d_run)
 int launch_local_map_set(nicp_context *ctx, const FrameSet &fs, int m, nicp_cloud *const *frames, const float *poses,
                          const float *baseline, const float *alpha, const float sensorOffset[16], nicp_cloud *map,
                          long long *d_run) {
-  const nicp_projector *proj = &fs.proj;
-  const int P = proj->rows * proj->cols;
+  const int P = fs.proj.rows * fs.proj.cols;
+  int rc;
+  if ((rc = launch_set_gaussians(ctx, fs, m, frames, baseline, alpha, sensorOffset))) return rc;
   LocalMapSet S;
   memset(&S, 0, sizeof S);
   for (int f = 0; f < m; f++) {
-    int rc = cloud_ensure_gaussians(ctx, frames[f]);
-    if (rc) return rc;
     S.points[f] = frames[f]->points;
     S.normals[f] = frames[f]->normals;
     S.omega[f] = frames[f]->omega;
@@ -625,6 +641,28 @@ int launch_local_map_set(nicp_context *ctx, const FrameSet &fs, int m, nicp_clou
     fix_last_row(T);
     S.pose[f] = affine_from(T);
     S.poseIdentity[f] = is_identity16(T) ? 1 : 0;
+  }
+  k_local_map_append<<<dim3((P + 255) / 256, m), 256, 0, ctx->stream>>>(S, m, d_run, map->capacity, map->points, map->normals,
+                                                                        map->omega, map->gauss, map->gflags);
+  NICP_CHECK_LAUNCH(ctx);
+  k_local_map_advance<<<1, 1, 0, ctx->stream>>>(S, m, d_run);
+  NICP_CHECK_LAUNCH(ctx);
+  return NICP_OK;
+}
+
+// the gaussians of the m frame clouds of the launch set that launch_raw_prep_batch has just queued, from its depth and
+// integral images in the batch scratch.  baseline, alpha: one per camera of fs.
+int launch_set_gaussians(nicp_context *ctx, const FrameSet &fs, int m, nicp_cloud *const *frames, const float *baseline,
+                         const float *alpha, const float sensorOffset[16]) {
+  const nicp_projector *proj = &fs.proj;
+  const int P = proj->rows * proj->cols;
+  LocalMapSet S;
+  memset(&S, 0, sizeof S);
+  for (int f = 0; f < m; f++) {
+    int rc = cloud_ensure_gaussians(ctx, frames[f]);
+    if (rc) return rc;
+    S.gauss[f] = frames[f]->gauss;
+    S.gflags[f] = frames[f]->gflags;
     frames[f]->has_gauss = true;
   }
   float M[16];
@@ -643,11 +681,90 @@ int launch_local_map_set(nicp_context *ctx, const FrameSet &fs, int m, nicp_clou
                                                                             sm.iKRt, sm.fB, alpha[0]);
   }
   NICP_CHECK_LAUNCH(ctx);
-  k_local_map_append<<<dim3((P + 255) / 256, m), 256, 0, ctx->stream>>>(S, m, d_run, map->capacity, map->points, map->normals,
-                                                                        map->omega, map->gauss, map->gflags);
-  NICP_CHECK_LAUNCH(ctx);
-  k_local_map_advance<<<1, 1, 0, ctx->stream>>>(S, m, d_run);
-  NICP_CHECK_LAUNCH(ctx);
+  return NICP_OK;
+}
+
+// Frames appended to their own maps in one launch (frame f = blockIdx.y of k_scene_append): source cloud, destination
+// cloud and the pose the frame is appended with.  A kernel parameter (about 150 B per frame).
+constexpr int kSceneAppendFrames = 64;
+struct SceneAppendSet {
+  const float4 *points[kSceneAppendFrames], *normals[kSceneAppendFrames], *omega[kSceneAppendFrames];
+  const float *gauss[kSceneAppendFrames];
+  const int *gflags[kSceneAppendFrames], *count[kSceneAppendFrames];
+  float4 *dp[kSceneAppendFrames], *dn[kSceneAppendFrames], *dom[kSceneAppendFrames];
+  float *dg[kSceneAppendFrames];
+  int *df[kSceneAppendFrames], *dstN[kSceneAppendFrames];
+  int dstCapacity[kSceneAppendFrames];
+  Affine pose[kSceneAppendFrames];
+  int poseIdentity[kSceneAppendFrames];
+};
+
+// Cloud::add (cloud.cpp:145-171) of m frames, each to its own map: point record and gaussian of point i of frame f moved
+// by pose f (append_point) and written behind *dstN[f] points.  The caller has checked that every
+// frame fits; a frame that would not fit writes nothing.  The counts advance in k_scene_append_advance.
+__global__ void __launch_bounds__(256) k_scene_append(SceneAppendSet S) {
+  const int f = blockIdx.y;
+  const int n = *S.count[f];
+  const long long base = *S.dstN[f];
+  if (base + n > S.dstCapacity[f]) return;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    append_point(S.points[f], S.normals[f], S.omega[f], S.gauss[f], S.gflags[f], i, S.pose[f], S.poseIdentity[f], S.dp[f],
+                 S.dn[f], S.dom[f], S.dg[f], S.df[f], (size_t)(base + i));
+}
+__global__ void k_scene_append_advance(SceneAppendSet S, int m) {
+  const int f = threadIdx.x;
+  if (f >= m) return;
+  const int n = *S.count[f];
+  if ((long long)*S.dstN[f] + n <= S.dstCapacity[f]) *S.dstN[f] += n;
+}
+
+// nicp_cloud_append(maps[k], frames[k], poses + 16 k) for n frames with gaussians and distinct maps that carry gaussians,
+// one launch per kSceneAppendFrames frames.  framePoints / mapPoints: the host's counts, which the caller has checked to
+// fit; they size the grid and the maps' host mirrors (the kernel reads the counts on the device).
+int launch_scene_append(nicp_context *ctx, int n, nicp_cloud *const *frames, nicp_cloud *const *maps, const float *poses,
+                        const int *framePoints, const int *mapPoints) {
+  for (int base = 0; base < n; base += kSceneAppendFrames) {
+    const int m = std::min(kSceneAppendFrames, n - base);
+    SceneAppendSet S;
+    memset(&S, 0, sizeof S);
+    int maxPoints = 0;
+    for (int f = 0; f < m; f++) {
+      const int k = base + f;
+      const nicp_cloud *src = frames[k];
+      nicp_cloud *dst = maps[k];
+      S.points[f] = src->points;
+      S.normals[f] = src->normals;
+      S.omega[f] = src->omega;
+      S.gauss[f] = src->gauss;
+      S.gflags[f] = src->gflags;
+      S.count[f] = src->d_n;
+      S.dp[f] = dst->points;
+      S.dn[f] = dst->normals;
+      S.dom[f] = dst->omega;
+      S.dg[f] = dst->gauss;
+      S.df[f] = dst->gflags;
+      S.dstN[f] = dst->d_n;
+      S.dstCapacity[f] = dst->capacity;
+      float T[16];
+      for (int i = 0; i < 16; i++) T[i] = poses[16 * (size_t)k + i];
+      fix_last_row(T);
+      S.pose[f] = affine_from(T);
+      S.poseIdentity[f] = is_identity16(T) ? 1 : 0;
+      maxPoints = std::max(maxPoints, framePoints[k]);
+    }
+    k_scene_append<<<dim3(std::max(1, (maxPoints + 255) / 256), m), 256, 0, ctx->stream>>>(S);
+    NICP_CHECK_LAUNCH(ctx);
+    k_scene_append_advance<<<1, kSceneAppendFrames, 0, ctx->stream>>>(S, m);
+    NICP_CHECK_LAUNCH(ctx);
+  }
+  for (int k = 0; k < n; k++) {  // like launch_local_map_commit
+    nicp_cloud *map = maps[k];
+    map->points3_valid = false; map->pn_valid = false;
+    map->has_stats = false;
+    map->has_gauss = true;
+    map->n_host = mapPoints[k] + framePoints[k];
+    map->n_known = true;
+  }
   return NICP_OK;
 }
 

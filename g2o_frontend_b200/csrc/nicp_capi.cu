@@ -441,6 +441,50 @@ int prep_frames(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *co
   return NICP_OK;
 }
 
+// The device half of a scene tracker's step before its alignment, for n sequences of one worker (the caller has checked
+// the arguments): frame k is prepared from raws[k] into frames[k] (keep_stats 0) with the gaussians of
+// nicp_cloud_compute_gaussians(baseline, alpha, sensorOffset); if maps[k] is not null, it is rendered as nicp_project renders
+// it from views + 16 k (KRt) into the depth slot of the set's scratch and subs[k] is prepared from that depth image as
+// nicp_depth_to_cloud prepares it.  mapPoints[k] is the host's count of maps[k].  Launch sets of up to 8 frames: one prep
+// of the frames, their gaussians, one render of the set's maps (z-buffers in the set's integral scratch, which the
+// subscenes' prep overwrites next), one prep of the subscenes.  Asynchronous.
+int prep_scene_frames(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *raws, const nicp_stats_params *sp,
+                      const float sensorOffset[16], float baseline, float alpha, nicp_cloud *const *frames,
+                      const nicp_cloud *const *maps, const int *mapPoints, const float *views, nicp_cloud *const *subs) {
+  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
+  const int sub = prep_set_frames(fs, n);
+  int rc;
+  if ((rc = ensure_batch_prep(ctx, sub, px, fs.rawPixels))) return rc;
+  static_assert(kIntegralCh * sizeof(float) >= sizeof(unsigned long long), "a z-buffer fits a frame's integral slot");
+  for (int base = 0; base < n; base += sub) {
+    const int m = std::min(sub, n - base);
+    if ((rc = prep_set(ctx, fs, m, raws + base, sp, sensorOffset, 0, frames + base)) ||
+        (rc = launch_set_gaussians(ctx, fs, m, frames + base, &baseline, &alpha, sensorOffset)))
+      return rc;
+    MapRenderSet R;
+    memset(&R, 0, sizeof R);
+    nicp_cloud *setSubs[kMaxPrepBatch];
+    int rm = 0, maxPoints = 0;
+    for (int f = 0; f < m; f++) {
+      const int k = base + f;
+      if (!maps[k]) continue;
+      R.points[rm] = maps[k]->points;
+      R.count[rm] = maps[k]->d_n;
+      R.KRt[rm] = affine_from(views + 16 * (size_t)k);
+      setSubs[rm++] = subs[k];
+      maxPoints = std::max(maxPoints, mapPoints[k]);
+    }
+    if (!rm) continue;
+    if ((rc = launch_render_maps(ctx, R, rm, maxPoints, &fs.proj, reinterpret_cast<unsigned long long *>(ctx->d_bIntegral),
+                                 ctx->batchPixels * kIntegralCh * sizeof(float) / sizeof(unsigned long long), ctx->d_bDepth,
+                                 ctx->batchPixels)) ||
+        (rc = launch_depth_prep_batch(ctx, fs, rm, sp, sensorOffset, setSubs)))
+      return rc;
+  }
+  ctx->lastRows = 0;
+  return NICP_OK;
+}
+
 static AlignConsts make_consts(const nicp_projector *proj, const nicp_align_params *ap, const float *refOffset) {
   AlignConsts ac;
   memset(&ac, 0, sizeof ac);

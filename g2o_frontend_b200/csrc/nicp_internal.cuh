@@ -275,6 +275,14 @@ struct FrameSet {
   int slotCap;                               // pairs per lock-step align chunk (NICP_BATCH_SLOTS can lower it)
 };
 
+// The maps a launch set of a scene tracker renders (map f = blockIdx.y of k_render_maps_z): points, device count and the
+// KRt of the view each is rendered from.  A kernel parameter, like PrepBatch.
+struct MapRenderSet {
+  const float4 *points[kMaxPrepBatch];
+  const int *count[kMaxPrepBatch];
+  Affine KRt[kMaxPrepBatch];
+};
+
 struct AlignConsts {
   float K[9];
   float refOffset[16];
@@ -459,6 +467,9 @@ int align_frame_pairs(nicp_context *ctx, const FrameSet &fs, int n, const nicp_c
                       const nicp_cloud *const *curs, const nicp_align_params *ap, const float refOffset[16],
                       const float curOffset[16], const float *guesses, const nicp_prior *priors, const int *priorOffsets,
                       float imgThr, nicp_align_result *results);
+int prep_scene_frames(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *raws, const nicp_stats_params *sp,
+                      const float sensorOffset[16], float baseline, float alpha, nicp_cloud *const *frames,
+                      const nicp_cloud *const *maps, const int *mapPoints, const float *views, nicp_cloud *const *subs);
 // frame_prep.cu
 int launch_depth_convert(nicp_context *ctx, const uint16_t *d_raw, int rows, int cols, float scale, int step,
                          float maxCov, float *d_out);
@@ -467,6 +478,8 @@ int launch_frame_prep(nicp_context *ctx, const float *d_depth, const nicp_projec
                       const CamSet *cams = nullptr);
 int launch_raw_prep_batch(nicp_context *ctx, const FrameSet &fs, int n, const uint16_t *const *d_raw,
                           const nicp_stats_params *sp, const float sensorOffset[16], int keepStats, nicp_cloud *const *clouds);
+int launch_depth_prep_batch(nicp_context *ctx, const FrameSet &fs, int n, const nicp_stats_params *sp,
+                            const float sensorOffset[16], nicp_cloud *const *clouds);
 int launch_stats_stage(nicp_context *ctx, const float4 *d_points, int n, const int *d_index, const int *d_interval, int rows,
                        int cols, const nicp_stats_params *sp, float *d_integral, float4 *d_normals, float *d_stats16,
                        float *d_eigvals, int *d_statsN, float *d_curvature);
@@ -486,6 +499,8 @@ int ensure_points3(nicp_context *ctx, nicp_cloud *cloud);
 int ensure_pn(nicp_context *ctx, nicp_cloud *cloud);
 int launch_decode_z(nicp_context *ctx, const unsigned long long *d_z, int n, int *d_index, float *d_depth,
                     float emptyDepth = FLT_MAX, int epoch = kEpochFresh);
+int launch_render_maps(nicp_context *ctx, const MapRenderSet &R, int m, int maxPoints, const nicp_projector *proj,
+                       unsigned long long *d_z, size_t zStride, float *d_depth, size_t depthStride);
 void cam_mats_KRt(const CamSet &cams, const float T[16], CamMats &out);
 CamGeom geom_of(const CamSet &c);
 int run_align_chunk(nicp_context *ctx, int nPairs, const AlignConsts &ac, const CamSet &cams, const float curOffset[16], int outerIters,
@@ -510,6 +525,10 @@ int launch_local_map_set(nicp_context *ctx, const FrameSet &fs, int m, nicp_clou
                          const float *baseline, const float *alpha, const float sensorOffset[16], nicp_cloud *map,
                          long long *d_run);
 int launch_local_map_commit(nicp_context *ctx, nicp_cloud *map, const long long *d_run, int newSize);
+int launch_set_gaussians(nicp_context *ctx, const FrameSet &fs, int m, nicp_cloud *const *frames, const float *baseline,
+                         const float *alpha, const float sensorOffset[16]);
+int launch_scene_append(nicp_context *ctx, int n, nicp_cloud *const *frames, nicp_cloud *const *maps, const float *poses,
+                        const int *framePoints, const int *mapPoints);
 int run_merge(nicp_context *ctx, nicp_cloud *cloud, const nicp_projector *proj, const float transform[16],
               const nicp_merge_params *mp, int n, int *collapsedHost, int *newSize);
 int run_voxelize(nicp_context *ctx, nicp_cloud *cloud, float resolution, int n, int *repHost, int *newSize);

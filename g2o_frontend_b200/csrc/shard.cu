@@ -29,6 +29,7 @@
 // each sequence stays on one worker with its keyframe and current cloud, and a step is one batched prep and one batched
 // alignment per worker, the pose bookkeeping being done in the calling thread once every worker has succeeded.
 #include <algorithm>
+#include <chrono>
 #include <climits>
 #include <cstdlib>
 #include <cstring>
@@ -80,6 +81,7 @@ struct nicp_shard_pool {
   int frameCap;  // NICP_SHARD_FRAMES (>= 2), 0 = unset
   std::vector<nicp_frame_store *> stores;  // released when the pool is destroyed
   std::vector<nicp_tracker *> trackers;    // likewise
+  std::vector<nicp_scene_tracker *> sceneTrackers;  // likewise
 };
 
 struct nicp_frame_store {
@@ -113,6 +115,32 @@ struct nicp_tracker {
   std::vector<TrackSeq> seqs;
 };
 
+// The state of one sequence of a scene tracker: the loop variables of pwn_aligner.cpp:129-222 (the localmap mode of
+// host/pwn_simple_aligner.cpp), with the local map, the cloud the next frame is prepared into and the subscene rendered
+// from the map living on the sequence's worker.
+struct SceneSeq {
+  int worker;
+  nicp_cloud *map, *frame, *sub;
+  float globalT[16], sceneT[16];  // column-major
+  int frames;                     // frames processed since create / reset (0: the next one is the driver's firstDepth)
+  int counter;                    // the driver's chunk counter
+  int mapPoints;                  // host mirror of the map's count
+  bool broken;                    // a step failed on the device after it had started changing this map: reset first
+};
+
+struct nicp_scene_tracker {
+  nicp_shard_pool *pool;  // null once the pool has been destroyed
+  nicp::FrameSet fs;
+  nicp_stats_params sp;
+  nicp_align_params ap;
+  nicp_merge_params mp;
+  float imgThr, baseline, alpha;
+  float sensorOffset[16];
+  int chunkStep, mapCapacity;
+  std::vector<SceneSeq> seqs;
+  double phaseMs[2];  // host time of phase 1 (prep, render, align) and phase 2 (append, merge), summed over steps
+};
+
 using namespace nicp;
 
 // frames a worker keeps as clouds of px pixels at once.  A cloud costs 112 B per pixel: 80 B of points, normals and Omega,
@@ -125,6 +153,40 @@ static int frame_cap(const nicp_shard_pool *pool, const nicp_shard_pool::Worker 
   int cap = (int)std::min<size_t>(fit, INT_MAX);
   if (pool->frameCap && pool->frameCap < cap) cap = pool->frameCap;
   return std::max(cap, 2);
+}
+
+// Runs work(g) for every worker of the pool, on one thread per worker when there are several; work sets the worker's rc
+// and error.  Returns the first failing worker's status, with its message, or NICP_OK.
+template <typename Work>
+static int run_workers(nicp_shard_pool *pool, Work &&work) {
+  const int G = (int)pool->workers.size();
+  if (G == 1) {
+    work(0);
+  } else {
+    std::vector<std::thread> threads;
+    threads.reserve(G);
+    for (int g = 0; g < G; g++) threads.emplace_back(work, g);
+    for (std::thread &t : threads) t.join();
+  }
+  for (int g = 0; g < G; g++)
+    if (pool->workers[g].rc != NICP_OK) {
+      set_error("device %d (shard %d of %d): %s", pool->workers[g].device, g, G, pool->workers[g].error.c_str());
+      return pool->workers[g].rc;
+    }
+  return NICP_OK;
+}
+
+// body() on worker w's device, then a synchronisation of its context (no upload of the step may still be reading the
+// caller's raw images when the call returns): the worker's rc and error
+template <typename Body>
+static void worker_step(nicp_shard_pool::Worker &w, Body &&body) {
+  w.rc = body();
+  if (w.rc) w.error = nicp_last_error();  // this worker thread's message
+  const int sync = nicp_synchronize(w.ctx);
+  if (!w.rc && sync) {
+    w.rc = sync;
+    w.error = nicp_last_error();
+  }
 }
 
 // The pairs of a sharded call, frames in and records out: every check in the calling thread, so that the error is the same
@@ -273,20 +335,7 @@ static int align_frames_sharded(nicp_shard_pool *pool, nicp_frame_store *store, 
     w.rc = hi > lo ? align_block(w, res, lo, hi) : NICP_OK;
     w.error = w.rc ? nicp_last_error() : "";  // this worker thread's message
   };
-  if (G == 1) {
-    work(0);
-  } else {
-    std::vector<std::thread> threads;
-    threads.reserve(G);
-    for (int g = 0; g < G; g++) threads.emplace_back(work, g);
-    for (std::thread &t : threads) t.join();
-  }
-  for (int g = 0; g < G; g++)
-    if (pool->workers[g].rc != NICP_OK) {
-      set_error("device %d (shard %d of %d): %s", pool->workers[g].device, g, G, pool->workers[g].error.c_str());
-      return pool->workers[g].rc;
-    }
-  return NICP_OK;
+  return run_workers(pool, work);
 }
 
 static int store_create(nicp_shard_pool *pool, const FrameSet &fs, const nicp_stats_params *sp,
@@ -379,22 +428,34 @@ static int tracker_usable(const nicp_tracker *t) {
   return NICP_OK;
 }
 
-static int tracker_create(nicp_shard_pool *pool, int S, const FrameSet &fs, const nicp_stats_params *sp,
-                          const float sensor_offset[16], const nicp_align_params *ap, float imgThr, float newFraction,
-                          nicp_tracker **out) {
+// The placement of a tracker's S sequences: sequence s on worker floor(s G / S), for the tracker's lifetime.  Each sequence
+// needs `units` clouds of px pixels on its worker (each named `each` in the message); NICP_ERR_INVALID when a worker's
+// sequences need more than its frame cap.
+static int place_sequences(const nicp_shard_pool *pool, int S, size_t px, long long units, const char *each,
+                           std::vector<int> &worker) {
   const int G = (int)pool->workers.size();
-  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
-  std::vector<int> worker(S), onWorker(G, 0);
+  std::vector<int> onWorker(G, 0);
+  worker.resize(S);
   for (int s = 0; s < S; s++) onWorker[worker[s] = (int)((long long)s * G / S)]++;
   for (int g = 0; g < G; g++) {
     const int cap = frame_cap(pool, pool->workers[g], px);
-    if ((long long)2 * onWorker[g] > cap) {
-      set_error("worker %d (GPU %d) would hold %d sequences at two clouds each, more than its frame cap of %d clouds of "
+    if (units * onWorker[g] > cap) {
+      set_error("worker %d (GPU %d) would hold %d sequences at %s each, more than its frame cap of %d clouds of "
                 "%zu pixels (NICP_SHARD_FRAMES lowers the cap): use more workers or fewer sequences",
-                g, pool->workers[g].device, onWorker[g], cap, px);
+                g, pool->workers[g].device, onWorker[g], each, cap, px);
       return NICP_ERR_INVALID;
     }
   }
+  return NICP_OK;
+}
+
+static int tracker_create(nicp_shard_pool *pool, int S, const FrameSet &fs, const nicp_stats_params *sp,
+                          const float sensor_offset[16], const nicp_align_params *ap, float imgThr, float newFraction,
+                          nicp_tracker **out) {
+  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
+  std::vector<int> worker;
+  int rc;
+  if ((rc = place_sequences(pool, S, px, 2, "two clouds", worker))) return rc;
   nicp_tracker *t = new nicp_tracker();
   t->pool = pool;
   t->fs = fs;
@@ -411,7 +472,6 @@ static int tracker_create(nicp_shard_pool *pool, int S, const FrameSet &fs, cons
     q.key = q.cur = nullptr;
     track_restart(q);
     nicp_context *ctx = pool->workers[q.worker].ctx;
-    int rc;
     if ((rc = nicp_cloud_create(ctx, (int)px, &q.key)) || (rc = nicp_cloud_create(ctx, (int)px, &q.cur))) {
       tracker_release(t);
       delete t;
@@ -424,12 +484,12 @@ static int tracker_create(nicp_shard_pool *pool, int S, const FrameSet &fs, cons
 }
 
 // n distinct sequences in [0, S)
-static int check_sequences(const nicp_tracker *t, int n, const int *sequences) {
-  std::vector<char> seen(t->seqs.size(), 0);
+static int check_sequences(int S, int n, const int *sequences) {
+  std::vector<char> seen(S, 0);
   for (int k = 0; k < n; k++) {
     const int s = sequences[k];
-    if (s < 0 || s >= (int)t->seqs.size()) {
-      set_error("entry %d names sequence %d outside [0, %d)", k, s, (int)t->seqs.size());
+    if (s < 0 || s >= S) {
+      set_error("entry %d names sequence %d outside [0, %d)", k, s, S);
       return NICP_ERR_INVALID;
     }
     if (seen[s]) {
@@ -439,6 +499,56 @@ static int check_sequences(const nicp_tracker *t, int n, const int *sequences) {
     seen[s] = 1;
   }
   return NICP_OK;
+}
+
+// ---- scene trackers -------------------------------------------------------------------------------------------------------
+
+static void scene_restart(SceneSeq &s, const float *pose) {
+  if (pose) {
+    memcpy(s.globalT, pose, sizeof s.globalT);
+    fix_last_row(s.globalT);
+  } else {
+    mat4_identity(s.globalT);
+  }
+  memcpy(s.sceneT, s.globalT, sizeof s.sceneT);
+  s.frames = s.counter = s.mapPoints = 0;
+  s.broken = false;
+}
+
+static void scene_release(nicp_scene_tracker *t) {
+  for (SceneSeq &s : t->seqs) {
+    nicp_cloud_destroy(s.map);
+    nicp_cloud_destroy(s.frame);
+    nicp_cloud_destroy(s.sub);
+    s.map = s.frame = s.sub = nullptr;
+  }
+}
+
+// NICP_ERR_INVALID (with a message) for a null scene tracker or one whose pool is gone
+static int scene_usable(const nicp_scene_tracker *t) {
+  if (!t) return NICP_ERR_INVALID;
+  if (!t->pool) {
+    set_error("the scene tracker's shard pool has been destroyed: only nicp_scene_tracker_destroy may be called");
+    return NICP_ERR_INVALID;
+  }
+  return NICP_OK;
+}
+
+// the frame caps count a sequence's map as its bytes in units of a frame cloud: 112 B per pixel (frame_cap), and 100 B of
+// gaussian and flag per point on top for the frame cloud and the map.  A map costs 80 B per point for its record, not
+// frame_cap's 112: it is never aligned, so it gets no interleaved point / normal copy (ensure_pn), and the merge and the
+// render project it with k_project_single / k_render_maps_z, which read the float4 points, not the packed copy
+// (ensure_points3).  The frame cloud and the subscene are aligned and get the copies.
+static long long scene_units(size_t px, int mapCapacity) {
+  const size_t unit = 112 * px;
+  const size_t bytes = (112 + 100) * px + 112 * px + (size_t)(80 + 100) * (size_t)mapCapacity;
+  return (long long)((bytes + unit - 1) / unit);
+}
+
+// a * b as Isometry3f * Isometry3f (include/pwn/compat.h), last row rewritten
+static void scene_mul(const float *a, const float *b, float *out) {
+  iso_mul(a, b, out);
+  fix_last_row(out);
 }
 
 extern "C" {
@@ -485,6 +595,10 @@ void nicp_shard_pool_destroy(nicp_shard_pool *pool) {
   }
   for (nicp_tracker *t : pool->trackers) {
     tracker_release(t);
+    t->pool = nullptr;
+  }
+  for (nicp_scene_tracker *t : pool->sceneTrackers) {
+    scene_release(t);
     t->pool = nullptr;
   }
   for (nicp_shard_pool::Worker &w : pool->workers) {
@@ -718,7 +832,7 @@ int nicp_tracker_reset(nicp_tracker *tracker, int n, const int *sequences) {
   if (n < 0) return NICP_ERR_INVALID;
   if (n == 0) return NICP_OK;
   if (!sequences) return NICP_ERR_INVALID;
-  if ((rc = check_sequences(tracker, n, sequences))) return rc;
+  if ((rc = check_sequences((int)tracker->seqs.size(), n, sequences))) return rc;
   for (int k = 0; k < n; k++) track_restart(tracker->seqs[sequences[k]]);
   return NICP_OK;
 }
@@ -730,7 +844,7 @@ int nicp_tracker_step(nicp_tracker *tracker, int n, const int *sequences, const 
   if (n < 0) return NICP_ERR_INVALID;
   if (n == 0) return NICP_OK;
   if (!sequences || !raws || !results) return NICP_ERR_INVALID;
-  if ((rc = check_sequences(tracker, n, sequences))) return rc;
+  if ((rc = check_sequences((int)tracker->seqs.size(), n, sequences))) return rc;
   const FrameSet &fs = tracker->fs;
   const int nc = fs.cams.n;
   for (int k = 0; k < n; k++)
@@ -799,28 +913,9 @@ int nicp_tracker_step(nicp_tracker *tracker, int n, const int *sequences, const 
       for (size_t i = 0; i < aligned.size(); i++) recs[aligned[i]] = out[i];
       return NICP_OK;
     };
-    w.rc = body();
-    if (w.rc) w.error = nicp_last_error();  // this worker thread's message
-    // no upload of this step may still be reading the caller's raw images when the call returns
-    const int sync = nicp_synchronize(w.ctx);
-    if (!w.rc && sync) {
-      w.rc = sync;
-      w.error = nicp_last_error();
-    }
+    worker_step(w, body);
   };
-  if (G == 1) {
-    work(0);
-  } else {
-    std::vector<std::thread> threads;
-    threads.reserve(G);
-    for (int g = 0; g < G; g++) threads.emplace_back(work, g);
-    for (std::thread &t : threads) t.join();
-  }
-  for (int g = 0; g < G; g++)
-    if (pool->workers[g].rc != NICP_OK) {
-      set_error("device %d (shard %d of %d): %s", pool->workers[g].device, g, G, pool->workers[g].error.c_str());
-      return pool->workers[g].rc;
-    }
+  if ((rc = run_workers(pool, work))) return rc;
   for (int k = 0; k < n; k++)
     if (tracker->seqs[sequences[k]].hasKey && recs[k].status != NICP_OK) {
       set_error("entry %d (sequence %d): the alignment's record has status %d", k, sequences[k], recs[k].status);
@@ -859,6 +954,322 @@ int nicp_tracker_step(nicp_tracker *tracker, int n, const int *sequences, const 
     memcpy(r.global_T, s.globalT, sizeof r.global_T);
     r.num_keyframes = s.numKeyframes;
   }
+  return NICP_OK;
+}
+
+int nicp_scene_tracker_create(nicp_shard_pool *pool, int n_sequences, int raw_rows, int raw_cols, float depth_scale, int step,
+                              float max_depth_cov, const nicp_projector *proj, const nicp_stats_params *sp,
+                              const float sensor_offset[16], float baseline, float alpha, const nicp_align_params *ap,
+                              float frame_inlier_depth_threshold, const nicp_merge_params *mp, int chunk_step,
+                              int map_capacity, nicp_scene_tracker **tracker) {
+  if (!tracker) return NICP_ERR_INVALID;
+  *tracker = nullptr;
+  if (!pool || !proj || !sp || !ap || !mp || raw_rows <= 0 || raw_cols <= 0 || n_sequences <= 0) return NICP_ERR_INVALID;
+  if (chunk_step < 0 || map_capacity <= 0) {
+    set_error("chunk_step %d must be >= 0 and map_capacity %d > 0", chunk_step, map_capacity);
+    return NICP_ERR_INVALID;
+  }
+  FrameSet fs;
+  int rc;
+  if ((rc = frames_pinhole(proj, raw_rows, raw_cols, depth_scale, step, max_depth_cov, fs))) return rc;
+  const size_t px = (size_t)fs.proj.rows * fs.proj.cols;
+  const long long units = scene_units(px, map_capacity);
+  char each[128];
+  snprintf(each, sizeof each, "%lld clouds (frame, subscene and a map of %d points)", units, map_capacity);
+  std::vector<int> worker;
+  if ((rc = place_sequences(pool, n_sequences, px, units, each, worker))) return rc;
+  nicp_scene_tracker *t = new nicp_scene_tracker();
+  t->pool = pool;
+  t->fs = fs;
+  t->sp = *sp;
+  t->ap = *ap;
+  t->mp = *mp;
+  t->imgThr = frame_inlier_depth_threshold;
+  t->baseline = baseline;
+  t->alpha = alpha;
+  if (sensor_offset)
+    memcpy(t->sensorOffset, sensor_offset, sizeof t->sensorOffset);
+  else
+    mat4_identity(t->sensorOffset);
+  t->chunkStep = chunk_step;
+  t->mapCapacity = map_capacity;
+  t->phaseMs[0] = t->phaseMs[1] = 0.0;
+  t->seqs.resize(n_sequences);
+  for (int s = 0; s < n_sequences; s++) {
+    SceneSeq &q = t->seqs[s];
+    q.worker = worker[s];
+    q.map = q.frame = q.sub = nullptr;
+    scene_restart(q, nullptr);
+    nicp_context *ctx = pool->workers[q.worker].ctx;
+    if ((rc = nicp_cloud_create(ctx, map_capacity, &q.map)) || (rc = cloud_ensure_gaussians(ctx, q.map)) ||
+        (rc = nicp_cloud_create(ctx, (int)px, &q.frame)) || (rc = cloud_ensure_gaussians(ctx, q.frame)) ||
+        (rc = nicp_cloud_create(ctx, (int)px, &q.sub))) {
+      scene_release(t);
+      delete t;
+      return rc;
+    }
+    q.map->has_gauss = true;  // an empty map with gaussians, as Cloud::add leaves it
+  }
+  pool->sceneTrackers.push_back(t);
+  *tracker = t;
+  return NICP_OK;
+}
+
+void nicp_scene_tracker_destroy(nicp_scene_tracker *tracker) {
+  if (!tracker) return;
+  if (tracker->pool) {
+    std::vector<nicp_scene_tracker *> &v = tracker->pool->sceneTrackers;
+    v.erase(std::remove(v.begin(), v.end(), tracker), v.end());
+    scene_release(tracker);
+  }
+  delete tracker;
+}
+
+int nicp_scene_tracker_size(const nicp_scene_tracker *tracker) {
+  return scene_usable(tracker) ? -1 : (int)tracker->seqs.size();
+}
+
+int nicp_scene_tracker_reset(nicp_scene_tracker *tracker, int n, const int *sequences, const float *initial_poses) {
+  int rc;
+  if ((rc = scene_usable(tracker))) return rc;
+  if (n < 0) return NICP_ERR_INVALID;
+  if (n == 0) return NICP_OK;
+  if (!sequences) return NICP_ERR_INVALID;
+  if ((rc = check_sequences((int)tracker->seqs.size(), n, sequences))) return rc;
+  // the map's device count is reset by the sequence's next step (it restarts the map)
+  for (int k = 0; k < n; k++) scene_restart(tracker->seqs[sequences[k]], initial_poses ? initial_poses + 16 * (size_t)k : nullptr);
+  return NICP_OK;
+}
+
+int nicp_scene_tracker_step(nicp_scene_tracker *tracker, int n, const int *sequences, const uint16_t *const *raws,
+                            nicp_scene_track_result *results) {
+  int rc;
+  if ((rc = scene_usable(tracker))) return rc;
+  if (n < 0) return NICP_ERR_INVALID;
+  if (n == 0) return NICP_OK;
+  if (!sequences || !raws || !results) return NICP_ERR_INVALID;
+  if ((rc = check_sequences((int)tracker->seqs.size(), n, sequences))) return rc;
+  for (int k = 0; k < n; k++) {
+    if (!raws[k]) {
+      set_error("null raw image in entry %d (sequence %d)", k, sequences[k]);
+      return NICP_ERR_INVALID;
+    }
+    if (tracker->seqs[sequences[k]].broken) {
+      set_error("sequence %d failed on the device in an earlier step: nicp_scene_tracker_reset it first", sequences[k]);
+      return NICP_ERR_INVALID;
+    }
+  }
+  nicp_shard_pool *pool = tracker->pool;
+  const FrameSet &fs = tracker->fs;
+  const float *so = tracker->sensorOffset;
+  const int G = (int)pool->workers.size();
+  std::vector<std::vector<int>> entries(G);  // entries of the step on worker g, in listed order
+  std::vector<float> views((size_t)16 * n);  // KRt of the render view sceneT * sensorOffset (pwn_aligner.cpp:160)
+  for (int k = 0; k < n; k++) {
+    const SceneSeq &s = tracker->seqs[sequences[k]];
+    entries[s.worker].push_back(k);
+    float T[16];
+    scene_mul(s.sceneT, so, T);
+    compute_KRt(fs.proj.K, T, &views[(size_t)16 * k]);
+  }
+  using Clock = std::chrono::steady_clock;
+  const Clock::time_point t0 = Clock::now();
+
+  // phase 1, every worker: frames, gaussians, renders and subscenes in one batched prep, one batched alignment of the
+  // sequences that have a map, the frames' point counts
+  std::vector<nicp_align_result> recs(n);
+  std::vector<int> framePoints(n, 0);
+  auto phase1 = [&](int g) {
+    nicp_shard_pool::Worker &w = pool->workers[g];
+    const std::vector<int> &mine = entries[g];
+    w.rc = NICP_OK;
+    w.error.clear();
+    if (mine.empty()) return;
+    std::vector<int> counts(mine.size(), 0);  // written by the device before worker_step's synchronisation
+    auto body = [&]() -> int {
+      NICP_CUDA(cudaSetDevice(w.device));
+      const size_t m = mine.size();
+      std::vector<const uint16_t *> frameRaws(m);
+      std::vector<nicp_cloud *> frames(m), subs(m);
+      std::vector<const nicp_cloud *> maps(m), refs, curs;
+      std::vector<int> mapPoints(m);
+      std::vector<float> mv((size_t)16 * m);
+      std::vector<int> aligned;
+      for (size_t i = 0; i < m; i++) {
+        const int k = mine[i];
+        const SceneSeq &s = tracker->seqs[sequences[k]];
+        frameRaws[i] = raws[k];
+        frames[i] = s.frame;
+        subs[i] = s.sub;
+        maps[i] = s.frames > 0 ? s.map : nullptr;
+        mapPoints[i] = s.mapPoints;
+        memcpy(&mv[16 * i], &views[(size_t)16 * k], 16 * sizeof(float));
+        if (s.frames > 0) {
+          refs.push_back(s.sub);
+          curs.push_back(s.frame);
+          aligned.push_back(k);
+        }
+      }
+      int rc;
+      if ((rc = prep_scene_frames(w.ctx, fs, (int)m, frameRaws.data(), &tracker->sp, so, tracker->baseline, tracker->alpha,
+                                  frames.data(), maps.data(), mapPoints.data(), mv.data(), subs.data())))
+        return rc;
+      if (!refs.empty()) {
+        std::vector<nicp_align_result> out(refs.size());
+        if ((rc = align_frame_pairs(w.ctx, fs, (int)refs.size(), refs.data(), curs.data(), &tracker->ap, so, so, nullptr,
+                                    nullptr, nullptr, tracker->imgThr, out.data())))
+          return rc;
+        for (size_t i = 0; i < aligned.size(); i++) recs[aligned[i]] = out[i];
+      }
+      for (size_t i = 0; i < m; i++)
+        NICP_CUDA(cudaMemcpyAsync(&counts[i], frames[i]->d_n, sizeof(int), cudaMemcpyDeviceToHost, w.ctx->stream));
+      return NICP_OK;
+    };
+    worker_step(w, body);
+    if (!w.rc)
+      for (size_t i = 0; i < mine.size(); i++) framePoints[mine[i]] = counts[i];
+  };
+  if ((rc = run_workers(pool, phase1))) return rc;
+  const Clock::time_point t1 = Clock::now();
+
+  // between the phases, in the calling thread: tentative poses, chunk decisions (pwn_aligner.cpp:194-205) and capacities
+  struct Next {
+    float globalT[16], sceneT[16];
+    int counter, newMap, base;  // base: the map's size before the append (0 when it restarts)
+  };
+  std::vector<Next> next(n);
+  for (int k = 0; k < n; k++) {
+    const SceneSeq &s = tracker->seqs[sequences[k]];
+    Next &x = next[k];
+    memcpy(x.globalT, s.globalT, sizeof x.globalT);
+    memcpy(x.sceneT, s.sceneT, sizeof x.sceneT);
+    x.counter = s.counter;
+    x.newMap = 0;
+    if (s.frames > 0) {
+      if (recs[k].status != NICP_OK) {
+        set_error("entry %d (sequence %d): the alignment's record has status %d", k, sequences[k], recs[k].status);
+        return recs[k].status;
+      }
+      scene_mul(x.globalT, recs[k].T, x.globalT);
+      scene_mul(x.sceneT, recs[k].T, x.sceneT);
+      if (tracker->chunkStep > 0 && x.counter++ % tracker->chunkStep == 0) {
+        mat4_identity(x.sceneT);
+        x.newMap = 1;
+      }
+    }
+    x.base = (x.newMap || s.frames == 0) ? 0 : s.mapPoints;
+    if ((long long)x.base + framePoints[k] > tracker->mapCapacity) {
+      set_error("entry %d (sequence %d): %d map points + %d frame points exceed the map capacity %d", k, sequences[k], x.base,
+                framePoints[k], tracker->mapCapacity);
+      return NICP_ERR_INVALID;
+    }
+  }
+
+  // phase 2, every worker: restarting maps emptied, one append launch, the merges
+  std::vector<int> merged(n, 0);
+  auto phase2 = [&](int g) {
+    nicp_shard_pool::Worker &w = pool->workers[g];
+    const std::vector<int> &mine = entries[g];
+    w.rc = NICP_OK;
+    w.error.clear();
+    if (mine.empty()) return;
+    auto body = [&]() -> int {
+      NICP_CUDA(cudaSetDevice(w.device));
+      const size_t m = mine.size();
+      std::vector<nicp_cloud *> frames(m), maps(m);
+      std::vector<float> poses((size_t)16 * m);
+      std::vector<int> fp(m), base(m);
+      for (size_t i = 0; i < m; i++) {
+        const int k = mine[i];
+        const SceneSeq &s = tracker->seqs[sequences[k]];
+        frames[i] = s.frame;
+        maps[i] = s.map;
+        memcpy(&poses[16 * i], next[k].sceneT, sizeof next[k].sceneT);
+        fp[i] = framePoints[k];
+        base[i] = next[k].base;
+        if (!base[i]) NICP_CUDA(cudaMemsetAsync(s.map->d_n, 0, sizeof(int), w.ctx->stream));
+      }
+      int rc;
+      if ((rc = launch_scene_append(w.ctx, (int)m, frames.data(), maps.data(), poses.data(), fp.data(), base.data())))
+        return rc;
+      for (size_t i = 0; i < m; i++) {
+        const int k = mine[i];
+        const int size = base[i] + fp[i];
+        if (!size) continue;  // nicp_merge leaves an empty map as it is
+        float T[16];
+        scene_mul(next[k].sceneT, so, T);  // Merger::merge(map, sceneT * sensorOffset), pwn_aligner.cpp:207
+        if ((rc = run_merge(w.ctx, maps[i], &fs.proj, T, &tracker->mp, size, nullptr, &merged[k]))) return rc;
+      }
+      return NICP_OK;
+    };
+    worker_step(w, body);
+  };
+  rc = run_workers(pool, phase2);
+  const Clock::time_point t2 = Clock::now();
+  tracker->phaseMs[0] += std::chrono::duration<double, std::milli>(t1 - t0).count();
+  tracker->phaseMs[1] += std::chrono::duration<double, std::milli>(t2 - t1).count();
+  if (rc) {
+    for (int k = 0; k < n; k++) tracker->seqs[sequences[k]].broken = true;
+    return rc;
+  }
+
+  // commit, in the calling thread
+  for (int k = 0; k < n; k++) {
+    SceneSeq &s = tracker->seqs[sequences[k]];
+    const Next &x = next[k];
+    nicp_scene_track_result &r = results[k];
+    memset(&r, 0, sizeof r);
+    r.frame = s.frames;
+    r.record.status = NICP_OK;
+    if (s.frames > 0) {
+      r.aligned = 1;
+      r.record = recs[k];
+    }
+    memcpy(s.globalT, x.globalT, sizeof s.globalT);
+    memcpy(s.sceneT, x.sceneT, sizeof s.sceneT);
+    s.counter = x.counter;
+    s.mapPoints = merged[k];
+    s.frames++;
+    memcpy(r.global_T, s.globalT, sizeof r.global_T);
+    memcpy(r.scene_T, s.sceneT, sizeof r.scene_T);
+    r.new_map = x.newMap;
+    r.added = x.base + framePoints[k];
+    r.map_points = s.mapPoints;
+  }
+  return NICP_OK;
+}
+
+int nicp_scene_tracker_download_map(nicp_scene_tracker *tracker, int sequence, int capacity, float *points4, float *normals4,
+                                    float *curvature, float *omega_p6, float *omega_n6, float *gauss24, int *gflags, int *n) {
+  int rc;
+  if ((rc = scene_usable(tracker))) return rc;
+  if (sequence < 0 || sequence >= (int)tracker->seqs.size()) {
+    set_error("sequence %d outside [0, %d)", sequence, (int)tracker->seqs.size());
+    return NICP_ERR_INVALID;
+  }
+  const SceneSeq &s = tracker->seqs[sequence];
+  if (s.broken) {
+    set_error("sequence %d failed on the device in an earlier step: its map is undefined until nicp_scene_tracker_reset",
+              sequence);
+    return NICP_ERR_INVALID;
+  }
+  if (n) *n = s.mapPoints;
+  if (capacity < s.mapPoints) {
+    set_error("the map of sequence %d holds %d points, more than the capacity %d", sequence, s.mapPoints, capacity);
+    return NICP_ERR_INVALID;
+  }
+  if (!s.mapPoints) return NICP_OK;
+  nicp_context *ctx = tracker->pool->workers[s.worker].ctx;
+  if ((rc = nicp_cloud_download(ctx, s.map, points4, normals4, curvature, omega_p6, omega_n6))) return rc;
+  if ((gauss24 || gflags) && (rc = nicp_cloud_download_gaussians(ctx, s.map, gauss24, gflags))) return rc;
+  return NICP_OK;
+}
+
+int nicp_scene_tracker_phase_ms(const nicp_scene_tracker *tracker, double *phase1_ms, double *phase2_ms) {
+  int rc;
+  if ((rc = scene_usable(tracker))) return rc;
+  if (phase1_ms) *phase1_ms = tracker->phaseMs[0];
+  if (phase2_ms) *phase2_ms = tracker->phaseMs[1];
   return NICP_OK;
 }
 

@@ -594,6 +594,79 @@ int nicp_tracker_step(nicp_tracker *tracker, int n, const int *sequences, const 
 /* the listed sequences start over: no keyframe, global pose identity, counters 0 */
 int nicp_tracker_reset(nicp_tracker *tracker, int n, const int *sequences);
 
+/* ---- batched scene-based odometry: many depth sequences against their own local maps on a shard pool ------------------
+ * The mapping loop of pwn_core/pwn_aligner.cpp:129-222 (the localmap mode of host/pwn_simple_aligner.cpp) for S independent
+ * pinhole sequences: every frame is aligned against the sequence's local map re-rendered at the predicted pose, added to
+ * the map (Cloud::add) and fused into it (Merger::merge); after the first alignment and then every chunk_step frames the map
+ * is closed and a new one starts from the current frame (chunk_step 0: one map for the whole sequence).
+ *   - Semantics: each listed sequence does on its frame exactly what this chain of single calls does, byte for byte:
+ *       1. frame cloud = nicp_raw_depth_to_cloud (keep_stats 0, sensor_offset) with the gaussians of
+ *          nicp_cloud_compute_gaussians(baseline, alpha, sensor_offset) of the same depth;
+ *       2. if the sequence processed a frame since create / reset: depth = nicp_project(map, KRt(sceneT * sensor_offset))
+ *          (FLT_MAX where empty), subscene = nicp_depth_to_cloud(depth, keep_stats 0, sensor_offset), record =
+ *          nicp_align(subscene, frame cloud, proj, ap, sensor_offset, sensor_offset, identity guess, no priors,
+ *          frame_inlier_depth_threshold), globalT = globalT * T, sceneT = sceneT * T; then, if chunk_step > 0 and
+ *          counter++ % chunk_step == 0, sceneT = identity and the map is emptied (new_map = 1);
+ *       3. nicp_cloud_append(map, frame cloud, sceneT), then nicp_merge(map, proj, sceneT * sensor_offset, mp).
+ *     The pose products are float32 Isometry3f products in the operation order of include/pwn/compat.h with the last row
+ *     rewritten, and nothing re-orthogonalises them (the reference loop does not).  Frames are aligned whatever their inliers.
+ *   - Placement and memory: sequence s lives on worker floor(s * G / S) and owns three device clouds there, allocated at
+ *     create: its map (map_capacity points, with gaussians), a frame cloud and a subscene cloud (image pixels each).
+ *     Creation fails with NICP_ERR_INVALID when a worker's sequences exceed the frame cap of the sharded entries
+ *     (NICP_SHARD_FRAMES lowers it), a map counting as its bytes in units of frame clouds.
+ *   - One step: every argument is checked in the calling thread first (null arrays or images, a sequence outside [0, S),
+ *     listed twice or needing a reset, a destroyed pool).  Phase 1, per worker: one batched prep of the frames with their
+ *     gaussians, in launch sets of up to 8, each set rendering its maps straight into the prep's depth scratch and building
+ *     the subscenes from there; one batched alignment of the (subscene, frame) pairs; a synchronisation.  Then, in the
+ *     calling thread, the tentative poses and chunk decisions, and the capacity of every listed map: its size (0 when it
+ *     restarts) plus the frame's points must fit map_capacity.  A record whose status is not NICP_OK, or a map too small,
+ *     fails the step with NICP_ERR_INVALID (or that status) and changes nothing.  Phase 2, per worker: the restarting maps
+ *     are emptied, every frame is appended to its own map with its own sceneT in one launch, each map is merged, and the
+ *     worker is synchronised; the poses and counters are committed when every worker succeeded.
+ *   - A CUDA error in phase 2 is returned and leaves the listed sequences' maps undefined: every later step or map download
+ *     that names one of them returns NICP_ERR_INVALID until nicp_scene_tracker_reset.
+ *   - nicp_shard_pool_destroy releases the trackers' clouds; every later call on such a tracker except
+ *     nicp_scene_tracker_destroy returns NICP_ERR_INVALID (nicp_scene_tracker_size returns -1).  Calls are synchronous; a
+ *     pool and its trackers are used from one host thread at a time. */
+typedef struct {
+  float global_T[16];        /* globalT after this frame (column-major) */
+  float scene_T[16];         /* sceneT after this frame (identity when this frame started a new map) */
+  int frame;                 /* frames this sequence processed before this one, since create / reset */
+  int aligned;               /* 0 for the first frame after create / reset: nothing to align against */
+  int new_map;               /* 1 when the map was closed and restarted from this frame */
+  int added;                 /* map points after the append, before the merge */
+  int map_points;            /* map points after the merge */
+  nicp_align_result record;  /* the alignment's record; zeroed with status NICP_OK when aligned = 0 */
+} nicp_scene_track_result;
+
+typedef struct nicp_scene_tracker nicp_scene_tracker;
+/* the frame description and loop parameters, fixed for the tracker's lifetime: raw size, depth_scale, step, max_depth_cov
+ * and proj (the camera after scaling) as in nicp_raw_depth_to_cloud; sensor_offset (NULL: identity) for the preparation,
+ * the gaussians, both sides of every alignment and the render and merge views; baseline and alpha of the sensor model; ap
+ * and frame_inlier_depth_threshold of every alignment; mp of every merge; chunk_step >= 0; map_capacity > 0 points */
+int nicp_scene_tracker_create(nicp_shard_pool *pool, int n_sequences, int raw_rows, int raw_cols, float depth_scale, int step,
+                              float max_depth_cov, const nicp_projector *proj, const nicp_stats_params *sp,
+                              const float sensor_offset[16], float baseline, float alpha, const nicp_align_params *ap,
+                              float frame_inlier_depth_threshold, const nicp_merge_params *mp, int chunk_step,
+                              int map_capacity, nicp_scene_tracker **tracker);
+void nicp_scene_tracker_destroy(nicp_scene_tracker *tracker);
+/* n_sequences; -1 for a null tracker or one whose pool was destroyed */
+int nicp_scene_tracker_size(const nicp_scene_tracker *tracker);
+/* one frame for each of n distinct sequences: raws[k] is sequence sequences[k]'s raw frame, exactly the raw size given at
+ * create; results[k] receives its result */
+int nicp_scene_tracker_step(nicp_scene_tracker *tracker, int n, const int *sequences, const uint16_t *const *raws,
+                            nicp_scene_track_result *results);
+/* the listed sequences start over with an empty map and counters 0: globalT = sceneT = initial_poses + 16 k (column-major,
+ * last row rewritten; NULL: identity), the driver's initialT */
+int nicp_scene_tracker_reset(nicp_scene_tracker *tracker, int n, const int *sequences, const float *initial_poses);
+/* the map of one sequence, as nicp_cloud_download and nicp_cloud_download_gaussians give it (each output may be NULL);
+ * *n = its size.  NICP_ERR_INVALID, with *n = the size, when capacity is smaller */
+int nicp_scene_tracker_download_map(nicp_scene_tracker *tracker, int sequence, int capacity, float *points4, float *normals4,
+                                    float *curvature, float *omega_p6, float *omega_n6, float *gauss24, int *gflags, int *n);
+/* host time of the two phases of every step since create, in milliseconds (either output may be NULL): phase 1 = prep,
+ * render and alignment up to its synchronisation, phase 2 = append and merges up to theirs */
+int nicp_scene_tracker_phase_ms(const nicp_scene_tracker *tracker, double *phase1_ms, double *phase2_ms);
+
 #ifdef __cplusplus
 }
 #endif
